@@ -9,6 +9,7 @@ env-step of every env on every rank.  `--config 3|4|5` selects the other BASELIN
   5  long slender rod n_elem=512 on the frictional plane, FP64 (the FP32 / FP64 speed ratio is added to the line)
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--scaling weak|strong]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0 (contract in the task statement).  The reference arm (`--impl reference`) times the
@@ -58,7 +59,14 @@ def parse():
     p.add_argument("--envs-per-gpu", type=int, default=None, help="override the env count (per GPU)")
     p.add_argument("--math", default="fast", choices=["fast", "faithful"])
     p.add_argument("--no-cpu-baseline", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the observations, rewards and terminations of the last timed step to DIR/<name>.npy")
+    a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
+    return a
 
 
 def envs_per_rank(args, world):
@@ -293,14 +301,14 @@ class Workload:
             gen = torch.Generator(device=dev).manual_seed(42 + rank)
             self.actions = (torch.rand((W + K, n_env, 24), generator=gen, device=dev) * 10 - 5).float()
             self.a_host = self.actions.cpu().pin_memory()
-            o6, self.rew, self.term = env._scratch
+            self.obs, self.rew, self.term = env._scratch
             W_ = env._W
             rkt = self.handle.rest_kappa_tensor().unflatten(0, (n_env, 8))
 
             def device_step(i):     # what env.step launches, minus the host-side reward / observation reductions
                 a3 = self.actions[i].double().reshape(n_env, 8, 3)
                 rkt[:, :, 0, :] = a3 @ W_.T
-                self.handle.step(None, S, o6, self.rew, self.term)
+                self.handle.step(None, S, self.obs, self.rew, self.term)
 
             def host_step(i):       # the public vector-env API: host actions in, host observations / rewards out
                 obs, rew, term, trunc, _ = env.step(self.a_host[i].to(dev, non_blocking=True))
@@ -321,6 +329,29 @@ class Workload:
 
     def close(self):
         (self.env or self.handle).close()
+
+
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, arrays, limit_bytes, suffix=""):
+    """Write per-env output rows as DIR/<name><suffix>.npy in float32 / float64 (integer outputs become float32).
+    Above `limit_bytes` a fixed, seeded sample of the envs is kept, and their indices go to env_index<suffix>.npy."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        host[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float32)
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a.nbytes for a in host.values()) // n
+    budget = limit_bytes - 4096          # room for the .npy headers
+    if n * row_bytes > budget:
+        keep = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        host = {name: a[keep] for name, a in host.items()}
+        host["env_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 def run_ours(args):
@@ -375,6 +406,9 @@ def run_ours(args):
     per_step_ms = [a.elapsed_time(b) for a, b in ev]
     total_s = max_over_ranks(sum(per_step_ms) * 1e-3)
     wl.check()
+    if args.dump_outputs:       # the end-to-end leg below resets the envs, so this is the last timed step's result
+        dump_outputs(args.dump_outputs, {"obs": wl.obs, "reward": wl.rew, "terminated": wl.term},
+                     DUMP_LIMIT_BYTES // world, f"_rank{rank}" if world > 1 else "")
     env_steps = n_env * world * K
     value = env_steps / total_s
     kernel_s = sum(per_step_ms) * 1e-3 / K          # this rank's average step (= launch) duration
