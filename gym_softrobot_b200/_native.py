@@ -21,7 +21,7 @@ MATH_FAST, MATH_FAITHFUL = 0, 1
 EXPORTED_SYMBOLS = [
     "sr_abi_version", "sr_last_error", "sr_create", "sr_destroy", "sr_obs_dim", "sr_action_dim",
     "sr_init_dim", "sr_reset", "sr_step", "sr_reset_host", "sr_step_host", "sr_observe",
-    "sr_get_state", "sr_set_state", "sr_copy_from", "sr_get_aux", "sr_get_head", "sr_get_rest_kappa", "sr_get_sucker", "sr_get_sucker_index", "sr_get_tm_activation", "sr_get_muscle_activation", "sr_get_fixed_suckers", "sr_get_ext_loads", "sr_get_muscle", "sr_get_spline", "sr_spline_basis", "sr_launch_count", "sr_fallback_count", "sr_fallback_causes", "sr_measure_fp64_peak", "sr_measure_fp64_peak_regs", "sr_selftest_reciprocals", "sr_probe_latency",
+    "sr_get_state", "sr_set_state", "sr_copy_from", "sr_get_aux", "sr_get_head", "sr_get_rest_kappa", "sr_get_sucker", "sr_get_sucker_index", "sr_get_tm_activation", "sr_get_muscle_activation", "sr_get_fixed_suckers", "sr_get_ext_loads", "sr_get_muscle", "sr_get_spline", "sr_spline_basis", "sr_launch_count", "sr_fallback_count", "sr_fallback_causes", "sr_nonplanar_count", "sr_measure_fp64_peak", "sr_measure_fp64_peak_regs", "sr_selftest_reciprocals", "sr_probe_latency",
 ]
 
 
@@ -117,6 +117,8 @@ def load_library():
     L.sr_fallback_count.argtypes = [C.c_void_p]
     L.sr_fallback_count.restype = C.c_int64
     L.sr_fallback_causes.argtypes = [C.c_void_p, C.POINTER(C.c_int64)]
+    L.sr_nonplanar_count.argtypes = [C.c_void_p]
+    L.sr_nonplanar_count.restype = C.c_int64
     L.sr_measure_fp64_peak.argtypes = [C.c_int, C.POINTER(C.c_double)]
     L.sr_measure_fp64_peak_regs.argtypes = [C.c_int, C.POINTER(C.c_double)]
     L.sr_selftest_reciprocals.argtypes = [C.c_int, C.c_int32, C.c_double, C.c_double, C.POINTER(C.c_double)]
@@ -279,6 +281,10 @@ class Handle:
         out = (C.c_int64 * 3)()
         _check(self._lib.sr_fallback_causes(self._h, out))
         return tuple(int(v) for v in out)
+
+    def nonplanar_count(self) -> int:
+        """env-steps the planar kernel handed to the 3D safe kernel for not being planar (sr_nonplanar_count; synchronises)."""
+        return int(self._lib.sr_nonplanar_count(self._h))
 
     # -- device-pointer entry points (torch tensors on self.device) -----------
     @staticmethod

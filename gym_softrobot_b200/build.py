@@ -25,6 +25,7 @@ NVCC_FLAGS = [
     "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
 ]
 LEAN_EXTRA_SIZES = [(160, 3), (320, 2)]   # experimental CTA shapes of the lean kernel (SOFTROD_LEAN_THREADS)
+PLANAR_SIZES = [(256, 2), (384, 1), (512, 1)]   # the planar variant (CVAR 8) at the lean kernel's CTA sizes for rods of <= 511 elements
 PACKED_SIZES = [(256, 2), (384, 1), (512, 1), (544, 1), (768, 1), (1024, 1)]   # (threads per CTA, CTAs per SM)
 
 
@@ -39,6 +40,9 @@ def translation_units():
         for cv in (1, 2, 3, 4, 5):
             tus.append((f"leanc{cv}_double_{nt}", "inst_lean.cu", ["-DSR_TU_T=double", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", f"-DSR_TU_CONTACT={cv}"],
                         _COMMON + ["rod_kernel_lean.cuh"]))
+    for nt, minb in PLANAR_SIZES:     # variant 0 for rods in the x-y plane (fast-only kernel; FP64)
+        tus.append((f"leanc8_double_{nt}_{minb}", "inst_lean.cu", ["-DSR_TU_T=double", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", "-DSR_TU_CONTACT=8"],
+                    _COMMON + ["rod_kernel_lean.cuh"]))
     for cv in (6, 7):     # plain / contact variant with the tip node folded into the last element's thread (n_elem = 512)
         tus.append((f"leanc{cv}_double_512", "inst_lean.cu", ["-DSR_TU_T=double", "-DSR_TU_NT=512", "-DSR_TU_MINB=1", f"-DSR_TU_CONTACT={cv}"],
                     _COMMON + ["rod_kernel_lean.cuh"]))

@@ -1,5 +1,5 @@
 // inst_lean.cu — the lean kernel (rod_kernel_lean.cuh) for one storage type and CTA size:
-//   -DSR_TU_T=double|float -DSR_TU_NT=<threads> -DSR_TU_MINB=<n> [-DSR_TU_CONTACT=1|2|3|4: contact variant without / with the muscle wave / for assemblies; 4: filter + moving base; 5: spline torques; 6 / 7: variants 0 / 1 with the tip node folded into the last thread; FP64 only]
+//   -DSR_TU_T=double|float -DSR_TU_NT=<threads> -DSR_TU_MINB=<n> [-DSR_TU_CONTACT=1|2|3|4: contact variant without / with the muscle wave / for assemblies; 4: filter + moving base; 5: spline torques; 6 / 7: variants 0 / 1 with the tip node folded into the last thread; 8: variant 0 in the x-y plane, fast-only kernel only; FP64 only]
 #include <atomic>
 #include "launch.cuh"
 #include "rod_kernel_lean.cuh"
@@ -41,8 +41,10 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT> int lean_cta
 #define SR_TU_CONTACT 0
 #endif
 template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, SR_TU_CONTACT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
-template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, SR_TU_CONTACT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
 template int lean_ctas_per_sm<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, SR_TU_CONTACT>();
+#if SR_TU_CONTACT != 8   // (the planar variant's fallback is variant 0's safe kernel)
+template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, SR_TU_CONTACT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
 template int lean_ctas_per_sm<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, SR_TU_CONTACT>();
+#endif
 
 }  // namespace sr

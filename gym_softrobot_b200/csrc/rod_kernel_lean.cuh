@@ -2,7 +2,8 @@
 // FP32 storage, single rod per env, no contact / filter / joints / forcing (SoftPendulum-v0 and plain rods: BASELINE
 // configs 2 and 3).  Variants 1-7 put the other models on the same skeleton (see the comment at the kernel):
 // 1 plane contact + rest curvature, 2 + travelling-wave muscle, 3 assemblies (arms + rigid head + joints), 4 Laplace
-// filter + moving base, 5 spline muscle torques, 6 / 7 = 0 / 1 with the tip node folded into the last thread.
+// filter + moving base, 5 spline muscle torques, 6 / 7 = 0 / 1 with the tip node folded into the last thread, 8 = 0 for
+// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits).
 //
 // Same mapping as rod_kernel_packed.cuh (one thread per node/element, rods packed back to back across a
 // 256-thread CTA, state in registers for the whole launch, neighbour data through array-of-structures
@@ -83,6 +84,22 @@ __device__ __forceinline__ void rotate_directors_lean(const double (&cg)[3], con
   for (int i = 0; i < 9; i++) Q[i] = nq[i];
 }
 
+// rotate_directors_lean for a rod in the lab x-y plane (variant 8): the rotation vector is (0, a1, 0) about d2 = +-z, and
+// only d1 = (Q0, Q1, 0) and d3 = (Q6, Q7, 0) move.  The same terms as above in the same order, with the ones that carry
+// an exact zero factor left out (D = [[-B a1^2, 0, -A a1], [0, 0, 0], [A a1, 0, -B a1^2]]): the same roundings.
+__device__ __forceinline__ void rotate_directors_planar(const double (&cg)[3], const double (&ch)[3], double a1, double q,
+                                                        double eps, double (&Q)[9]) {
+  const double d = eps * rcp_approx(fma(q, rsqrt_approx(q), eps));
+  double pa = fma(cg[2], q, cg[1]), pb = fma(ch[2], q, ch[1]);
+  pa = fma(pa, q, cg[0]); pb = fma(pb, q, ch[0]);
+  const double A1 = fma(pa, q, 1.0), B = fma(pb, q, 0.5);
+  const double A = fma(-A1, d, A1);
+  const double Aa1 = A * a1, Ba11 = (B * a1) * a1;
+  const double q0 = fma(-Aa1, Q[6], fma(-Ba11, Q[0], Q[0])), q1 = fma(-Aa1, Q[7], fma(-Ba11, Q[1], Q[1]));
+  const double q6 = fma(-Ba11, Q[6], fma(Aa1, Q[0], Q[6])), q7 = fma(-Ba11, Q[7], fma(Aa1, Q[1], Q[7]));
+  Q[0] = q0; Q[1] = q1; Q[6] = q6; Q[7] = q7;
+}
+
 constexpr int LEAN_REC = 18;        // exchange record per thread (doubles), 144-byte stride: conflict-free LDS.128
 constexpr int LEAN_JREC = 10;      // assemblies: joint record of an arm's first thread {reaction force, couple on the head, couple on element 0, -}
 // filter variant: records of 6 doubles with 6 ghost records on either side of every rod (rods of >= 9 threads)
@@ -133,6 +150,15 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   // instead of a 544-thread one capped at 96 (17 warps put five on one scheduler).  One rod per CTA.
   constexpr bool FOLD = CVAR == 6 || CVAR == 7;
   constexpr bool CONTACT = (CVAR >= 1 && CVAR <= 3) || CVAR == 7, MUS = CVAR == 2, MULTI = CVAR == 3;
+  // 8: variant 0 for a rod that stays in the lab x-y plane (SoftPendulum-v0, planar clamped / free rods; the host checks
+  // gravity and the base force).  x_z, v_z, d1_z, d3_z, d2_x, d2_y, w_0, w_2, kappa_0, kappa_2 and sigma_1 are exact zeros
+  // at every substep, and every product that carries one of them is left out: the same terms in the same order, so the
+  // same roundings as variant 0 (up to the sign of zeros).  Nine state registers per thread instead of 18.  Each segment
+  // checks those zeros in its input (and the padding of slot n: Q = I, w = 0, which the stale observables of the last
+  // element and the tip assume); a rod that fails is flagged like a range failure (cause bit 8) and re-run by the 3D
+  // safe kernel.
+  constexpr bool PLANAR = CVAR == 8;
+  static_assert(!PLANAR || FASTONLY, "the planar variant is fast-only: its fallback is the 3D safe kernel");
   static_assert(CVAR == 0 || !MIXED, "the variants are FP64 only");
   static_assert(!FOLD || LEAN_SCR_FOLD >= 27, "hand-over rows of the folded tip");
   constexpr int SCR = FOLD ? LEAN_SCR_FOLD : CONTACT ? LEAN_SCR_CONTACT : LEAN_REC;   // rows of a slot's hand-over scratch
@@ -216,6 +242,14 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   const D c_dt = MIXED ? A.k_dt : (D)A.dt, c_half_dt = MIXED ? A.k_half_dt : (D)A.half_dt;
   const D c_cv = MIXED ? A.k_c_v : (D)A.c_v;
 
+  // redo_count: [0] env-steps handed over for leaving the fast-math range, [1..3] by cause (an env can count under
+  // several); [4] env-steps the planar variant handed over for not being planar (no range failure)
+  auto count_redo = [&](int dom) {
+    if (PLANAR && (dom & 8)) { atomicAdd(A.redo_count + 4, 1ULL); return; }
+    atomicAdd(A.redo_count, 1ULL);
+    for (int b = 0; b < 3; b++) if (dom >> b & 1) atomicAdd(A.redo_count + 1 + b, 1ULL);
+  };
+
   // ---- the segments this CTA runs ------------------------------------------------------------------------------
   const int K = A.n_substeps;
   const int P = gridDim.x, p = blockIdx.x;
@@ -279,10 +313,15 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       }
       __syncthreads();
       const D *sc = A.sk_scratch + (size_t)(p - 1) * SCR * NT;
+      if constexpr (PLANAR) {   // rows: x0 x1 v0 v1 w1 Q0 Q1 Q6 Q7
+        x[0] = sc[tid]; x[1] = sc[NT + tid]; v[0] = sc[2 * NT + tid]; v[1] = sc[3 * NT + tid]; w[1] = sc[4 * NT + tid];
+        Q[0] = sc[5 * NT + tid]; Q[1] = sc[6 * NT + tid]; Q[6] = sc[7 * NT + tid]; Q[7] = sc[8 * NT + tid];
+      } else {
 #pragma unroll
-      for (int c = 0; c < 3; c++) { x[c] = sc[c * NT + tid]; v[c] = sc[(3 + c) * NT + tid]; w[c] = sc[(15 + c) * NT + tid]; }
+        for (int c = 0; c < 3; c++) { x[c] = sc[c * NT + tid]; v[c] = sc[(3 + c) * NT + tid]; w[c] = sc[(15 + c) * NT + tid]; }
 #pragma unroll
-      for (int c = 0; c < 9; c++) Q[c] = sc[(6 + c) * NT + tid];
+        for (int c = 0; c < 9; c++) Q[c] = sc[(6 + c) * NT + tid];
+      }
       if (CONTACT) { mus_S = sc[18 * NT + tid]; mus_C = sc[19 * NT + tid]; mus_t = sc[20 * NT + tid]; }
       if (FOLD) {
 #pragma unroll
@@ -291,7 +330,13 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       __syncthreads();
       if (tid == 0) A.sk_flag[p - 1] = 0;   // (graph-safe: the flag is back to 0 before the launch ends)
     } else {
-      if (active) {
+      if (PLANAR && active) {
+        x[0] = (D)st[F_POS * stride + j]; x[1] = (D)st[(F_POS + 1) * stride + j];
+        v[0] = (D)st[F_VEL * stride + j]; v[1] = (D)st[(F_VEL + 1) * stride + j];
+        w[1] = (D)st[(F_OMEGA + 1) * stride + j];
+        Q[0] = (D)st[F_DIR * stride + j]; Q[1] = (D)st[(F_DIR + 1) * stride + j];
+        Q[6] = (D)st[(F_DIR + 6) * stride + j]; Q[7] = (D)st[(F_DIR + 7) * stride + j];
+      } else if (active) {
 #pragma unroll
         for (int c = 0; c < 3; c++) {
           x[c] = (D)st[(F_POS + c) * stride + j];
@@ -346,7 +391,29 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // BCs pin node 0 / element 0 by overwriting after every kinematic update; applying the overwrite once and
     // never moving the pinned quantities is the same thing (see rod_kernel_packed.cuh): the BC thread integrates its
     // frame with a zero rotation vector
-    if (bc_thread) {
+    if constexpr (PLANAR) {
+      // the zeros this variant relies on, in the pre-launch state (the same for every segment of an item)
+      if (active) {
+        auto f = [&](int field) { return (D)st[field * stride + j]; };
+        bool flat = f(F_POS + 2) == D(0) && f(F_VEL + 2) == D(0);
+        if (j < n)
+          flat = flat && f(F_DIR + 2) == D(0) && f(F_DIR + 3) == D(0) && f(F_DIR + 4) == D(0) && f(F_DIR + 8) == D(0) &&
+                 f(F_OMEGA) == D(0) && f(F_OMEGA + 2) == D(0);
+        else      // slot n: the padding
+          flat = flat && f(F_DIR) == D(1) && f(F_DIR + 1) == D(0) && f(F_DIR + 2) == D(0) && f(F_DIR + 3) == D(0) &&
+                 f(F_DIR + 4) == D(1) && f(F_DIR + 5) == D(0) && f(F_DIR + 6) == D(0) && f(F_DIR + 7) == D(0) &&
+                 f(F_DIR + 8) == D(1) && f(F_OMEGA) == D(0) && f(F_OMEGA + 1) == D(0) && f(F_OMEGA + 2) == D(0);
+        if (bc_thread)
+          flat = flat && (D)bc[2] == D(0) && (D)bc[5] == D(0) && (D)bc[11] == D(0) &&
+                 (A.bc_kind == BC_PENDULUM_SLIDER || ((D)bc[6] == D(0) && (D)bc[7] == D(0)));
+        if (!flat) dom_bad |= 8;
+      }
+      if (bc_thread) {
+        if (A.bc_kind != BC_PENDULUM_SLIDER) x[0] = (D)bc[0];
+        x[1] = (D)bc[1];
+        Q[0] = (D)bc[3]; Q[1] = (D)bc[4]; Q[6] = (D)bc[9]; Q[7] = (D)bc[10];
+      }
+    } else if (bc_thread) {
       if (A.bc_kind == BC_PENDULUM_SLIDER) {
         x[1] = (D)bc[1]; x[2] = (D)bc[2];
 #pragma unroll
@@ -448,6 +515,14 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // x += hh v ; Q <- R(hh w) Q (merged half steps)
     auto kinematic = [&](D hh, D eps) {
       const D hw = bc_thread ? D(0) : hh;
+      if constexpr (PLANAR) {
+        const D a1 = hw * w[1];
+        x[0] = fma(hh, v[0], x[0]); x[1] = fma(hh, v[1], x[1]);
+        const D q = fma(a1, a1, D(1e-300));
+        if (hi_abs(q) > A.lim_rot_hi) dom_bad |= 1;
+        rotate_directors_planar(A.sincg, A.cosch, a1, q, eps, Q);
+        return;
+      }
       D a0 = hw * w[0], a1 = hw * w[1], a2 = hw * w[2];
 #pragma unroll
       for (int c = 0; c < 3; c++) x[c] = fma(hh, v[c], x[c]);
@@ -1105,12 +1180,139 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       kinematic(last ? c_half_dt : c_dt, last ? D(1e-14) : D(2e-14));
       head_constrain_values();
     };
+    // variant 8: the substep above with the out-of-plane terms left out (see PLANAR).  Records {x0 x1 | v0 v1 | Q0 Q1 |
+    // Q6 Q7} and {s0 s1 | N1}.  The pseudo-element of the tip / idle threads lies along x here instead of z (same
+    // length; its stress is discarded either way), so the tip's stale observables are rebuilt in the last substep.
+    auto substep_planar = [&](auto last_tag) {
+      constexpr bool last = decltype(last_tag)::value;
+      {
+        double2 *o = reinterpret_cast<double2 *>(rec + LEAN_REC * tid);
+        o[0] = make_double2(x[0], x[1]); o[1] = make_double2(v[0], v[1]);
+        o[2] = make_double2(Q[0], Q[1]); o[3] = make_double2(Q[6], Q[7]);
+      }
+      rod_sync();
+      D dx0, dx1, dv0, dv1, dn0, dn1, Qn0, Qn1, Qn6, Qn7;
+      {
+        const double2 *qq = reinterpret_cast<const double2 *>(rec + LEAN_REC * t_next);
+        const double2 a0 = qq[0], a1 = qq[1], a2 = qq[2], a3 = qq[3];
+        const double2 b0 = *reinterpret_cast<const double2 *>(rec + LEAN_REC * t_next2);
+        Qn0 = a2.x; Qn1 = a2.y; Qn6 = a3.x; Qn7 = a3.y;
+        dx0 = a0.x - x[0]; dx1 = a0.y - x[1]; dv0 = a1.x - v[0]; dv1 = a1.y - v[1];
+        dn0 = b0.x - a0.x; dn1 = b0.y - a0.y;
+      }
+      if (!elem_ok) dx0 = (D)A.rest_len;
+      if (!vor_ok) dn0 = (D)A.rest_len;
+      const D l2 = fma(dx1, dx1, dx0 * dx0), l2n = fma(dn1, dn1, dn0 * dn0);
+      const D il = rsqrt_nr(l2), iln = rsqrt_nr(l2n);
+      const D lg = fma(l2, il, D(1e-14));
+      const D ilg = fma(D(-1e-14) * il, il, il);
+      const D lgn = fma(l2n, iln, D(1e-14));
+      const D e = lg * irg;
+      const D em1 = fma(lg, irg, D(-1.0));
+      const D inv_e = A.rest_len * ilg;
+      const D inv_e_s = elem_ok ? inv_e : D(0);
+      const D ede = fma(dx1, dv1, dx0 * dv0) * (ilg * ilg);
+      const D Qdx0 = fma(Q[1], dx1, Q[0] * dx0), Qdx2 = fma(Q[7], dx1, Q[6] * dx0);   // Q dx = (Qdx0, 0, Qdx2)
+      const D s3 = fma(Qdx2, irg, D(-1.0));
+      const D n0 = A.S_over_l[0] * Qdx0;
+      const D n2 = fma((D)A.S[2], Qdx2 * irg, -(D)A.S[2]);
+      const D sf0 = fma(Q[6], n2, Q[0] * n0) * inv_e_s, sf1 = fma(Q[7], n2, Q[1] * n0) * inv_e_s;
+      // curvature: axial(Qn Q^T - Q Qn^T) = (0, vec1, 0)
+      const D vec1 = fma(-Qn7, Q[1], fma(-Qn6, Q[0], fma(Qn1, Q[7], Qn0 * Q[6])));
+      D w2 = vec1 * vec1;
+      if (!vor_ok) w2 = D(0);
+      bool bend_out = out_of_range(w2, A.lim_bend_hi, A.limf_bend);
+      if (check_trace) {
+        check_trace = false;
+        if (vor_ok) {
+          // d2 = (0, 0, d2z) of this element and the next: invariant under in-plane rotations, read from the
+          // pre-launch state (the clamp's from its anchor)
+          const D z_own = pin_fixed ? (D)bc[8] : (D)st[(F_DIR + 5) * stride + j], z_next = (D)st[(F_DIR + 5) * stride + j + 1];
+          const D tr = fma(Qn7, Q[7], fma(Qn6, Q[6], fma(z_next, z_own, fma(Qn1, Q[1], Qn0 * Q[0]))));
+          bend_out = bend_out || !(tr > D(2.0));
+        }
+      }
+      if (bend_out) dom_bad |= 2;
+      D fs;
+      {
+        D c[10];
+#pragma unroll
+        for (int k = 0; k < 10; k++) c[k] = (D)A.bendw[k];   // (F = D here)
+        const D z = w2 * w2;
+        D pe = fma(c[8], z, c[6]), po = fma(c[9], z, c[7]);
+        pe = fma(pe, z, c[4]); po = fma(po, z, c[5]);
+        pe = fma(pe, z, c[2]); po = fma(po, z, c[3]);
+        pe = fma(pe, z, c[0]); po = fma(po, z, c[1]);
+        fs = fma(po, w2, pe);
+      }
+      const D kp1 = vec1 * fs;
+      const D tau1 = A.B[0] * kp1;
+      const D eps_v = (lgn + lg) * A.half_inv_rest_vor;
+      D ie3 = rcp_nr(eps_v * eps_v * eps_v);
+      if (!vor_ok) ie3 = D(0);
+      const D m1 = tau1 * ie3;
+      const D cc = fma(-(D)A.S_over_l[0], Qdx2, n2);
+      const D je = ede * A.J[0];
+      const D h1 = fma(-Qdx0, cc, je * w[1]);
+      const D tql1 = fma(h1, inv_e, m1);
+      {
+        double2 *o = reinterpret_cast<double2 *>(sn + SNR * tid);
+        o[0] = make_double2(sf0, sf1);
+        sn[SNR * tid + 2] = -m1;
+      }
+      D cw0;
+      {
+        if (out_of_range(em1, A.lim_em1_hi, A.limf_em1) && elem_ok) dom_bad |= 4;
+        cw0 = fma(fma((D)A.cwp[0][2], em1, (D)A.cwp[0][1]), em1, (D)A.cwp[0][0]);
+      }
+      if (last && active) {
+        // stale observables, as variant 0 computes them.  Its tip thread holds Q = I and the edge (0, 0, l0); its
+        // last element forms the curvature against that I: axial(I Q^T - Q) = (d2z - Q7, Q6, Q1).
+        D tg[3] = {dx0 * ilg, dx1 * ilg, D(0)}, kp[3] = {D(0), kp1, D(0)};
+        D sg0 = Qdx0 * irg, sg2 = s3;
+        if (j == n) {
+          tg[0] = D(0); tg[2] = dx0 * ilg; kp[1] = D(0); sg0 = D(0); sg2 = fma(Qdx0, irg, D(-1.0));
+        } else if (j == n - 1) {
+          const D z_own = pin_fixed ? (D)bc[8] : (D)st[(F_DIR + 5) * stride + j];
+          kp[0] = (z_own - Q[7]) * fs; kp[2] = Q[1] * fs;
+        }
+#pragma unroll
+        for (int i = 0; i < 3; i++) {
+          st[(F_TAN + i) * stride + j] = (ST)tg[i];
+          st[(F_KAPPA + i) * stride + j] = (ST)kp[i];
+        }
+        st[F_SIGMA * stride + j] = (ST)sg0;
+        st[(F_SIGMA + 1) * stride + j] = ST(0);
+        st[(F_SIGMA + 2) * stride + j] = (ST)sg2;
+        st[F_DIL * stride + j] = (ST)e;
+      }
+      rod_sync();
+      D f0, f1, tq1;
+      {
+        const double2 l = *reinterpret_cast<const double2 *>(sn + SNR * t_prev);
+        f0 = sf0 - l.x; f1 = sf1 - l.y; tq1 = tql1 + sn[SNR * t_prev + 2];
+      }
+      v[0] = fma(f0, dtim_cv, fma(v[0], c_cv, base0));
+      v[1] = fma(f1, dtim_cv, fma(v[1], c_cv, (D)A.gdt_cv[1]));
+      {
+        const D g = elem_ok ? e * A.dt_Jinv0 : D(0);
+        w[1] = fma(g, tq1, w[1]) * cw0;
+      }
+      v[0] = pin_fixed ? D(0) : v[0]; v[1] = z12 ? D(0) : v[1]; w[1] = pin_fixed ? D(0) : w[1];
+      kinematic(last ? c_half_dt : c_dt, last ? D(1e-14) : D(2e-14));
+    };
     // the item's last substep ends with a half kinematic step and exports the stale observables: its own copy of the
     // body, so that the loop carries neither the selects nor the branch
     const int s_loop_end = (s_end == K) ? K - 1 : s_end;
+    if constexpr (PLANAR) {
 #pragma unroll 1
-    for (int s = s_begin; s < s_loop_end; s++) substep(std::false_type{}, s);
-    if (s_end == K && s_begin < K) substep(std::true_type{}, K - 1);
+      for (int s = s_begin; s < s_loop_end; s++) substep_planar(std::false_type{});
+      if (s_end == K && s_begin < K) substep_planar(std::true_type{});
+    } else {
+#pragma unroll 1
+      for (int s = s_begin; s < s_loop_end; s++) substep(std::false_type{}, s);
+      if (s_end == K && s_begin < K) substep(std::true_type{}, K - 1);
+    }
 
     __syncthreads();   // all reads of the exchange buffers are done
     if (s_end < K) {
@@ -1120,16 +1322,18 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         __syncthreads();
         if (live && dom_bad) atomicOr(&sh_dom[r], dom_bad);
         __syncthreads();
-        if (active && lead && sh_dom[r] != 0 && atomicExch(&A.redo[env], 1) == 0 && A.redo_count) {
-          atomicAdd(A.redo_count, 1ULL);
-          for (int b = 0; b < 3; b++) if (sh_dom[r] >> b & 1) atomicAdd(A.redo_count + 1 + b, 1ULL);
-        }
+        if (active && lead && sh_dom[r] != 0 && atomicExch(&A.redo[env], 1) == 0 && A.redo_count) count_redo(sh_dom[r]);
       }
       D *sc = A.sk_scratch + (size_t)p * SCR * NT;
+      if constexpr (PLANAR) {
+        sc[tid] = x[0]; sc[NT + tid] = x[1]; sc[2 * NT + tid] = v[0]; sc[3 * NT + tid] = v[1]; sc[4 * NT + tid] = w[1];
+        sc[5 * NT + tid] = Q[0]; sc[6 * NT + tid] = Q[1]; sc[7 * NT + tid] = Q[6]; sc[8 * NT + tid] = Q[7];
+      } else {
 #pragma unroll
-      for (int c = 0; c < 3; c++) { sc[c * NT + tid] = x[c]; sc[(3 + c) * NT + tid] = v[c]; sc[(15 + c) * NT + tid] = w[c]; }
+        for (int c = 0; c < 3; c++) { sc[c * NT + tid] = x[c]; sc[(3 + c) * NT + tid] = v[c]; sc[(15 + c) * NT + tid] = w[c]; }
 #pragma unroll
-      for (int c = 0; c < 9; c++) sc[(6 + c) * NT + tid] = Q[c];
+        for (int c = 0; c < 9; c++) sc[(6 + c) * NT + tid] = Q[c];
+      }
       if (CONTACT) { sc[18 * NT + tid] = mus_S; sc[19 * NT + tid] = mus_C; sc[20 * NT + tid] = mus_t; }
       if (FOLD) {
 #pragma unroll
@@ -1150,10 +1354,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       __syncthreads();
       // (a part of this item run by the previous slot may have flagged the env already)
       redo = live && (sh_dom[r] != 0 || A.redo[env] != 0);
-      if (redo && lead && atomicExch(&A.redo[env], 1) == 0 && A.redo_count) {
-        atomicAdd(A.redo_count, 1ULL);     // [0] env-steps handed over, [1..3] by cause (an env can count under several)
-        for (int b = 0; b < 3; b++) if (sh_dom[r] >> b & 1) atomicAdd(A.redo_count + 1 + b, 1ULL);
-      }
+      if (redo && lead && atomicExch(&A.redo[env], 1) == 0 && A.redo_count) count_redo(sh_dom[r]);
     }
     constexpr int RS = NT + 2;
     if (MIXED) {       // edge vectors of the final FP64 positions: the strain state the next launch starts from
@@ -1175,7 +1376,19 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       float *o = A.obs + (size_t)env * A.obs_dim;
       for (int c = 0; c < 3; c++) { o[c] = (float)x[c]; o[3 + c] = (float)v[c]; }
     }
-    if (active && !redo) {
+    if (PLANAR && active && !redo) {   // the out-of-plane fields keep their zeros (the clamp's d2z is its anchor's)
+      for (int c = 0; c < 2; c++) {
+        st[(F_POS + c) * stride + j] = (ST)x[c];
+        st[(F_VEL + c) * stride + j] = (ST)v[c];
+        bad = bad || (x[c] != x[c]) || (v[c] != v[c]);
+      }
+      if (j < n) {
+        st[(F_OMEGA + 1) * stride + j] = (ST)w[1];
+        st[F_DIR * stride + j] = (ST)Q[0]; st[(F_DIR + 1) * stride + j] = (ST)Q[1];
+        st[(F_DIR + 6) * stride + j] = (ST)Q[6]; st[(F_DIR + 7) * stride + j] = (ST)Q[7];
+        if (pin_fixed) st[(F_DIR + 5) * stride + j] = bc[8];
+      }
+    } else if (active && !redo) {
       if (CONTACT) { to_lab(x); to_lab(v); rows_to_lab(Q); }   // (final: nothing below reads them in the internal frame)
 #pragma unroll
       for (int c = 0; c < 3; c++) {

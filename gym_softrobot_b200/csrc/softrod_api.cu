@@ -53,9 +53,10 @@ struct sr_handle {
   double *mus_act = nullptr;       // per-element activations of the three muscle layers [n_rods][3][n_elem]
   double *msucker = nullptr;       // ratios of the fixed-index ControllableFixConstraints [n_rods][3]
   int *redo = nullptr;   // per-env flags of the fast-only / fallback kernel pair
-  unsigned long long *redo_count = nullptr, *h_redo_count = nullptr, pair_last_count = 0;
+  unsigned long long *redo_count = nullptr, *h_redo_count = nullptr, pair_last_count = 0;   // counts: see count_redo (lean kernel)
   cudaEvent_t pair_event = nullptr; bool pair_copy_pending = false;
   long long pair_steps = 0, pair_off_until = 0, pair_steps_at_copy = 0, pair_steps_at_prev_copy = 0;
+  unsigned long long planar_last_count = 0; long long planar_off_until = 0;   // the planar variant's own window
   int n_rod = 1, init_dim = 9;
   sr::RodArgs<double> a64;
   sr::RodArgs<float> a32;
@@ -66,8 +67,8 @@ struct sr_handle {
   int32_t *d_idx = nullptr;
   cudaStream_t own_stream = nullptr;
   int64_t launches = 0;
-  // stream-K schedule of the lean kernel: resident CTA slots, hand-over scratch and flags
-  int sk_slots = 0; void *sk_scratch = nullptr; int *sk_flag = nullptr;
+  // stream-K schedule of the lean kernel: SM count, slots the hand-over scratch and flags are allocated for
+  int sk_sms = 0, sk_slots = 0; void *sk_scratch = nullptr; int *sk_flag = nullptr;
 };
 
 namespace {
@@ -273,14 +274,18 @@ template <typename T> bool use_fast_pair(sr_handle *h, sr::RodArgs<T> &A, cudaSt
   if (h->pair_copy_pending && q == cudaErrorNotReady) (void)cudaGetLastError();   // "not ready" is an answer, not an error to report later
   if (h->pair_copy_pending && q == cudaSuccess) {
     h->pair_copy_pending = false;
-    const unsigned long long seen = *h->h_redo_count, delta = seen - h->pair_last_count;
+    const unsigned long long seen = h->h_redo_count[0], delta = seen - h->pair_last_count;
+    const unsigned long long seen_np = h->h_redo_count[4], delta_np = seen_np - h->planar_last_count;
     const long long window = (h->pair_steps_at_copy - h->pair_steps_at_prev_copy) * (long long)A.n_env;
     h->pair_last_count = seen;
+    h->planar_last_count = seen_np;
     h->pair_steps_at_prev_copy = h->pair_steps_at_copy;
+    // the same rule for envs that are not planar: the handle steps with the 3D pair for a while (see use_planar)
+    if (window > 0 && (double)delta_np > 0.01 * (double)window) h->planar_off_until = h->pair_steps + 512;
     if (window > 0 && (double)delta > 0.01 * (double)window) { h->pair_off_until = h->pair_steps + 512; return false; }
   }
   if (!h->pair_copy_pending && h->pair_steps % 8 == 0) {
-    cudaMemcpyAsync(h->h_redo_count, h->redo_count, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(h->h_redo_count, h->redo_count, 5 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s);
     cudaEventRecord(h->pair_event, s);
     h->pair_copy_pending = true;
     h->pair_steps_at_copy = h->pair_steps;
@@ -312,32 +317,63 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int laun
   const int rods_per_cta = NT / group;   // env groups per CTA
   if (rods_per_cta < 1) return fail(SR_E_INVALID, "environment does not fit one CTA of the lean kernel");
   const int items = (A.n_env + rods_per_cta - 1) / rods_per_cta;
-  if (h->sk_slots == 0) {
+  // resident CTAs per SM of this kernel (a property of the kernel and the device model: asked once); the slot count
+  // differs between the kernels of a handle, the scratch is sized for the largest
+  static int ctas_per_sm = 0;
+  if (ctas_per_sm == 0) ctas_per_sm = sr::lean_ctas_per_sm<T, NT, MINB, FASTONLY, CONTACT>();
+  if (ctas_per_sm < 1) return fail(SR_E_CUDA, "lean kernel: occupancy query failed");
+  if (h->sk_sms == 0) {
     cudaDeviceProp prop;
     SR_CUDA(cudaGetDeviceProperties(&prop, h->cfg.device));
-    // both variants of a pair are sized alike (same launch bounds); take the smaller answer to be safe
-    const int a = sr::lean_ctas_per_sm<T, NT, MINB, true, CONTACT>(), b = sr::lean_ctas_per_sm<T, NT, MINB, false, CONTACT>();
-    h->sk_slots = prop.multiProcessorCount * (a < b ? a : b);
-    if (h->sk_slots < 1) return fail(SR_E_CUDA, "lean kernel: occupancy query failed");
-    SR_CUDA(cudaMalloc(&h->sk_scratch, (size_t)h->sk_slots * sr::LEAN_SCR_FOLD * NT * sizeof(double)));
-    SR_CUDA(cudaMalloc(&h->sk_flag, (size_t)h->sk_slots * sizeof(int)));
-    SR_CUDA(cudaMemset(h->sk_flag, 0, (size_t)h->sk_slots * sizeof(int)));
+    h->sk_sms = prop.multiProcessorCount;
+  }
+  const int slots = h->sk_sms * ctas_per_sm;
+  if (slots > h->sk_slots) {
+    cudaFree(h->sk_scratch); cudaFree(h->sk_flag);
+    h->sk_scratch = nullptr; h->sk_flag = nullptr; h->sk_slots = 0;
+    SR_CUDA(cudaMalloc(&h->sk_scratch, (size_t)slots * sr::LEAN_SCR_FOLD * NT * sizeof(double)));
+    SR_CUDA(cudaMalloc(&h->sk_flag, (size_t)slots * sizeof(int)));
+    SR_CUDA(cudaMemset(h->sk_flag, 0, (size_t)slots * sizeof(int)));
+    h->sk_slots = slots;
   }
   A.sk_rods_per_cta = rods_per_cta; A.sk_items = items;
-  A.sk_split = (streamk_setting() && !A.redo_filter && items > h->sk_slots && A.n_substeps > 0) ? 1 : 0;
+  A.sk_split = (streamk_setting() && !A.redo_filter && items > slots && A.n_substeps > 0) ? 1 : 0;
   A.sk_scratch = (double *)h->sk_scratch; A.sk_flag = h->sk_flag;
   A.sk_rodsync = rodsync_setting();
-  const int grid = A.sk_split ? h->sk_slots : items;
+  const int grid = A.sk_split ? slots : items;
   cudaError_t e = sr::launch_lean_kernel<T, NT, MINB, FASTONLY, CONTACT>(A, grid, s);
   h->launches++;
   if (e != cudaSuccess) return cuda_fail("rod_lean_kernel launch", e);
   return SR_OK;
 }
 
+int planar_setting() {     // SOFTROD_LEAN_PLANAR=0: rods in the x-y plane take the 3D kernels too (A/B; same bits)
+  static int v = -1;
+  if (v < 0) { const char *e = getenv("SOFTROD_LEAN_PLANAR"); v = e ? atoi(e) != 0 : 1; }
+  return v;
+}
+
+// Whether the fast-only kernel of a pair may be the planar variant (CVAR 8).  It needs a model whose out-of-plane
+// components stay exact zeros once the state has them: the plain lean model in FP64 with the fast maps, gravity in the
+// x-y plane, the base point force along x (the only direction the kernel applies it in), and a BC that pins in-plane
+// rows (slider, clamp) or none.  The state itself is checked by the kernel, per rod; when more than 1 % of a window's
+// env-steps are handed over for not being planar, the handle uses the 3D pair for the next 512 steps (use_fast_pair).
+template <typename T> bool is_lean_config(const sr::RodArgs<T> &A);
+template <typename T> bool use_planar(const sr_handle *h, const sr::RodArgs<T> &A) {
+  if (!std::is_same<T, double>::value || !planar_setting() || !is_lean_config(A)) return false;
+  if (h->cfg.math != SR_MATH_FAST || (double)A.gdt_cv[2] != 0.0) return false;
+  if (A.bc_kind != sr::BC_FREE && A.bc_kind != sr::BC_ONE_END_FIXED && A.bc_kind != sr::BC_PENDULUM_SLIDER) return false;
+  return h->pair_steps >= h->planar_off_until;
+}
+
 template <typename T, int NT, int MINB, int CONTACT = 0> int launch_lean_pair(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
   if (use_fast_pair(h, A, s)) {
     // fast-only kernel, then the safe one over the envs it flagged (an empty launch in the normal case)
-    int rc = launch_lean_impl<T, NT, MINB, true, CONTACT>(h, A, s);
+    int rc;
+    if constexpr (std::is_same<T, double>::value && CONTACT == 0 && NT <= 512 && NT % 128 == 0)
+      rc = use_planar(h, A) ? launch_lean_impl<T, NT, MINB, true, 8>(h, A, s) : launch_lean_impl<T, NT, MINB, true, CONTACT>(h, A, s);
+    else
+      rc = launch_lean_impl<T, NT, MINB, true, CONTACT>(h, A, s);
     if (rc != SR_OK) return rc;
     A.redo_filter = 1;
   }
@@ -760,9 +796,9 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
       (e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking)) != cudaSuccess ||
       (e = cudaMalloc(&h->redo, n_env * sizeof(int))) != cudaSuccess ||
       (e = cudaMemset(h->redo, 0, n_env * sizeof(int))) != cudaSuccess ||
-      (e = cudaMalloc(&h->redo_count, 4 * sizeof(unsigned long long))) != cudaSuccess ||     // [0] total, [1..3] by cause (lean kernel)
-      (e = cudaMemset(h->redo_count, 0, 4 * sizeof(unsigned long long))) != cudaSuccess ||
-      (e = cudaMallocHost(&h->h_redo_count, sizeof(unsigned long long))) != cudaSuccess ||
+      (e = cudaMalloc(&h->redo_count, 5 * sizeof(unsigned long long))) != cudaSuccess ||     // [0] total, [1..3] by cause, [4] not planar (lean kernel)
+      (e = cudaMemset(h->redo_count, 0, 5 * sizeof(unsigned long long))) != cudaSuccess ||
+      (e = cudaMallocHost(&h->h_redo_count, 5 * sizeof(unsigned long long))) != cudaSuccess ||
       (e = cudaEventCreateWithFlags(&h->pair_event, cudaEventDisableTiming)) != cudaSuccess ||
       (e = cudaMemset(h->state, 0, state_bytes)) != cudaSuccess) {
     std::string m = std::string("sr_create: allocation failed: ") + cudaGetErrorString(e);
@@ -879,7 +915,7 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
       return fail(SR_E_ALLOC, m);
     }
   }
-  *h->h_redo_count = 0;
+  for (int i = 0; i < 5; i++) h->h_redo_count[i] = 0;
   fill_args<double>(*cfg, h->stride, h->a64);
   h->a64.spline = h->spline; h->a64.spline_tab = h->spline_tab;
   h->a64.redo = h->redo;
@@ -922,8 +958,8 @@ int sr_obs_dim(const sr_handle *h) { return h ? h->obs_dim : 0; }
 int sr_action_dim(const sr_handle *h) { return h ? h->action_dim : 0; }
 int sr_init_dim(const sr_handle *h) { return h ? h->init_dim : 0; }
 int64_t sr_launch_count(const sr_handle *h) { return h ? h->launches : 0; }
-static void read_fallback_counters(const sr_handle *h, unsigned long long (&v)[4]) {
-  for (int i = 0; i < 4; i++) v[i] = 0;
+static void read_fallback_counters(const sr_handle *h, unsigned long long (&v)[5]) {
+  for (int i = 0; i < 5; i++) v[i] = 0;
   if (!h || !h->redo_count) return;
   int prev = 0;
   cudaGetDevice(&prev); cudaSetDevice(h->cfg.device);
@@ -932,16 +968,21 @@ static void read_fallback_counters(const sr_handle *h, unsigned long long (&v)[4
   cudaSetDevice(prev);
 }
 int64_t sr_fallback_count(const sr_handle *h) {
-  unsigned long long v[4];
+  unsigned long long v[5];
   read_fallback_counters(h, v);
   return (int64_t)v[0];
 }
 int sr_fallback_causes(const sr_handle *h, int64_t out[3]) {
   if (!h || !out) return fail(SR_E_INVALID, "sr_fallback_causes: null argument");
-  unsigned long long v[4];
+  unsigned long long v[5];
   read_fallback_counters(h, v);
   for (int i = 0; i < 3; i++) out[i] = (int64_t)v[1 + i];
   return SR_OK;
+}
+int64_t sr_nonplanar_count(const sr_handle *h) {
+  unsigned long long v[5];
+  read_fallback_counters(h, v);
+  return (int64_t)v[4];
 }
 
 int sr_reset(sr_handle *h, const int32_t *env_idx_dev, int n, const double *init_dev, void *stream) {
