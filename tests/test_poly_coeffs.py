@@ -106,3 +106,18 @@ def test_lean_kernel_maps():
     assert np.abs(A / wantA - 1.0).max() < 1.5e-15 and np.abs(B / wantB - 1.0).max() < 6e-16
     # the damper's quadratic drops z^3 / 6
     assert const("kLeanExpZ") ** 3 / 6 < 1.5e-15
+    # the lean kernels test a range on the high 32 bits of the argument only (hi_abs(x) > lim_hi, rod_kernel_lean.cuh),
+    # so the polynomials also run on the largest double that shares the limit's high word (2^-20 relative beyond it)
+    q = top_of_high_word(const("kNarrowRotQ"))
+    assert abs(1.0 + q * horner(g, q) - float(SINC(mp.mpf(q)))) / float(SINC(mp.mpf(q))) < 1.5e-15
+    assert abs(0.5 + q * horner(h, q) - float(COSC(mp.mpf(q)))) / float(COSC(mp.mpf(q))) < 6e-16
+    w = top_of_high_word(hi)
+    assert abs(horner(c, w) / ref(w) - 1.0) < 8e-16
+    w = top_of_high_word(him)
+    assert abs(horner(cm, w) / ref(w) - 1.0) < 1.5e-15
+
+
+def top_of_high_word(x):
+    """The largest double whose high 32 bits are those of x (x > 0)."""
+    b = np.array([x]).view(np.uint64) | np.uint64(0xFFFFFFFF)
+    return float(b.view(np.float64)[0])
