@@ -3,7 +3,8 @@
 // configs 2 and 3).  Variants 1-7 put the other models on the same skeleton (see the comment at the kernel):
 // 1 plane contact + rest curvature, 2 + travelling-wave muscle, 3 assemblies (arms + rigid head + joints), 4 Laplace
 // filter + moving base, 5 spline muscle torques, 6 / 7 = 0 / 1 with the tip node folded into the last thread, 8 = 0 for
-// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits).
+// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits), 9 = 0 for rods of 512-4095 elements,
+// one rod per thread-block cluster of 2-8 CTAs (same substep, same bits).
 //
 // Same mapping as rod_kernel_packed.cuh (one thread per node/element, rods packed back to back across a
 // 256-thread CTA, state in registers for the whole launch, neighbour data through array-of-structures
@@ -35,6 +36,7 @@
 // Algorithm: SURVEY.md Appendix A.2/A.3; reference boundary
 // /root/reference/gym_softrobot/envs/soft_pendulum/soft_pendulum.py:183-184.
 #pragma once
+#include <cooperative_groups.h>
 #include <type_traits>
 #include "rod_kernels.cuh"
 
@@ -106,9 +108,18 @@ constexpr int LEAN_JREC = 10;      // assemblies: joint record of an arm's first
 // (8 ghost records per side, 6 used: a rod's records then start a multiple of 8 records = 96 words after where the
 // previous rod's would continue, so a quarter-warp that straddles two rods still hits eight distinct 4-bank groups)
 constexpr int lean_ghost_records(int nt) { return nt + 16 * (nt / 9) + 16; }
+// records of each exchange array beyond the NT threads' own: variant 9 has a halo record before thread 0, two after
+// thread NT - 1 and a zero record; the others a zero record and a spare one
+__host__ __device__ constexpr int lean_extra_records(int cvar) { return cvar == 9 ? 4 : 2; }
 constexpr int lean_smem_words(int nt, int cvar = 0) {
-  return (LEAN_REC + 6 + (cvar == 3 ? LEAN_JREC : 0)) * (nt + 2) + (cvar == 4 ? 6 * lean_ghost_records(nt) : 0);
+  return (LEAN_REC + 6 + (cvar == 3 ? LEAN_JREC : 0)) * (nt + lean_extra_records(cvar)) + (cvar == 4 ? 6 * lean_ghost_records(nt) : 0);
 }
+
+// variant 9: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
+template <typename T> __device__ __forceinline__ T *cluster_smem(T *p, int rank) {
+  return cooperative_groups::this_cluster().map_shared_rank(p, (unsigned)rank);
+}
+__device__ __forceinline__ void cluster_sync() { cooperative_groups::this_cluster().sync(); }
 
 // float overloads of the reciprocal helpers for the FP32 force evaluation of the mixed mode
 __device__ __forceinline__ bool out_of_range(double x, int lim_hi, float) { return hi_abs(x) > lim_hi; }
@@ -159,15 +170,27 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   // safe kernel.
   constexpr bool PLANAR = CVAR == 8;
   static_assert(!PLANAR || FASTONLY, "the planar variant is fast-only: its fallback is the 3D safe kernel");
+  // 9: variant 0 for a rod of 512-4095 elements spread over a thread-block cluster of C = ceil((n + 1) / NT) CTAs (one rod
+  // per cluster, launched with the cluster dimension set at run time): CTA rank c holds nodes / elements j = NT c + tid.
+  // The substep is variant 0's, instruction for instruction.  Only where the records come from changes: each exchange
+  // array has a halo record before thread 0 (the stress record of element j - 1, stored there by the previous rank's
+  // last thread) and two after thread NT - 1 (the x, v, Q records of nodes j + 1, j + 2, stored there by the next rank's
+  // threads 0 and 1), so every read of the substep stays a local shared-memory load at the same offset.  The substep's
+  // two barriers become cluster barriers; they order the DSMEM halo stores as the CTA barriers order the local ones (a
+  // halo slot is rewritten only after the barrier that follows its last read).  Env-level decisions (range flags, NaN
+  // flag) are reduced into rank 0's shared memory through DSMEM atomics and read back by every CTA.
+  constexpr bool CLUSTER = CVAR == 9;
   static_assert(CVAR == 0 || !MIXED, "the variants are FP64 only");
   static_assert(!FOLD || LEAN_SCR_FOLD >= 27, "hand-over rows of the folded tip");
   constexpr int SCR = FOLD ? LEAN_SCR_FOLD : CONTACT ? LEAN_SCR_CONTACT : LEAN_REC;   // rows of a slot's hand-over scratch
   using F = typename std::conditional<MIXED, float, double>::type;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  D *rec = reinterpret_cast<D *>(smem_raw);            // {x0 x1 | x2 v0 | v1 v2 | Q0 Q1 | ... | Q6 Q7 | Q8 - | - -}
-  // {s0 s1 | s2 N0 | N1 m2} (FP64: 48-byte records; mixed: 8 floats, 32-byte records); record NT = zeros (left of element 0)
-  F *sn = reinterpret_cast<F *>(rec + LEAN_REC * (NT + 2));
   constexpr int SNR = MIXED ? 8 : 6;
+  constexpr int RX = lean_extra_records(CVAR);
+  constexpr int ZR = CLUSTER ? NT + 2 : NT;   // record ZR = zeros (left of element 0); variant 9: -1, NT, NT + 1 are halos
+  D *rec = reinterpret_cast<D *>(smem_raw) + (CLUSTER ? LEAN_REC : 0);   // {x0 x1 | x2 v0 | v1 v2 | Q0 Q1 | ... | Q6 Q7 | Q8 - | - -}
+  // {s0 s1 | s2 N0 | N1 m2} (FP64: 48-byte records; mixed: 8 floats, 32-byte records)
+  F *sn = reinterpret_cast<F *>(reinterpret_cast<D *>(smem_raw) + LEAN_REC * (NT + RX)) + (CLUSTER ? SNR : 0);
   __shared__ int sh_flag[256], sh_dom[256];   // one per rod of the CTA (<= NT / 4)
   __shared__ int sh_need[CVAR == 5 ? 128 : 1];          // spline variant: which directions re-fit their magnitudes this substep, per rod
   __shared__ double sh_base[CVAR == 4 ? 128 : 1][4];   // filter variant: the moving base's command, per rod (rods of >= 9 threads)
@@ -178,20 +201,24 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   const int n_rod = MULTI ? A.n_rod : 1, has_head = MULTI ? A.has_head : 0;
   const int G = n_rod * tpr + has_head;
   const int rods_per_cta = A.sk_rods_per_cta;       // env groups per CTA
-  const int r = tid / G, u_grp = tid - r * G;
+  const int c_rank = CLUSTER ? (int)cooperative_groups::this_cluster().block_rank() : 0;
+  const int c_size = CLUSTER ? (int)cooperative_groups::this_cluster().num_blocks() : 1;
+  const int r = CLUSTER ? 0 : tid / G, u_grp = CLUSTER ? NT * c_rank + tid : tid - r * G;
   const bool is_head = MULTI && has_head && (u_grp == G - 1);
   const int arm = (MULTI && !is_head) ? u_grp / tpr : 0;
   const int j = is_head ? 0 : u_grp - arm * tpr;
-  const bool in_cta = r < rods_per_cta;
+  const bool in_cta = r < rods_per_cta && (!CLUSTER || j <= n);   // (variant 9: the last rank's threads past the tip idle)
   const bool first = (j == 0) && !is_head;          // first thread of a rod
   const bool lead = first && arm == 0;              // one thread per env: env-level flags and outputs
   const int t_head = r * G + G - 1;                 // where this env's head publishes its state
   D *sj = reinterpret_cast<D *>(sn + 6 * (NT + 2)); // assemblies: joint records (LEAN_JREC doubles per thread slot)
   D *gb = sj;                                       // filter variant: ghost-padded records of the filtered rates
-  if (tid < SNR) sn[SNR * NT + tid] = F(0);
+  if (tid < SNR) sn[SNR * ZR + tid] = F(0);
+  if (CLUSTER && tid < 256) { sh_dom[tid] = 0; sh_flag[tid] = 0; }   // (rank 0's are the cluster's env-level flags)
   if (CONTACT && tid < 2) rec[LEAN_REC * NT + 16 + tid] = D(0);   // stage-1 contact load "left of element 0"
   if (FOLD && tid < LEAN_REC) rec[LEAN_REC * NT + tid] = D(0);     // the folded tip's record: x, v published by the last thread, the rest finite
   __syncthreads();   // (the per-rod barriers below do not order this store against the other rods' reads)
+  if constexpr (CLUSTER) cluster_sync();   // every CTA of the cluster runs, with its flags zeroed, before DSMEM is touched
 
   // Barriers: data only crosses threads of the same rod, so a substep's two synchronisations can be per rod
   // (named barriers over the warps that hold the rod's threads; a warp holding the end of one rod and the start of
@@ -210,6 +237,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     }
   }
   auto rod_sync = [&]() {
+    if (CLUSTER) { cluster_sync(); return; }
     if (!rod_barriers) { __syncthreads(); return; }
     if (bar_cnt0) asm volatile("bar.sync %0, %1;" ::"r"(bar_id0), "r"(bar_cnt0) : "memory");
     if (bar_cnt1) asm volatile("bar.sync %0, %1;" ::"r"(bar_id1), "r"(bar_cnt1) : "memory");
@@ -252,7 +280,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
 
   // ---- the segments this CTA runs ------------------------------------------------------------------------------
   const int K = A.n_substeps;
-  const int P = gridDim.x, p = blockIdx.x;
+  const int P = gridDim.x, p = CLUSTER ? blockIdx.x / c_size : blockIdx.x;   // (variant 9: one item per cluster)
   int i0, i1, off0, end1;
   if (A.sk_split) {
     const long long W = (long long)A.sk_items * K, b0 = W * p / P, b1 = W * (p + 1) / P;
@@ -291,7 +319,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // (folded variants: the tip node's record is record NT, published by the last element's thread)
     const int t_next = elem_ok ? ((FOLD && j == n - 1) ? NT : tid + 1) : tid;
     const int t_next2 = vor_ok ? ((FOLD && j == n - 2) ? NT : tid + 2) : t_next;
-    const int t_prev = (active && j > 0) ? tid - 1 : NT;
+    const int t_prev = (active && j > 0) ? tid - 1 : ZR;
 
     D x[3] = {D(0), D(0), D(0)}, v[3] = {D(0), D(0), D(0)}, w[3] = {D(0), D(0), D(0)};
     D Q[9] = {D(1), D(0), D(0), D(0), D(1), D(0), D(0), D(0), D(1)};
@@ -581,6 +609,12 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         o[0] = make_double2(x[0], x[1]); o[1] = make_double2(x[2], v[0]); o[2] = make_double2(v[1], v[2]);
         o[3] = make_double2(Q[0], Q[1]); o[4] = make_double2(Q[2], Q[3]); o[5] = make_double2(Q[4], Q[5]);
         o[6] = make_double2(Q[6], Q[7]); rec[LEAN_REC * tid + 14] = Q[8];
+        if (CLUSTER && tid < 2 && c_rank > 0) {   // nodes j + 1, j + 2 of the previous rank's last two threads
+          double2 *h = cluster_smem(reinterpret_cast<double2 *>(rec + LEAN_REC * (NT + tid)), c_rank - 1);
+#pragma unroll
+          for (int k = 0; k < 7; k++) h[k] = o[k];
+          reinterpret_cast<D *>(h)[14] = Q[8];
+        }
         if (FOLD && is_last) {
           double2 *ot = reinterpret_cast<double2 *>(rec + LEAN_REC * NT);
           ot[0] = make_double2(xt[0], xt[1]); ot[1] = make_double2(xt[2], vt[0]); ot[2] = make_double2(vt[1], vt[2]);
@@ -834,6 +868,10 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         o[0] = make_double2((double)sfl[0], (double)sfl[1]);
         o[1] = make_double2((double)sfl[2], (double)fma(kx0, ie3, -m0));
         o[2] = make_double2((double)fma(kx1, ie3, -m1), CONTACT ? (double)fma(-kx2, ie3, m2) : (double)m2);   // (the reader subtracts)
+        if (CLUSTER && tid == NT - 1 && c_rank + 1 < c_size) {   // element j - 1 of the next rank's thread 0
+          double2 *h = cluster_smem(reinterpret_cast<double2 *>(sn - SNR), c_rank + 1);
+          h[0] = o[0]; h[1] = o[1]; h[2] = o[2];
+        }
       }
       // rotational damper c_w^e = c_w exp((e-1) ln c_w) as a quadratic in (e-1) (coefficients made on the host; the
       // range limit keeps the dropped cubic term below 1.4e-15); c_w1 = c_w2 for a circular cross-section
@@ -1347,7 +1385,16 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
 
     // ---- write back, NaN guard, model outputs --------------------------------------------------------------------
     bool redo = false;
-    if (FASTONLY) {    // env-level OR of the range flags; a flagged env keeps its pre-launch state in global memory
+    if (FASTONLY && CLUSTER) {
+      // the cluster's OR in rank 0's sh_dom[0], which every CTA reads back: a flagged env leaves no part of its rod
+      // written back.  (redo[env] is read ahead of the barrier after which the lead may set it.)
+      const bool flagged = live && A.redo[env] != 0;
+      if (live && dom_bad) atomicOr(cluster_smem(&sh_dom[0], 0), dom_bad);
+      cluster_sync();
+      const int dom = *cluster_smem(&sh_dom[0], 0);
+      redo = live && (dom != 0 || flagged);
+      if (redo && lead && atomicExch(&A.redo[env], 1) == 0 && A.redo_count) count_redo(dom);
+    } else if (FASTONLY) {    // env-level OR of the range flags; a flagged env keeps its pre-launch state in global memory
       if (tid < 256) sh_dom[tid] = 0;
       __syncthreads();
       if (live && dom_bad) atomicOr(&sh_dom[r], dom_bad);
@@ -1418,20 +1465,30 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     }
     // per-rod NaN flag and tangents for the observation (rod r occupies tids r*tpr .. r*tpr+n)
     D *sh_t = rec;   // 3 rows of NT + 2
-    if (tid < 256) sh_flag[tid] = 0;
-    if (active && (A.model == MODEL_SOFT_PENDULUM || (LAPL && A.model == MODEL_SOFT_PENDULUM_3D))) {
+    if constexpr (CLUSTER) {
+      // the cluster's OR in rank 0's sh_flag[0]; the barrier also orders every rank's tangents (written to the state
+      // block in the last substep) before the lead's reads of them
+      if (active && bad) atomicOr(cluster_smem(&sh_flag[0], 0), 1);
+      cluster_sync();
+    } else {
+      if (tid < 256) sh_flag[tid] = 0;
+      if (active && (A.model == MODEL_SOFT_PENDULUM || (LAPL && A.model == MODEL_SOFT_PENDULUM_3D))) {
 #pragma unroll
-      for (int i = 0; i < 3; i++) sh_t[i * RS + tid] = (j < n) ? (D)st[(F_TAN + i) * stride + j] : D(0);
+        for (int i = 0; i < 3; i++) sh_t[i * RS + tid] = (j < n) ? (D)st[(F_TAN + i) * stride + j] : D(0);
+      }
+      __syncthreads();
+      if (active && bad) atomicOr(&sh_flag[r], 1);
+      __syncthreads();
     }
-    __syncthreads();
-    if (active && bad) atomicOr(&sh_flag[r], 1);
-    __syncthreads();
     if (!FASTONLY && A.redo_filter && active && lead) A.redo[env] = 0;
     if (active && lead && !redo) {
       const bool invalid = sh_flag[r] != 0;
       if (mus) A.muscle[(size_t)env * A.muscle_dim] = mus_t;
       if (A.model == MODEL_SOFT_PENDULUM) {
-        soft_pendulum_outputs<D>(sh_t + tid, RS, n, x[0], v[0],
+        const D *tan = sh_t + tid;
+        int tan_stride = RS;
+        if constexpr (CLUSTER) { tan = st + F_TAN * stride; tan_stride = stride; }   // (the state block: every rank's)
+        soft_pendulum_outputs<D>(tan, tan_stride, n, x[0], v[0],
                                  A.action_dim > 0 ? A.action[(size_t)env * A.action_dim] : 0.0f, invalid,
                                  A.obs + (size_t)env * A.obs_dim, A.reward + env, A.terminated + env);
       } else if (LAPL && A.model == MODEL_SOFT_PENDULUM_3D) {
@@ -1456,6 +1513,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     }
     __syncthreads();   // the staging rows are free again before the next item publishes
   }
+  if constexpr (CLUSTER) cluster_sync();   // no CTA leaves while another may still access its shared memory
 }
 
 }  // namespace sr

@@ -275,17 +275,22 @@ template <typename T> __device__ __noinline__ T bend_factor_ref(T u) {
 template <typename T> __device__ __noinline__ T exp_ref(T x) { return exp_(x); }
 
 // numpy's pairwise float64 row sum (np.mean over the contiguous axis): 8 running sums for
-// blocks of <= 128 values, recursive halving above (numpy/core/src/umath/loops_utils.h.src)
-template <typename T> __device__ double np_pairwise_sum(const T *a, int n) {
+// blocks of <= 128 values, recursive halving above (numpy/core/src/umath/loops_utils.h.src).  The halving is unrolled
+// into DEPTH levels of distinct functions instead of recursion, so that the stack a kernel needs is known at compile
+// time (a recursive call chain runs in the default 1 KB stack, which a 2048-element rod's five levels overflow).
+// DEPTH = 6 covers n <= 128 * 2^6 = 8192 (every level halves).
+template <int DEPTH = 6, typename T> __device__ __noinline__ double np_pairwise_sum(const T *a, int n) {
   if (n < 8) {
     double r = 0.0;
     for (int i = 0; i < n; i++) r += (double)a[i];
     return r;
   }
-  if (n > 128) {
-    int n2 = n / 2;
-    n2 -= n2 % 8;
-    return np_pairwise_sum(a, n2) + np_pairwise_sum(a + n2, n - n2);
+  if constexpr (DEPTH > 0) {
+    if (n > 128) {
+      int n2 = n / 2;
+      n2 -= n2 % 8;
+      return np_pairwise_sum<DEPTH - 1>(a, n2) + np_pairwise_sum<DEPTH - 1>(a + n2, n - n2);
+    }
   }
   double r[8];
   for (int j = 0; j < 8; j++) r[j] = (double)a[j];

@@ -434,6 +434,40 @@ template <typename T> bool is_lean_config(const sr::RodArgs<T> &A) {
            A.laplace_order > 0 || A.bc_kind == sr::BC_MOVING_BASE || A.sucker || A.ext_force || A.ext_couple || A.elem_tab);
 }
 
+int cluster_setting() {    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster variant too (A/B; same bits)
+  static int v = -1;
+  if (v < 0) { const char *e = getenv("SOFTROD_LEAN_CLUSTER"); v = (e && atoi(e) != 0) ? 1 : 0; }
+  return v;
+}
+
+// CTAs of the cluster that holds one rod of n elements in the cluster variant (variant 9): n + 1 threads of 512 per CTA
+int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
+
+// Rods of 1024-4095 elements (sr_create admits only variant 0's model there) and, with SOFTROD_LEAN_CLUSTER=1, plain
+// lean FP64 rods of 512-1023 elements: one rod per thread-block cluster (rod_kernel_lean.cuh, variant 9)
+bool use_lean_cluster(const sr_handle *h, const sr::RodArgs<double> &A) {
+  if (A.n_elem >= 1024) return true;
+  return cluster_setting() && A.n_elem >= 512 && is_lean_config(A) &&
+         (A.model == sr::MODEL_ROD || A.model == sr::MODEL_SOFT_PENDULUM) && h->cfg.math == SR_MATH_FAST;
+}
+
+// fast-only kernel + fallback over the envs it flagged, as launch_lean_pair; one cluster per env, no stream-K split
+int launch_lean_cluster(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
+  const int C = lean_cluster_size(A.n_elem);
+  A.sk_rods_per_cta = 1; A.sk_items = A.n_env; A.sk_split = 0; A.sk_rodsync = 0;
+  A.sk_scratch = nullptr; A.sk_flag = nullptr;
+  if (use_fast_pair(h, A, s)) {
+    cudaError_t e = sr::launch_lean_cluster_kernel<true>(A, C, s);
+    h->launches++;
+    if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
+    A.redo_filter = 1;
+  }
+  cudaError_t e = sr::launch_lean_cluster_kernel<false>(A, C, s);
+  h->launches++;
+  if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
+  return SR_OK;
+}
+
 // tapered rods: safe kernel with per-element constants in registers (CTA sizes 384 / 1024 only)
 template <int NT> int launch_tapered(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
   const bool multi = A.n_rod > 1 || A.has_head;
@@ -586,6 +620,7 @@ template <typename T> int dispatch_packed(sr_handle *h, sr::RodArgs<T> &A, cudaS
         default: return launch_lean_pair<T, 256, 2, 4>(h, A, s);
       }
     }
+    if (use_lean_cluster(h, A)) return launch_lean_cluster(h, A, s);
     // a rod of exactly 512 elements: 512 threads with the tip node folded into the last one (128 registers) instead of
     // 513 threads in a 544-thread CTA (96 registers); SOFTROD_LEAN_FOLD=0 switches back (A/B)
     static int fold_off = -1;
@@ -660,7 +695,17 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   if (cfg->struct_size != (int32_t)sizeof(sr_config))
     return fail(SR_E_INVALID, "sr_create: sr_config.struct_size mismatch (ABI skew)");
   if (cfg->n_env <= 0 || cfg->n_elem < 3) return fail(SR_E_INVALID, "sr_create: n_env > 0 and n_elem >= 3 required");
-  if (cfg->n_elem > 1023) return fail(SR_E_INVALID, "sr_create: n_elem <= 1023 in this build (one rod per CTA)");
+  if (cfg->n_elem > 4095)
+    return fail(SR_E_INVALID, "sr_create: n_elem <= 4095 (rods of 1024-4095 elements span a thread-block cluster of up to 8 CTAs)");
+  if (cfg->n_elem > 1023 &&
+      (cfg->dtype != SR_DTYPE_F64 || cfg->math != SR_MATH_FAST ||
+       (cfg->model != SR_MODEL_ROD && cfg->model != SR_MODEL_SOFT_PENDULUM) ||
+       (cfg->bc_kind != SR_BC_FREE && cfg->bc_kind != SR_BC_ONE_END_FIXED && cfg->bc_kind != SR_BC_PENDULUM_SLIDER) ||
+       cfg->laplace_filter_order != 0 || cfg->contact_on || cfg->muscle_on || cfg->spline_dir_mask || cfg->n_rod_per_env > 1 ||
+       cfg->has_head || cfg->tip_radius > 0.0 || cfg->sucker_on || cfg->tm_muscle_on || cfg->muscle_layers_on))
+    return fail(SR_E_INVALID, "sr_create: n_elem of 1024-4095 is built for SR_DTYPE_F64, SR_MATH_FAST, SR_MODEL_ROD or "
+                              "SR_MODEL_SOFT_PENDULUM, one untapered rod per env with a free, clamped or slider end, gravity, "
+                              "damping and the base point force; no contact, muscle or spline torques, suckers or Laplace filter");
   if (cfg->n_elem > 127 && cfg->math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_create: faithful math supports n_elem <= 127");
   if (cfg->dtype != SR_DTYPE_F64 && cfg->dtype != SR_DTYPE_F32) return fail(SR_E_INVALID, "sr_create: bad dtype");
   if (cfg->dtype == SR_DTYPE_F32 && cfg->math != SR_MATH_FAST)
@@ -761,6 +806,12 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   }
   if (cfg->device < 0 || cfg->device >= ndev) return fail(SR_E_INVALID, "sr_create: bad device ordinal");
   SR_CUDA(cudaSetDevice(cfg->device));
+  if (cfg->n_elem > 1023) {
+    const int C = lean_cluster_size(cfg->n_elem);
+    if (sr::lean_cluster_max_active(C) < 1)
+      return fail(SR_E_CUDA, "sr_create: n_elem = " + std::to_string(cfg->n_elem) + " needs a cluster of " + std::to_string(C) +
+                                 " CTAs of 512 threads, and this device cannot launch one");
+  }
 
   sr_handle *h = new (std::nothrow) sr_handle();
   if (!h) return fail(SR_E_ALLOC, "sr_create: out of host memory");
@@ -1154,6 +1205,7 @@ int sr_spline_basis(int32_t P, double base_length, double *out) {
 int sr_get_rest_kappa(sr_handle *h, void **rest_kappa_dev) {
   if (!h || !rest_kappa_dev) return fail(SR_E_INVALID, "sr_get_rest_kappa: null argument");
   if (h->cfg.math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for SR_MATH_FAST only");
+  if (h->cfg.n_elem > 1023) return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for n_elem <= 1023");
   if (!h->rest_kappa) {
     SR_CUDA(cudaSetDevice(h->cfg.device));
     size_t bytes = (size_t)h->cfg.n_env * h->n_rod * 3 * h->stride * h->elem_size;
@@ -1206,6 +1258,7 @@ int sr_get_ext_loads(sr_handle *h, void **force_dev, void **couple_dev) {
   if (h->cfg.math != SR_MATH_FAST || h->cfg.model != SR_MODEL_ROD || h->cfg.laplace_filter_order != 0 ||
       h->cfg.bc_kind == SR_BC_MOVING_BASE)
     return fail(SR_E_INVALID, "sr_get_ext_loads: external loads are built for SR_MATH_FAST / SR_MODEL_ROD without filter / moving base");
+  if (h->cfg.n_elem > 1023) return fail(SR_E_INVALID, "sr_get_ext_loads: external loads are built for n_elem <= 1023");
   if (!h->ext_force) {
     SR_CUDA(cudaSetDevice(h->cfg.device));
     const size_t bytes = (size_t)h->cfg.n_env * h->n_rod * 3 * h->stride * h->elem_size;

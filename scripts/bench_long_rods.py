@@ -1,0 +1,140 @@
+"""Long rods on thread-block clusters (variant 9 of rod_kernel_lean.cuh): device time per launch of K = 100 substeps.
+
+Clamped rods (BASELINE config 3's model), with enough envs that the state block exceeds the 126 MB L2 (>= 256 MB).
+Cases: n = 600 and 1023 on the one-CTA kernel (768 / 1024 threads) and on the forced cluster kernel (C = 2), which
+run as alternating subprocesses (SOFTROD_LEAN_CLUSTER is read once per process), two rounds each; n = 1024, 2047 and
+4095, where the cluster kernel is the only one.  Reported: ms per launch (median of 20 CUDA-event-timed launches after
+warm-up), element-substeps/s, and the share of the measured FP64 peak (sr_measure_fp64_peak) at 440 FLOP per
+element-substep.  A probe compiled into a temporary directory reports how many clusters of C one-CTA-per-SM blocks
+(512 threads, > 114 KB of shared memory each) the device keeps resident, and so what fraction of the SMs a full wave
+of C-CTA clusters leaves idle.
+
+    python scripts/bench_long_rods.py [--out FILE]     (the report goes to stdout, and to FILE if given)
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import tempfile
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+K, TIMED, WARMUP = 100, 20, 5
+FLOP_PER_ELEMENT_SUBSTEP = 440
+STATE_BYTES = 256 << 20
+
+_PROBE = r"""
+#include <cstdio>
+#include <cuda_runtime.h>
+__global__ void __launch_bounds__(512, 1) probe(int *p) { extern __shared__ int s[]; if (p) p[threadIdx.x] = s[threadIdx.x]; }
+int main() {
+  const int smem = 120 * 1024;   // one CTA per SM, like the lean kernel's 512 threads x 128 registers
+  if (cudaFuncSetAttribute(probe, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return 1;
+  for (int c = 1; c <= 8; c++) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(c); cfg.blockDim = dim3(512); cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute a; a.id = cudaLaunchAttributeClusterDimension;
+    a.val.clusterDim.x = c; a.val.clusterDim.y = 1; a.val.clusterDim.z = 1;
+    cfg.attrs = &a; cfg.numAttrs = 1;
+    int n = 0;
+    if (cudaOccupancyMaxActiveClusters(&n, probe, &cfg) != cudaSuccess) return 2;
+    printf("%d %d\n", c, n);
+  }
+  return 0;
+}
+"""
+
+
+def one(n, cluster):
+    """Runs in a subprocess of its own: time one case, print one JSON line."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    from gym_softrobot_b200 import _native as nat
+    stride = 32 * ((n + 1 + 31) // 32)
+    n_env = -(-STATE_BYTES // (32 * stride * 8))
+    h = nat.Handle(model=nat.MODEL_ROD, n_env=n_env, n_elem=n, dt=2e-6 * 1023 / n, base_length=1.0, base_radius=0.004,
+                   density=1000.0, youngs_modulus=1e6, gravity=(0.0, -9.80665, 0.0), damping_constant=2e-3,
+                   bc_kind=nat.BC_ONE_END_FIXED, math=nat.MATH_FAST)
+    ang = np.deg2rad(np.random.default_rng(n).uniform(-5, 5, n_env))
+    init = np.zeros((n_env, 9))
+    init[:, 3], init[:, 4], init[:, 6], init[:, 7] = np.cos(ang), np.sin(ang), -np.sin(ang), np.cos(ang)
+    h.reset_host(init)
+    obs = torch.empty((n_env, h.obs_dim), dtype=torch.float32, device="cuda")
+    rew = torch.empty(n_env, dtype=torch.float64, device="cuda")
+    term = torch.empty(n_env, dtype=torch.uint8, device="cuda")
+    s = torch.cuda.current_stream()
+    for _ in range(WARMUP):
+        h.step(None, K, obs, rew, term)
+    torch.cuda.synchronize()
+    times = []
+    for _ in range(TIMED):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(s)
+        h.step(None, K, obs, rew, term)
+        e1.record(s)
+        e1.synchronize()
+        times.append(e0.elapsed_time(e1))
+    assert np.isfinite(h.state_tensor().cpu().numpy()).all() and int(term.sum()) == 0
+    ms = float(np.median(times))
+    rate = n_env * n * K / (ms * 1e-3)
+    print(json.dumps(dict(n=n, kernel="cluster" if cluster else "one-CTA", C=(n + 512) // 512 if cluster else 1,
+                          n_env=n_env, state_MB=round(n_env * 32 * stride * 8 / 2**20), ms=ms, ms_min=min(times),
+                          ms_max=max(times), elem_substeps_per_s=rate, fallbacks=h.fallback_count())))
+    h.close()
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default=None, help="also write the report to this file")
+    ap.add_argument("--one", nargs=2, type=int, help=argparse.SUPPRESS)
+    a = ap.parse_args()
+    if a.one:
+        return one(*a.one)
+    import torch
+    sys.path.insert(0, ROOT)
+    from gym_softrobot_b200 import _native as nat
+    assert torch.cuda.is_available(), "this benchmark needs the GPU"
+    lines = []
+
+    def say(s):
+        print(s, flush=True)
+        lines.append(s)
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                         capture_output=True, text=True).stdout.strip()
+    sm = torch.cuda.get_device_properties(0).multi_processor_count
+    say(f"device: {torch.cuda.get_device_name(0)}, {sm} SMs; nvidia-smi name, power limit, max SM clock: {smi}")
+    peak = nat.measure_fp64_peak(0)
+    say(f"measured FP64 peak (sr_measure_fp64_peak): {peak:.2f} TFLOP/s")
+    with tempfile.TemporaryDirectory() as tmp:
+        src, exe = os.path.join(tmp, "probe.cu"), os.path.join(tmp, "probe")
+        open(src, "w").write(_PROBE)
+        nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+        subprocess.run([nvcc, "-gencode", "arch=compute_100a,code=sm_100a", src, "-o", exe], check=True)
+        for line in subprocess.run([exe], check=True, capture_output=True, text=True).stdout.split("\n"):
+            if line.strip():
+                c, nc = map(int, line.split())
+                say(f"clusters of {c} one-CTA-per-SM blocks resident at once: {nc} ({nc * c} of {sm} SMs busy, "
+                    f"{100.0 * (sm - nc * c) / sm:.1f} % idle)")
+    cases = [(600, 0), (600, 1), (1023, 0), (1023, 1)] * 2 + [(1024, 1), (2047, 1), (4095, 1)]
+    for n, cl in cases:
+        env = dict(os.environ)
+        env.pop("SOFTROD_LEAN_CLUSTER", None)
+        if cl:
+            env["SOFTROD_LEAN_CLUSTER"] = "1"
+        out = subprocess.run([sys.executable, os.path.abspath(__file__), "--one", str(n), str(cl)], env=env,
+                             capture_output=True, text=True)
+        if out.returncode != 0:
+            raise SystemExit(out.stdout + out.stderr)
+        r = json.loads(out.stdout.strip().splitlines()[-1])
+        share = r["elem_substeps_per_s"] * FLOP_PER_ELEMENT_SUBSTEP / (peak * 1e12)
+        say(f"n={r['n']:5d} {r['kernel']:8s} C={r['C']} n_env={r['n_env']:5d} state={r['state_MB']} MB: "
+            f"{r['ms']:.3f} ms/launch (min {r['ms_min']:.3f}, max {r['ms_max']:.3f}), "
+            f"{r['elem_substeps_per_s'] / 1e9:.2f} G element-substeps/s, {100 * share:.1f} % of FP64 peak, "
+            f"fallbacks {r['fallbacks']}")
+    if a.out:
+        open(a.out, "w").write("\n".join(lines) + "\n")
+
+
+if __name__ == "__main__":
+    main()
