@@ -3,8 +3,8 @@
 // configs 2 and 3).  Variants 1-7 put the other models on the same skeleton (see the comment at the kernel):
 // 1 plane contact + rest curvature, 2 + travelling-wave muscle, 3 assemblies (arms + rigid head + joints), 4 Laplace
 // filter + moving base, 5 spline muscle torques, 6 / 7 = 0 / 1 with the tip node folded into the last thread, 8 = 0 for
-// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits), 9 = 0 for rods of 512-4095 elements,
-// one rod per thread-block cluster of 2-8 CTAs (same substep, same bits).
+// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits), 9 / 10 = 0 / 4 for rods of 512-4095
+// elements, one rod per thread-block cluster of 2-8 CTAs (same substep, same bits).
 //
 // Same mapping as rod_kernel_packed.cuh (one thread per node/element, rods packed back to back across a
 // 256-thread CTA, state in registers for the whole launch, neighbour data through array-of-structures
@@ -106,16 +106,22 @@ constexpr int LEAN_REC = 18;        // exchange record per thread (doubles), 144
 constexpr int LEAN_JREC = 10;      // assemblies: joint record of an arm's first thread {reaction force, couple on the head, couple on element 0, -}
 // filter variant: records of 6 doubles with 6 ghost records on either side of every rod (rods of >= 9 threads)
 // (8 ghost records per side, 6 used: a rod's records then start a multiple of 8 records = 96 words after where the
-// previous rod's would continue, so a quarter-warp that straddles two rods still hits eight distinct 4-bank groups)
-constexpr int lean_ghost_records(int nt) { return nt + 16 * (nt / 9) + 16; }
-// records of each exchange array beyond the NT threads' own: variant 9 has a halo record before thread 0, two after
-// thread NT - 1 and a zero record; the others a zero record and a spare one
-__host__ __device__ constexpr int lean_extra_records(int cvar) { return cvar == 9 ? 4 : 2; }
+// previous rod's would continue, so a quarter-warp that straddles two rods still hits eight distinct 4-bank groups).
+// A CTA of more than 512 threads holds one rod of >= 512 elements and at most the head of an idle second group, whose
+// records and taps end within 30 records past NT: sized as rods of >= 9 threads, its ghost array alone would take
+// 73 KB at 544 threads and push the 768- and 1024-thread CTAs past the 227 KB a CTA can have.
+constexpr int lean_ghost_records(int nt) { return nt <= 512 ? nt + 16 * (nt / 9) + 16 : nt + 48; }
+// records of each exchange array beyond the NT threads' own: the cluster variants 9 / 10 have a halo record before
+// thread 0, two after thread NT - 1 and a zero record; the others a zero record and a spare one
+__host__ __device__ constexpr int lean_extra_records(int cvar) { return cvar == 9 || cvar == 10 ? 4 : 2; }
+// variant 10: each rank's ghost-padded filter records hold the rod indices [NT c - 8, NT c + NT + 8) (6 of the 8 halo
+// records per side used, as variant 4 pads them)
 constexpr int lean_smem_words(int nt, int cvar = 0) {
-  return (LEAN_REC + 6 + (cvar == 3 ? LEAN_JREC : 0)) * (nt + lean_extra_records(cvar)) + (cvar == 4 ? 6 * lean_ghost_records(nt) : 0);
+  return (LEAN_REC + 6 + (cvar == 3 ? LEAN_JREC : 0)) * (nt + lean_extra_records(cvar)) +
+         (cvar == 4 ? 6 * lean_ghost_records(nt) : cvar == 10 ? 6 * (nt + 16) : 0);
 }
 
-// variant 9: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
+// variants 9 / 10: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
 template <typename T> __device__ __forceinline__ T *cluster_smem(T *p, int rank) {
   return cooperative_groups::this_cluster().map_shared_rank(p, (unsigned)rank);
 }
@@ -152,8 +158,8 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   constexpr bool MIXED = sizeof(ST) == 4;
   // CVAR: 0 plain rod, 1 contact variant, 2 contact variant + travelling-wave muscle, 3 contact variant for assemblies
   // (several rods + one rigid head thread per env, FixedJoint2Rigid joints, BodyBoundaryCondition on the head)
-  // 4: SoftPendulum3D-v0 — LaplaceDissipationFilter + host-commanded moving base (no contact)
-  constexpr bool LAPL = CVAR == 4;
+  // 4: SoftPendulum3D-v0 — LaplaceDissipationFilter + host-commanded moving base (no contact); 10: the same on a cluster
+  constexpr bool LAPL = CVAR == 4 || CVAR == 10;
   // 5: clamped / free rod + MuscleTorquesWithVaryingBetaSplines (SoftArmTracking-v0); safe variant only, see below
   constexpr bool SPL = CVAR == 5;
   // 6 / 7: variants 0 / 1 with the tip node folded into the last element's thread: a rod of n elements then takes n
@@ -179,7 +185,12 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   // two barriers become cluster barriers; they order the DSMEM halo stores as the CTA barriers order the local ones (a
   // halo slot is rewritten only after the barrier that follows its last read).  Env-level decisions (range flags, NaN
   // flag) are reduced into rank 0's shared memory through DSMEM atomics and read back by every CTA.
-  constexpr bool CLUSTER = CVAR == 9;
+  // 10: variant 4 in variant 9's layout (SoftPendulum3D-v0 at 512-4095 elements).  The filter's pass 0 reads the rate
+  // records of j - 1 and j + 1: rec gets a halo at -1 too, and the filter's own record is pushed into the neighbours'
+  // halos -1 / NT.  Each rank's ghost-padded array gb holds the rod indices [NT c - 8, NT c + NT + 8), and a g record
+  // of index k is stored into every rank whose taps read it (put_g below); the reflected ghosts follow the same rule.
+  // The filter's two barriers become cluster barriers as well: four per substep.
+  constexpr bool CLUSTER = CVAR == 9 || CVAR == 10;
   static_assert(CVAR == 0 || !MIXED, "the variants are FP64 only");
   static_assert(!FOLD || LEAN_SCR_FOLD >= 27, "hand-over rows of the folded tip");
   constexpr int SCR = FOLD ? LEAN_SCR_FOLD : CONTACT ? LEAN_SCR_CONTACT : LEAN_REC;   // rows of a slot's hand-over scratch
@@ -193,7 +204,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   F *sn = reinterpret_cast<F *>(reinterpret_cast<D *>(smem_raw) + LEAN_REC * (NT + RX)) + (CLUSTER ? SNR : 0);
   __shared__ int sh_flag[256], sh_dom[256];   // one per rod of the CTA (<= NT / 4)
   __shared__ int sh_need[CVAR == 5 ? 128 : 1];          // spline variant: which directions re-fit their magnitudes this substep, per rod
-  __shared__ double sh_base[CVAR == 4 ? 128 : 1][4];   // filter variant: the moving base's command, per rod (rods of >= 9 threads)
+  __shared__ double sh_base[CVAR == 4 ? 128 : 1][4];   // filter variant: the moving base's command, per rod (rods of >= 9 threads; variant 10: rank 0's one rod)
 
   const int tid = threadIdx.x;
   const int n = A.n_elem, stride = A.stride, tpr = FOLD ? n : n + 1;
@@ -211,7 +222,8 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   const bool first = (j == 0) && !is_head;          // first thread of a rod
   const bool lead = first && arm == 0;              // one thread per env: env-level flags and outputs
   const int t_head = r * G + G - 1;                 // where this env's head publishes its state
-  D *sj = reinterpret_cast<D *>(sn + 6 * (NT + 2)); // assemblies: joint records (LEAN_JREC doubles per thread slot)
+  // past the stress records: assemblies: joint records (LEAN_JREC doubles per thread slot)
+  D *sj = reinterpret_cast<D *>(sn - (CLUSTER ? SNR : 0) + 6 * (NT + RX));
   D *gb = sj;                                       // filter variant: ghost-padded records of the filtered rates
   if (tid < SNR) sn[SNR * ZR + tid] = F(0);
   if (CLUSTER && tid < 256) { sh_dom[tid] = 0; sh_flag[tid] = 0; }   // (rank 0's are the cluster's env-level flags)
@@ -1150,6 +1162,12 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
             const bool node_in = active && j > 0 && j < n, elem_in = active && j > 0 && j < n - 1;
             double2 *own = reinterpret_cast<double2 *>(rec + LEAN_REC * tid);
             own[0] = make_double2(v[0], v[1]); own[1] = make_double2(v[2], w[0]); own[2] = make_double2(w[1], w[2]);
+            if constexpr (CLUSTER) {   // the neighbours of pass 0 across the rank boundary: halos NT and -1
+              double2 *h = nullptr;
+              if (tid == 0 && c_rank > 0) h = cluster_smem(reinterpret_cast<double2 *>(rec + LEAN_REC * NT), c_rank - 1);
+              if (tid == NT - 1 && c_rank + 1 < c_size) h = cluster_smem(reinterpret_cast<double2 *>(rec - LEAN_REC), c_rank + 1);
+              if (h) { h[0] = make_double2(v[0], v[1]); h[1] = make_double2(v[2], w[0]); h[2] = make_double2(w[1], w[2]); }
+            }
             rod_sync();
             D g[6];
             {
@@ -1163,22 +1181,43 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
 #pragma unroll
               for (int c = 0; c < 6; c++) g[c] = ((-rv[c] - lv[c]) + D(2) * mv[c]) * D(0.25);
             }
-            D *slot = gb + 6 * (r * (tpr + 16) + 8 + j);
-            {
-              double2 *o = reinterpret_cast<double2 *>(slot);
-              if (j < n) { o[0] = make_double2(g[0], g[1]); o[1] = make_double2(g[2], g[3]); o[2] = make_double2(g[4], g[5]); }
-              else { o[0] = make_double2(g[0], g[1]); slot[2] = g[2]; }   // tip node: its record's element half is element n-2's ghost
+            D *slot = gb + 6 * (CLUSTER ? 8 + tid : r * (tpr + 16) + 8 + j);
+            // put_g(k, store): `store` writes into the record of rod index k.  Variant 10: into that of every rank whose
+            // taps read index k, i.e. whose window [NT c - 6, NT c + NT + 6) holds it — its owner, the previous rank for
+            // the first six indices of a rank, the next one for the last six; the ghosts beyond both ends alike.  A
+            // thread stores its own index and ghosts at most 13 indices away, so only its own rank and the two next to
+            // it can hold them.
+            auto put_g = [&](int k, auto &&store) {
+              if constexpr (!CLUSTER) {
+                store(slot + 6 * (k - j));
+              } else {
+                static_assert(NT > 13 + 6, "a rank's window reaches into its neighbours only");
+#pragma unroll
+                for (int d = -1; d <= 1; d++) {
+                  const int t = c_rank + d, loc = k - NT * t + 8;
+                  if (t < 0 || t >= c_size || loc < 2 || loc >= NT + 14) continue;
+                  if (d == 0) store(gb + 6 * loc);
+                  else store(cluster_smem(gb + 6 * loc, t));
+                }
+              }
+            };
+            if (!CLUSTER || in_cta) {   // (variant 10: the last rank's idle threads hold indices past the ghosts)
+              put_g(j, [&](D *p) {
+                double2 *o = reinterpret_cast<double2 *>(p);
+                if (j < n) { o[0] = make_double2(g[0], g[1]); o[1] = make_double2(g[2], g[3]); o[2] = make_double2(g[4], g[5]); }
+                else { o[0] = make_double2(g[0], g[1]); p[2] = g[2]; }   // tip node: its record's element half is element n-2's ghost
+              });
               if (j >= 1 && j <= 6) {              // left ghosts: both fields reflect about index 0
-                double2 *gl = reinterpret_cast<double2 *>(slot - 12 * j);
-                gl[0] = make_double2(-g[0], -g[1]); gl[1] = make_double2(-g[2], -g[3]); gl[2] = make_double2(-g[4], -g[5]);
+                put_g(-j, [&](D *p) {
+                  double2 *gl = reinterpret_cast<double2 *>(p);
+                  gl[0] = make_double2(-g[0], -g[1]); gl[1] = make_double2(-g[2], -g[3]); gl[2] = make_double2(-g[4], -g[5]);
+                });
               }
               if (j >= n - 6 && j <= n - 1) {      // right ghosts of the node field: about node n
-                D *gr = slot + 12 * (n - j);
-                gr[0] = -g[0]; gr[1] = -g[1]; gr[2] = -g[2];
+                put_g(2 * n - j, [&](D *gr) { gr[0] = -g[0]; gr[1] = -g[1]; gr[2] = -g[2]; });
               }
               if (j >= n - 7 && j <= n - 2) {      // right ghosts of the element field: about element n - 1
-                D *gr = slot + 12 * (n - 1 - j);
-                gr[3] = -g[3]; gr[4] = -g[4]; gr[5] = -g[5];
+                put_g(2 * (n - 1) - j, [&](D *gr) { gr[3] = -g[3]; gr[4] = -g[4]; gr[5] = -g[5]; });
               }
             }
             rod_sync();
@@ -1484,10 +1523,10 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     if (active && lead && !redo) {
       const bool invalid = sh_flag[r] != 0;
       if (mus) A.muscle[(size_t)env * A.muscle_dim] = mus_t;
+      const D *tan = sh_t + tid;
+      int tan_stride = RS;
+      if constexpr (CLUSTER) { tan = st + F_TAN * stride; tan_stride = stride; }   // (the state block: every rank's)
       if (A.model == MODEL_SOFT_PENDULUM) {
-        const D *tan = sh_t + tid;
-        int tan_stride = RS;
-        if constexpr (CLUSTER) { tan = st + F_TAN * stride; tan_stride = stride; }   // (the state block: every rank's)
         soft_pendulum_outputs<D>(tan, tan_stride, n, x[0], v[0],
                                  A.action_dim > 0 ? A.action[(size_t)env * A.action_dim] : 0.0f, invalid,
                                  A.obs + (size_t)env * A.obs_dim, A.reward + env, A.terminated + env);
@@ -1499,7 +1538,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         }
         const float act_f0 = A.action_dim > 0 ? A.action[(size_t)env * A.action_dim] : 0.0f;
         const float act_f1 = A.action_dim > 1 ? A.action[(size_t)env * A.action_dim + 1] : 0.0f;
-        soft_pendulum_3d_outputs<D>(sh_t + tid, RS, n, x0, v0, act_f0, act_f1, (double)aux[0], (double)aux[1],
+        soft_pendulum_3d_outputs<D>(tan, tan_stride, n, x0, v0, act_f0, act_f1, (double)aux[0], (double)aux[1],
                                     invalid, A.obs + (size_t)env * A.obs_dim, A.reward + env, A.terminated + env,
                                     reinterpret_cast<D *>(aux + 6));
       } else {

@@ -434,35 +434,40 @@ template <typename T> bool is_lean_config(const sr::RodArgs<T> &A) {
            A.laplace_order > 0 || A.bc_kind == sr::BC_MOVING_BASE || A.sucker || A.ext_force || A.ext_couple || A.elem_tab);
 }
 
-int cluster_setting() {    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster variant too (A/B; same bits)
+int cluster_setting() {    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster variants too (A/B; same bits)
   static int v = -1;
   if (v < 0) { const char *e = getenv("SOFTROD_LEAN_CLUSTER"); v = (e && atoi(e) != 0) ? 1 : 0; }
   return v;
 }
 
-// CTAs of the cluster that holds one rod of n elements in the cluster variant (variant 9): n + 1 threads of 512 per CTA
+// CTAs of the cluster that holds one rod of n elements in the cluster variants (9, 10): n + 1 threads of 512 per CTA
 int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
 
-// Rods of 1024-4095 elements (sr_create admits only variant 0's model there) and, with SOFTROD_LEAN_CLUSTER=1, plain
-// lean FP64 rods of 512-1023 elements: one rod per thread-block cluster (rod_kernel_lean.cuh, variant 9)
-bool use_lean_cluster(const sr_handle *h, const sr::RodArgs<double> &A) {
-  if (A.n_elem >= 1024) return true;
-  return cluster_setting() && A.n_elem >= 512 && is_lean_config(A) &&
-         (A.model == sr::MODEL_ROD || A.model == sr::MODEL_SOFT_PENDULUM) && h->cfg.math == SR_MATH_FAST;
+// The cluster variant of rod_kernel_lean.cuh that steps this rod, one rod per thread-block cluster (0: none).  Rods of
+// 1024-4095 elements always take one (sr_create admits variant 0's model and SoftPendulum3D-v0's there: 9 and 10), and
+// so do the filter rods of 768-1023 elements: variant 4 in the 1024-thread CTA they would need takes 243 KB of shared
+// memory, more than a CTA can have.  With SOFTROD_LEAN_CLUSTER=1 so do the other FP64 fast-math rods of 512-1023
+// elements that variant 0 or 4 would step in one CTA.
+int lean_cluster_variant(const sr_handle *h, const sr::RodArgs<double> &A) {
+  if (A.n_elem >= 1024) return A.laplace_order > 0 ? 10 : 9;
+  if (A.n_elem >= 768 && h->cfg.math == SR_MATH_FAST && is_lean_filter_config(A)) return 10;
+  if (!cluster_setting() || A.n_elem < 512 || h->cfg.math != SR_MATH_FAST) return 0;
+  if (is_lean_config(A) && (A.model == sr::MODEL_ROD || A.model == sr::MODEL_SOFT_PENDULUM)) return 9;
+  return is_lean_filter_config(A) ? 10 : 0;
 }
 
 // fast-only kernel + fallback over the envs it flagged, as launch_lean_pair; one cluster per env, no stream-K split
-int launch_lean_cluster(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
+template <int CVAR> int launch_lean_cluster(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
   const int C = lean_cluster_size(A.n_elem);
   A.sk_rods_per_cta = 1; A.sk_items = A.n_env; A.sk_split = 0; A.sk_rodsync = 0;
   A.sk_scratch = nullptr; A.sk_flag = nullptr;
   if (use_fast_pair(h, A, s)) {
-    cudaError_t e = sr::launch_lean_cluster_kernel<true>(A, C, s);
+    cudaError_t e = sr::launch_lean_cluster_kernel<true, CVAR>(A, C, s);
     h->launches++;
     if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
     A.redo_filter = 1;
   }
-  cudaError_t e = sr::launch_lean_cluster_kernel<false>(A, C, s);
+  cudaError_t e = sr::launch_lean_cluster_kernel<false, CVAR>(A, C, s);
   h->launches++;
   if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
   return SR_OK;
@@ -590,6 +595,11 @@ template <typename T> int dispatch_packed(sr_handle *h, sr::RodArgs<T> &A, cudaS
     }
   }
   if constexpr (std::is_same<T, double>::value) {
+    // (ahead of the one-CTA variants: the filter variant's CTAs cannot hold a rod of more than 1023 elements)
+    switch (lean_cluster_variant(h, A)) {
+      case 9: return launch_lean_cluster<9>(h, A, s);
+      case 10: return launch_lean_cluster<10>(h, A, s);
+    }
     if (is_lean_multi_config(A)) {
       switch (packed_threads_setting(h->cfg.n_elem, h->n_rod, h->cfg.has_head)) {
         case 1024: return launch_lean_pair<T, 1024, 1, 3>(h, A, s);
@@ -620,7 +630,6 @@ template <typename T> int dispatch_packed(sr_handle *h, sr::RodArgs<T> &A, cudaS
         default: return launch_lean_pair<T, 256, 2, 4>(h, A, s);
       }
     }
-    if (use_lean_cluster(h, A)) return launch_lean_cluster(h, A, s);
     // a rod of exactly 512 elements: 512 threads with the tip node folded into the last one (128 registers) instead of
     // 513 threads in a 544-thread CTA (96 registers); SOFTROD_LEAN_FOLD=0 switches back (A/B)
     static int fold_off = -1;
@@ -697,15 +706,22 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   if (cfg->n_env <= 0 || cfg->n_elem < 3) return fail(SR_E_INVALID, "sr_create: n_env > 0 and n_elem >= 3 required");
   if (cfg->n_elem > 4095)
     return fail(SR_E_INVALID, "sr_create: n_elem <= 4095 (rods of 1024-4095 elements span a thread-block cluster of up to 8 CTAs)");
+  // rods of 1024-4095 elements: variant 0's model (cluster variant 9) or SoftPendulum3D-v0's (cluster variant 10)
+  const bool long_rod_model =
+      ((cfg->model == SR_MODEL_ROD || cfg->model == SR_MODEL_SOFT_PENDULUM) &&
+       (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED || cfg->bc_kind == SR_BC_PENDULUM_SLIDER) &&
+       cfg->laplace_filter_order == 0) ||
+      (cfg->model == SR_MODEL_SOFT_PENDULUM_3D && cfg->bc_kind == SR_BC_MOVING_BASE && cfg->laplace_filter_order == 7 &&
+       !cfg->point_force_on_base);
   if (cfg->n_elem > 1023 &&
-      (cfg->dtype != SR_DTYPE_F64 || cfg->math != SR_MATH_FAST ||
-       (cfg->model != SR_MODEL_ROD && cfg->model != SR_MODEL_SOFT_PENDULUM) ||
-       (cfg->bc_kind != SR_BC_FREE && cfg->bc_kind != SR_BC_ONE_END_FIXED && cfg->bc_kind != SR_BC_PENDULUM_SLIDER) ||
-       cfg->laplace_filter_order != 0 || cfg->contact_on || cfg->muscle_on || cfg->spline_dir_mask || cfg->n_rod_per_env > 1 ||
-       cfg->has_head || cfg->tip_radius > 0.0 || cfg->sucker_on || cfg->tm_muscle_on || cfg->muscle_layers_on))
+      (cfg->dtype != SR_DTYPE_F64 || cfg->math != SR_MATH_FAST || !long_rod_model || cfg->contact_on || cfg->muscle_on ||
+       cfg->spline_dir_mask || cfg->n_rod_per_env > 1 || cfg->has_head || cfg->tip_radius > 0.0 || cfg->sucker_on ||
+       cfg->tm_muscle_on || cfg->muscle_layers_on))
     return fail(SR_E_INVALID, "sr_create: n_elem of 1024-4095 is built for SR_DTYPE_F64, SR_MATH_FAST, SR_MODEL_ROD or "
                               "SR_MODEL_SOFT_PENDULUM, one untapered rod per env with a free, clamped or slider end, gravity, "
-                              "damping and the base point force; no contact, muscle or spline torques, suckers or Laplace filter");
+                              "damping and the base point force; no contact, muscle or spline torques, suckers or Laplace filter; "
+                              "and for SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE and laplace_filter_order = 7, "
+                              "without the base point force");
   if (cfg->n_elem > 127 && cfg->math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_create: faithful math supports n_elem <= 127");
   if (cfg->dtype != SR_DTYPE_F64 && cfg->dtype != SR_DTYPE_F32) return fail(SR_E_INVALID, "sr_create: bad dtype");
   if (cfg->dtype == SR_DTYPE_F32 && cfg->math != SR_MATH_FAST)
@@ -808,7 +824,8 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   SR_CUDA(cudaSetDevice(cfg->device));
   if (cfg->n_elem > 1023) {
     const int C = lean_cluster_size(cfg->n_elem);
-    if (sr::lean_cluster_max_active(C) < 1)
+    const int n_active = cfg->model == SR_MODEL_SOFT_PENDULUM_3D ? sr::lean_cluster_max_active<10>(C) : sr::lean_cluster_max_active<9>(C);
+    if (n_active < 1)
       return fail(SR_E_CUDA, "sr_create: n_elem = " + std::to_string(cfg->n_elem) + " needs a cluster of " + std::to_string(C) +
                                  " CTAs of 512 threads, and this device cannot launch one");
   }

@@ -68,8 +68,10 @@ typedef struct sr_config {
   int32_t math;         /* SR_MATH_* */
   int32_t n_env;        /* independent environments (one rod each) */
   int32_t n_elem;       /* elements per rod: 3-1023; 1024-4095 (one rod per thread-block cluster of up to 8 CTAs) for
-                         * SR_DTYPE_F64, SR_MATH_FAST, SR_MODEL_ROD / SR_MODEL_SOFT_PENDULUM, one untapered rod per env
-                         * with a free, clamped or slider end, no contact, muscle / spline torques, suckers or filter */
+                         * SR_DTYPE_F64, SR_MATH_FAST, one untapered rod per env without contact, muscle / spline
+                         * torques or suckers, and either SR_MODEL_ROD / SR_MODEL_SOFT_PENDULUM with a free, clamped or
+                         * slider end and no filter, or SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE,
+                         * laplace_filter_order = 7 and no base point force */
   int32_t bc_kind;      /* SR_BC_* */
   int32_t point_force_on_base; /* F_ext[0,0] = action[env,0] each substep (build.py:94-105) */
   int32_t damping_before_constraints; /* 1: [dampen_rates, constrain_rates]; 0 (the envs): [constrain_rates, dampers] = build-code call order */

@@ -1,15 +1,18 @@
-"""Long rods on thread-block clusters (variant 9 of rod_kernel_lean.cuh): device time per launch of K = 100 substeps.
+"""Long rods on thread-block clusters (variants 9 / 10 of rod_kernel_lean.cuh): device time per launch of K = 100 substeps.
 
-Clamped rods (BASELINE config 3's model), with enough envs that the state block exceeds the 126 MB L2 (>= 256 MB).
-Cases: n = 600 and 1023 on the one-CTA kernel (768 / 1024 threads) and on the forced cluster kernel (C = 2), which
+Clamped rods (BASELINE config 3's model, variant 9), or with --model pendulum3d SoftPendulum3D-v0's rod (Laplace filter
+and moving base, variant 10; base held still, 608 FLOP per element-substep), with enough envs that the state block
+exceeds the 126 MB L2 (>= 256 MB).
+Cases: n = 600 and 1023 (SoftPendulum3D: 600 and 767, whose one-CTA kernel ends at 768 threads; 1023 on the cluster
+kernel alone) on the one-CTA kernel (768 / 1024 threads) and on the forced cluster kernel (C = 2), which
 run as alternating subprocesses (SOFTROD_LEAN_CLUSTER is read once per process), two rounds each; n = 1024, 2047 and
 4095, where the cluster kernel is the only one.  Reported: ms per launch (median of 20 CUDA-event-timed launches after
 warm-up), element-substeps/s, and the share of the measured FP64 peak (sr_measure_fp64_peak) at 440 FLOP per
-element-substep.  A probe compiled into a temporary directory reports how many clusters of C one-CTA-per-SM blocks
+element-substep (608 for SoftPendulum3D).  A probe compiled into a temporary directory reports how many clusters of C one-CTA-per-SM blocks
 (512 threads, > 114 KB of shared memory each) the device keeps resident, and so what fraction of the SMs a full wave
 of C-CTA clusters leaves idle.
 
-    python scripts/bench_long_rods.py [--out FILE]     (the report goes to stdout, and to FILE if given)
+    python scripts/bench_long_rods.py [--model rod|pendulum3d] [--out FILE]   (the report goes to stdout, and to FILE if given)
 """
 import argparse
 import json
@@ -20,7 +23,7 @@ import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 K, TIMED, WARMUP = 100, 20, 5
-FLOP_PER_ELEMENT_SUBSTEP = 440
+FLOP_PER_ELEMENT_SUBSTEP = {"rod": 440, "pendulum3d": 608}
 STATE_BYTES = 256 << 20
 
 _PROBE = r"""
@@ -45,7 +48,7 @@ int main() {
 """
 
 
-def one(n, cluster):
+def one(n, cluster, model):
     """Runs in a subprocess of its own: time one case, print one JSON line."""
     import numpy as np
     import torch
@@ -53,25 +56,32 @@ def one(n, cluster):
     from gym_softrobot_b200 import _native as nat
     stride = 32 * ((n + 1 + 31) // 32)
     n_env = -(-STATE_BYTES // (32 * stride * 8))
-    h = nat.Handle(model=nat.MODEL_ROD, n_env=n_env, n_elem=n, dt=2e-6 * 1023 / n, base_length=1.0, base_radius=0.004,
-                   density=1000.0, youngs_modulus=1e6, gravity=(0.0, -9.80665, 0.0), damping_constant=2e-3,
-                   bc_kind=nat.BC_ONE_END_FIXED, math=nat.MATH_FAST)
-    ang = np.deg2rad(np.random.default_rng(n).uniform(-5, 5, n_env))
-    init = np.zeros((n_env, 9))
-    init[:, 3], init[:, 4], init[:, 6], init[:, 7] = np.cos(ang), np.sin(ang), -np.sin(ang), np.cos(ang)
-    h.reset_host(init)
+    act = None
+    if model == "pendulum3d":
+        from gym_softrobot_b200.envs.soft_pendulum_3d import _make_handle, pendulum3d_init_params
+        h = _make_handle(n_env, n, 2e-6 * 1023 / n, K, 0)
+        h.reset_host(pendulum3d_init_params(np.random.default_rng(n).uniform(-1, 1, n_env)))
+        act = torch.zeros((n_env, 2), dtype=torch.float32, device="cuda")
+    else:
+        h = nat.Handle(model=nat.MODEL_ROD, n_env=n_env, n_elem=n, dt=2e-6 * 1023 / n, base_length=1.0,
+                       base_radius=0.004, density=1000.0, youngs_modulus=1e6, gravity=(0.0, -9.80665, 0.0),
+                       damping_constant=2e-3, bc_kind=nat.BC_ONE_END_FIXED, math=nat.MATH_FAST)
+        ang = np.deg2rad(np.random.default_rng(n).uniform(-5, 5, n_env))
+        init = np.zeros((n_env, 9))
+        init[:, 3], init[:, 4], init[:, 6], init[:, 7] = np.cos(ang), np.sin(ang), -np.sin(ang), np.cos(ang)
+        h.reset_host(init)
     obs = torch.empty((n_env, h.obs_dim), dtype=torch.float32, device="cuda")
     rew = torch.empty(n_env, dtype=torch.float64, device="cuda")
     term = torch.empty(n_env, dtype=torch.uint8, device="cuda")
     s = torch.cuda.current_stream()
     for _ in range(WARMUP):
-        h.step(None, K, obs, rew, term)
+        h.step(act, K, obs, rew, term)
     torch.cuda.synchronize()
     times = []
     for _ in range(TIMED):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(s)
-        h.step(None, K, obs, rew, term)
+        h.step(act, K, obs, rew, term)
         e1.record(s)
         e1.synchronize()
         times.append(e0.elapsed_time(e1))
@@ -87,10 +97,11 @@ def one(n, cluster):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=None, help="also write the report to this file")
+    ap.add_argument("--model", choices=sorted(FLOP_PER_ELEMENT_SUBSTEP), default="rod")
     ap.add_argument("--one", nargs=2, type=int, help=argparse.SUPPRESS)
     a = ap.parse_args()
     if a.one:
-        return one(*a.one)
+        return one(*a.one, a.model)
     import torch
     sys.path.insert(0, ROOT)
     from gym_softrobot_b200 import _native as nat
@@ -100,10 +111,11 @@ def main():
     def say(s):
         print(s, flush=True)
         lines.append(s)
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm,clocks.sm", "--format=csv,noheader"],
                          capture_output=True, text=True).stdout.strip()
     sm = torch.cuda.get_device_properties(0).multi_processor_count
-    say(f"device: {torch.cuda.get_device_name(0)}, {sm} SMs; nvidia-smi name, power limit, max SM clock: {smi}")
+    say(f"model: {a.model}; device: {torch.cuda.get_device_name(0)}, {sm} SMs; nvidia-smi name, power limit, max SM "
+        f"clock, SM clock: {smi}")
     peak = nat.measure_fp64_peak(0)
     say(f"measured FP64 peak (sr_measure_fp64_peak): {peak:.2f} TFLOP/s")
     with tempfile.TemporaryDirectory() as tmp:
@@ -116,18 +128,21 @@ def main():
                 c, nc = map(int, line.split())
                 say(f"clusters of {c} one-CTA-per-SM blocks resident at once: {nc} ({nc * c} of {sm} SMs busy, "
                     f"{100.0 * (sm - nc * c) / sm:.1f} % idle)")
-    cases = [(600, 0), (600, 1), (1023, 0), (1023, 1)] * 2 + [(1024, 1), (2047, 1), (4095, 1)]
+    if a.model == "rod":
+        cases = [(600, 0), (600, 1), (1023, 0), (1023, 1)] * 2 + [(1024, 1), (2047, 1), (4095, 1)]
+    else:    # (variant 4's largest CTA is 768 threads: from 768 elements on the cluster variant is the only one)
+        cases = [(600, 0), (600, 1), (767, 0), (767, 1)] * 2 + [(1023, 1), (1024, 1), (2047, 1), (4095, 1)]
     for n, cl in cases:
         env = dict(os.environ)
         env.pop("SOFTROD_LEAN_CLUSTER", None)
         if cl:
             env["SOFTROD_LEAN_CLUSTER"] = "1"
-        out = subprocess.run([sys.executable, os.path.abspath(__file__), "--one", str(n), str(cl)], env=env,
+        out = subprocess.run([sys.executable, os.path.abspath(__file__), "--model", a.model, "--one", str(n), str(cl)], env=env,
                              capture_output=True, text=True)
         if out.returncode != 0:
             raise SystemExit(out.stdout + out.stderr)
         r = json.loads(out.stdout.strip().splitlines()[-1])
-        share = r["elem_substeps_per_s"] * FLOP_PER_ELEMENT_SUBSTEP / (peak * 1e12)
+        share = r["elem_substeps_per_s"] * FLOP_PER_ELEMENT_SUBSTEP[a.model] / (peak * 1e12)
         say(f"n={r['n']:5d} {r['kernel']:8s} C={r['C']} n_env={r['n_env']:5d} state={r['state_MB']} MB: "
             f"{r['ms']:.3f} ms/launch (min {r['ms_min']:.3f}, max {r['ms_max']:.3f}), "
             f"{r['elem_substeps_per_s'] / 1e9:.2f} G element-substeps/s, {100 * share:.1f} % of FP64 peak, "
