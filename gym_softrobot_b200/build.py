@@ -24,7 +24,6 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
 ]
-LEAN_EXTRA_SIZES = [(160, 3), (320, 2)]   # experimental CTA shapes of the lean kernel (SOFTROD_LEAN_THREADS)
 PLANAR_SIZES = [(256, 2), (384, 1), (512, 1)]   # the planar variant (CVAR 8) at the lean kernel's CTA sizes for rods of <= 511 elements
 PACKED_SIZES = [(256, 2), (384, 1), (512, 1), (544, 1), (768, 1), (1024, 1)]   # (threads per CTA, CTAs per SM)
 
@@ -33,11 +32,11 @@ def translation_units():
     """[(object name, source, extra -D flags, header deps)]"""
     tus = [("api", "softrod_api.cu", [], _COMMON), ("warp", "inst_warp.cu", [], _COMMON)]
     for t in ("double", "float"):
-        for nt, minb in LEAN_EXTRA_SIZES + PACKED_SIZES:
+        for nt, minb in PACKED_SIZES:
             tus.append((f"lean_{t}_{nt}", "inst_lean.cu", [f"-DSR_TU_T={t}", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}"],
                         _COMMON + ["rod_kernel_lean.cuh"]))
     for nt, minb in PACKED_SIZES:      # the lean kernel's contact variant (FP64): plain, with the travelling-wave muscle, for assemblies; 4 = filter + moving base; 5 = spline torques
-        for cv in (1, 2, 3, 4, 5):
+        for cv in (1, 2, 3, 4, 5) if nt <= 768 else (1, 2, 3, 5):   # (filter rods of >= 768 elements take variant 10)
             tus.append((f"leanc{cv}_double_{nt}", "inst_lean.cu", ["-DSR_TU_T=double", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", f"-DSR_TU_CONTACT={cv}"],
                         _COMMON + ["rod_kernel_lean.cuh"]))
     for nt, minb in PLANAR_SIZES:     # variant 0 for rods in the x-y plane (fast-only kernel; FP64)

@@ -116,7 +116,9 @@ template <typename T> struct RodArgs {
   int lim_rot_hi, lim_bend_hi, lim_em1_hi;   // range limits as high words (integer-pipe compares)
   // stream-K schedule: items of sk_rods_per_cta envs; sk_split = slots own equal substep ranges and hand partial
   // items over through sk_scratch[slot][18][NT] / sk_flag[slot]
-  int sk_rods_per_cta, sk_items, sk_split, sk_rodsync;   // sk_rodsync: per-rod named barriers inside the substep loop
+  // sk_rodsync: per-rod named barriers inside the substep loop where the layout allows them; always 1 (fill_args), but
+  // kept a run-time operand: folding it into the barrier choice changes ptxas's register allocation and spills
+  int sk_rods_per_cta, sk_items, sk_split, sk_rodsync;
   double *sk_scratch; int *sk_flag;
   // ---- COOMM muscle layers with per-element activations (LMUS instantiation of the packed kernel; OctoReach-v0 /
   // OctoArmTwo-v0: reach_env.py:214-227, arm_two_env.py:222-247, create_es_muscle_layers build.py:292-338) ----

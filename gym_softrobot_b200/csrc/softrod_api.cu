@@ -112,6 +112,7 @@ template <typename T> void fill_args(const sr_config &c, int stride, sr::RodArgs
   A.base_step_f32 = (float)c.base_step;
   A.rest_kappa = nullptr;
   A.n_rod = c.n_rod_per_env > 1 ? c.n_rod_per_env : 1; A.has_head = c.has_head; A.head = nullptr;
+  A.sk_rodsync = 1;
   A.joint_k = (T)c.joint_k; A.joint_nu = (T)c.joint_nu; A.joint_kt = (T)c.joint_kt; A.joint_radius = (T)c.joint_radius;
   for (int a = 0; a < 16; a++) {   // z_rotation(): theta = angle / 180 * pi
     double th = c.joint_angle_deg[a] / 180.0 * PI;
@@ -241,22 +242,21 @@ int cuda_fail(const char *what, cudaError_t e) {
   return fail(SR_E_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
 
-int fastpath_setting() {   // SOFTROD_FASTPATH=0: single safe kernel with per-thread fallbacks (experiments; same bits)
-  static int v = -1;
-  if (v < 0) { const char *e = getenv("SOFTROD_FASTPATH"); v = e ? atoi(e) != 0 : 1; }
-  return v;
-}
-
-int rodsync_setting() {    // SOFTROD_RODSYNC=0: CTA-wide barriers instead of per-rod named barriers (experiments; same bits)
-  static int v = -1;
-  if (v < 0) { const char *e = getenv("SOFTROD_RODSYNC"); v = e ? atoi(e) != 0 : 1; }
-  return v;
-}
-
-int streamk_setting() {    // SOFTROD_STREAMK=0: one CTA per item instead of equal substep ranges per slot (experiments; same bits)
-  static int v = -1;
-  if (v < 0) { const char *e = getenv("SOFTROD_STREAMK"); v = e ? atoi(e) != 0 : 1; }
-  return v;
+// The run-time switches, read once per process.  Each picks between kernels that give every env the same bits (FOLD:
+// outside the padding slots); the default is the measured winner, the other serves as the reference in tests and A/B runs.
+struct Switches {
+  bool fastpath;   // SOFTROD_FASTPATH=0: the single safe kernel with per-thread fallbacks instead of the pair
+  bool planar;     // SOFTROD_LEAN_PLANAR=0: rods in the x-y plane take the 3D kernels too
+  bool cluster;    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster variants too
+  bool fold;       // SOFTROD_LEAN_FOLD=0: a rod of 512 elements takes a 544-thread CTA instead of the folded-tip variant
+};
+const Switches &switches() {
+  static const Switches s = [] {
+    auto on = [](const char *name, bool dflt) { const char *e = getenv(name); return e ? atoi(e) != 0 : dflt; };
+    return Switches{on("SOFTROD_FASTPATH", true), on("SOFTROD_LEAN_PLANAR", true), on("SOFTROD_LEAN_CLUSTER", false),
+                    on("SOFTROD_LEAN_FOLD", true)};
+  }();
+  return s;
 }
 
 // Whether this step runs the fast-only kernel + fallback pair.  Both ways give every env the same bits (the safe
@@ -267,7 +267,7 @@ int streamk_setting() {    // SOFTROD_STREAMK=0: one CTA per item instead of equ
 // when more than 1 % of a window's env-steps fell back (violently actuated arms do) the handle uses the single
 // safe kernel for the next 512 steps, then probes again.
 template <typename T> bool use_fast_pair(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
-  if (!fastpath_setting() || !A.redo) return false;
+  if (!switches().fastpath || !A.redo) return false;
   h->pair_steps++;
   if (h->pair_off_until > h->pair_steps) return false;
   cudaError_t q = h->pair_copy_pending ? cudaEventQuery(h->pair_event) : cudaErrorNotReady;
@@ -280,7 +280,7 @@ template <typename T> bool use_fast_pair(sr_handle *h, sr::RodArgs<T> &A, cudaSt
     h->pair_last_count = seen;
     h->planar_last_count = seen_np;
     h->pair_steps_at_prev_copy = h->pair_steps_at_copy;
-    // the same rule for envs that are not planar: the handle steps with the 3D pair for a while (see use_planar)
+    // the same rule for envs that are not planar: the handle steps with the 3D pair for a while (see launch_lean)
     if (window > 0 && (double)delta_np > 0.01 * (double)window) h->planar_off_until = h->pair_steps + 512;
     if (window > 0 && (double)delta > 0.01 * (double)window) { h->pair_off_until = h->pair_steps + 512; return false; }
   }
@@ -294,6 +294,88 @@ template <typename T> bool use_fast_pair(sr_handle *h, sr::RodArgs<T> &A, cudaSt
   return true;
 }
 
+// The one pair runner: the fast-only kernel, then the safe one over the envs it flagged (an empty launch in the normal
+// case), or the safe kernel alone.  use_fast_pair is asked only for a kernel that pairs, since asking advances the
+// pair's step count, its polling of the fallback counts and its windows.  launch(std::true_type()) launches the
+// fast-only kernel, launch(std::false_type()) the safe one.
+template <typename T, typename L> int run_pair(sr_handle *h, sr::RodArgs<T> &A, bool pair, cudaStream_t s, L &&launch) {
+  if (pair && use_fast_pair(h, A, s)) {
+    const int rc = launch(std::true_type());
+    if (rc != SR_OK) return rc;
+    A.redo_filter = 1;
+  }
+  return launch(std::false_type());
+}
+
+// The one CTA-size dispatcher: a run-time CTA size to the <NT, MINB> template arguments of the sizes build.py compiles
+// (PACKED_SIZES; MINB = the resident CTAs per SM the kernels are compiled for).
+template <int NT_, int MINB_> struct Cta { static constexpr int NT = NT_, MINB = MINB_; };
+template <typename F> int with_cta(int nt, F &&launch) {
+  switch (nt) {
+    case 256: return launch(Cta<256, 2>());
+    case 384: return launch(Cta<384, 1>());
+    case 512: return launch(Cta<512, 1>());
+    case 544: return launch(Cta<544, 1>());
+    case 768: return launch(Cta<768, 1>());
+    case 1024: return launch(Cta<1024, 1>());
+  }
+  return fail(SR_E_INVALID, "no kernel is built for CTAs of " + std::to_string(nt) + " threads");
+}
+
+// Of those sizes, the ones build.py compiles lean variant CV at: the folded-tip variants at 512 threads only, the planar
+// variant up to 512 and the filter variant up to 768 (its 1024-thread CTA would need 243 KB of shared memory).
+constexpr bool lean_built(int cv, int nt) {
+  return (cv == 6 || cv == 7) ? nt == 512 : cv == 8 ? nt <= 512 : cv == 4 ? nt <= 768 : true;
+}
+
+// CTA size of the generic kernel and of the assembly variant.  Registers cap the SM at 512 resident threads (128 regs),
+// so the choice is 2 x 256 or 1 x 512; take whichever wastes fewer lanes for this rod length
+// (n = 50: 5 x 51 = 255/256; n = 100: 2 x 101 = 202/256 but 5 x 101 = 505/512).
+int packed_threads_setting(int n_elem, int n_rod = 1, int has_head = 0) {
+  const int tpr = (n_rod > 1 ? n_rod : 1) * (n_elem + 1) + has_head;   // threads per env group
+  auto util = [&](int nt) { return (double)((nt / tpr) * tpr) / nt; };
+  // 2 x 256 (128 regs) is the default; 1 x 384 (168 regs) / 1 x 512 (128 regs) only when they waste
+  // clearly fewer lanes for this group size
+  int best = 256;
+  if (util(384) > util(best) + 0.02) best = 384;
+  if (util(512) > util(best) + 0.02) best = 512;
+  // long rods: one rod per CTA, as few warps as hold it so that each thread keeps as many registers as
+  // possible (544 threads: 120 registers, 768: 80, 1024: 64)
+  if (tpr > 512) best = tpr <= 544 ? 544 : (tpr <= 768 ? 768 : 1024);
+  return best;
+}
+
+// CTA size of the one-CTA lean variants of a single rod.  With per-rod barriers one 512-thread CTA per SM (16 warps,
+// 10 rods of n = 50) beats two of 256 (measured: 1.51 vs 1.64 ms per 4096-env step): take 512 whenever it wastes no
+// more lanes.
+int lean_threads_setting(int n_elem) {
+  const int tpr = n_elem + 1;
+  if (tpr > 512) return packed_threads_setting(n_elem);
+  auto util = [&](int nt) { return (double)((nt / tpr) * tpr) / nt; };
+  int best = 512;
+  if (util(384) > util(best) + 0.02) best = 384;
+  if (util(256) > util(best) + 0.02) best = 256;
+  return best;
+}
+
+// CTAs of the cluster that holds one rod of n elements in the cluster variants (9, 10): n + 1 threads of 512 per CTA
+int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
+
+// The cluster variant that steps a rod of the plain model (9: variant 0's substep) or of SoftPendulum3D-v0's (10:
+// variant 4's, with the Laplace filter and the moving base).  sr_create checks its cluster shape for rods of
+// 1024-4095 elements, the only models it admits there.
+int lean_cluster_variant(int laplace_order, int bc_kind) {
+  return laplace_order > 0 || bc_kind == sr::BC_MOVING_BASE ? 10 : 9;
+}
+
+// What steps a handle (classify): the launcher of one kernel, and the launch's shape.
+template <typename T> struct StepKernel {
+  int (*launch)(sr_handle *, sr::RodArgs<T> &, const StepKernel &, cudaStream_t);
+  int nt;        // CTA size of the one-CTA lean variants and the generic kernel
+  bool pair;     // fast-only kernel + fallback (run_pair)
+  bool planar;   // lean variant 0: the fast-only kernel is the planar variant 8 while the handle's planar window allows
+};
+
 template <typename T, int NT, int MINB, bool LAPLACE, bool MOVING, bool CONTACT, bool MULTI, bool TORQUE = false,
           bool FASTONLY = false>
 int launch_packed_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
@@ -301,7 +383,6 @@ int launch_packed_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
   const int rods_per_cta = NT / group;
   if (rods_per_cta < 1) return fail(SR_E_INVALID, "environment does not fit one CTA of the packed kernel");
   const int grid = (A.n_env + rods_per_cta - 1) / rods_per_cta;
-  A.sk_rodsync = rodsync_setting();
   cudaError_t e = sr::launch_packed_kernel<T, NT, MINB, LAPLACE, MOVING, CONTACT, MULTI, TORQUE, FASTONLY>(A, rods_per_cta, grid, s);
   h->launches++;
   if (e != cudaSuccess) return cuda_fail("rod_packed_kernel launch", e);
@@ -337,9 +418,8 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int laun
     h->sk_slots = slots;
   }
   A.sk_rods_per_cta = rods_per_cta; A.sk_items = items;
-  A.sk_split = (streamk_setting() && !A.redo_filter && items > slots && A.n_substeps > 0) ? 1 : 0;
+  A.sk_split = (!A.redo_filter && items > slots && A.n_substeps > 0) ? 1 : 0;
   A.sk_scratch = (double *)h->sk_scratch; A.sk_flag = h->sk_flag;
-  A.sk_rodsync = rodsync_setting();
   const int grid = A.sk_split ? slots : items;
   cudaError_t e = sr::launch_lean_kernel<T, NT, MINB, FASTONLY, CONTACT>(A, grid, s);
   h->launches++;
@@ -347,140 +427,62 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int laun
   return SR_OK;
 }
 
-int planar_setting() {     // SOFTROD_LEAN_PLANAR=0: rods in the x-y plane take the 3D kernels too (A/B; same bits)
-  static int v = -1;
-  if (v < 0) { const char *e = getenv("SOFTROD_LEAN_PLANAR"); v = e ? atoi(e) != 0 : 1; }
-  return v;
+// one-CTA lean variant CV of rod_kernel_lean.cuh in CTAs of k.nt threads
+template <typename T, int CV> int launch_lean(sr_handle *h, sr::RodArgs<T> &A, const StepKernel<T> &k, cudaStream_t s) {
+  return with_cta(k.nt, [&](auto cta) {
+    using C = decltype(cta);
+    if constexpr (!lean_built(CV, C::NT)) {
+      return fail(SR_E_INVALID, "rod_lean_kernel: variant " + std::to_string(CV) + " is not built for " + std::to_string(C::NT) + " threads");
+    } else {
+      return run_pair(h, A, k.pair, s, [&](auto fast) {
+        constexpr bool FAST = decltype(fast)::value;
+        if constexpr (FAST && CV == 0 && std::is_same<T, double>::value && lean_built(8, C::NT)) {
+          // when more than 1 % of a window's env-steps were handed over for not being planar, the handle steps with
+          // the 3D pair for the next 512 steps (use_fast_pair)
+          if (k.planar && h->pair_steps >= h->planar_off_until) return launch_lean_impl<T, C::NT, C::MINB, true, 8>(h, A, s);
+        }
+        return launch_lean_impl<T, C::NT, C::MINB, FAST, CV>(h, A, s);
+      });
+    }
+  });
 }
 
-// Whether the fast-only kernel of a pair may be the planar variant (CVAR 8).  It needs a model whose out-of-plane
-// components stay exact zeros once the state has them: the plain lean model in FP64 with the fast maps, gravity in the
-// x-y plane, the base point force along x (the only direction the kernel applies it in), and a BC that pins in-plane
-// rows (slider, clamp) or none.  The state itself is checked by the kernel, per rod; when more than 1 % of a window's
-// env-steps are handed over for not being planar, the handle uses the 3D pair for the next 512 steps (use_fast_pair).
-template <typename T> bool is_lean_config(const sr::RodArgs<T> &A);
-template <typename T> bool use_planar(const sr_handle *h, const sr::RodArgs<T> &A) {
-  if (!std::is_same<T, double>::value || !planar_setting() || !is_lean_config(A)) return false;
-  if (h->cfg.math != SR_MATH_FAST || (double)A.gdt_cv[2] != 0.0) return false;
-  if (A.bc_kind != sr::BC_FREE && A.bc_kind != sr::BC_ONE_END_FIXED && A.bc_kind != sr::BC_PENDULUM_SLIDER) return false;
-  return h->pair_steps >= h->planar_off_until;
-}
-
-template <typename T, int NT, int MINB, int CONTACT = 0> int launch_lean_pair(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
-  if (use_fast_pair(h, A, s)) {
-    // fast-only kernel, then the safe one over the envs it flagged (an empty launch in the normal case)
-    int rc;
-    if constexpr (std::is_same<T, double>::value && CONTACT == 0 && NT <= 512 && NT % 128 == 0)
-      rc = use_planar(h, A) ? launch_lean_impl<T, NT, MINB, true, 8>(h, A, s) : launch_lean_impl<T, NT, MINB, true, CONTACT>(h, A, s);
-    else
-      rc = launch_lean_impl<T, NT, MINB, true, CONTACT>(h, A, s);
-    if (rc != SR_OK) return rc;
-    A.redo_filter = 1;
-  }
-  return launch_lean_impl<T, NT, MINB, false, CONTACT>(h, A, s);
-}
-
-// single rod on the frictional plane / with rest-curvature actuation / travelling-wave muscle: the lean kernel's contact
-// variant (FP64).  Everything else the generic kernel offers (spline forcing, suckers, external loads, tapered rods,
-// assemblies, the moving base, the Laplace filter, the base point force) stays with rod_kernel_packed.cuh.
-template <typename T> bool is_lean_contact_config(const sr::RodArgs<T> &A) {
-  if (!std::is_same<T, double>::value) return false;
-  static int off = -1;
-  if (off < 0) { const char *e = getenv("SOFTROD_LEAN_CONTACT"); off = (e && atoi(e) == 0) ? 1 : 0; }   // =0: generic kernel (A/B)
-  if (off) return false;
-  if (A.n_rod > 1 || A.has_head || A.spline_mask || A.laplace_order > 0 || A.sucker || A.ext_force || A.ext_couple || A.elem_tab ||
-      A.point_force) return false;
-  if (A.bc_kind != sr::BC_FREE && A.bc_kind != sr::BC_ONE_END_FIXED) return false;
-  return A.contact_on || A.rest_kappa || A.muscle_on;
-}
-
-// SoftPendulum3D-v0's model: LaplaceDissipationFilter (order 7, or none) + moving base or clamp, no contact: variant 4
-template <typename T> bool is_lean_filter_config(const sr::RodArgs<T> &A) {
-  if (!std::is_same<T, double>::value) return false;
-  static int off = -1;
-  if (off < 0) { const char *e = getenv("SOFTROD_LEAN_FILTER"); off = (e && atoi(e) == 0) ? 1 : 0; }   // =0: generic kernel (A/B)
-  if (off) return false;
-  if (A.n_rod > 1 || A.has_head || A.spline_mask || A.muscle_on || A.contact_on || A.rest_kappa || A.sucker || A.ext_force ||
-      A.ext_couple || A.elem_tab || A.point_force) return false;
-  if (!(A.laplace_order == 7 || (A.laplace_order == 0 && A.bc_kind == sr::BC_MOVING_BASE))) return false;
-  if (A.bc_kind != sr::BC_MOVING_BASE && A.bc_kind != sr::BC_ONE_END_FIXED && A.bc_kind != sr::BC_FREE) return false;
-  return A.n_elem >= 8;     // (the filter's ghost records assume one reflection per end)
-}
-
-// SoftArmTracking-v0's model: clamped / free rod + spline muscle torques, nothing else: variant 5 (safe kernel only)
-template <typename T> bool is_lean_spline_config(const sr::RodArgs<T> &A) {
-  if (!std::is_same<T, double>::value) return false;
-  static int off = -1;
-  if (off < 0) { const char *e = getenv("SOFTROD_LEAN_SPLINE"); off = (e && atoi(e) == 0) ? 1 : 0; }   // =0: generic kernel (A/B)
-  if (off) return false;
-  if (!A.spline_mask || A.n_rod > 1 || A.has_head || A.muscle_on || A.contact_on || A.rest_kappa || A.sucker || A.ext_force ||
-      A.ext_couple || A.elem_tab || A.point_force || A.laplace_order > 0) return false;
-  return A.bc_kind == sr::BC_ONE_END_FIXED || A.bc_kind == sr::BC_FREE;
-}
-
-// assemblies (OctoFlat: arms + rigid head + FixedJoint2Rigid joints on the plane): the lean kernel's third contact variant
-template <typename T> bool is_lean_multi_config(const sr::RodArgs<T> &A) {
-  if (!std::is_same<T, double>::value) return false;
-  static int off = -1;
-  if (off < 0) { const char *e = getenv("SOFTROD_LEAN_MULTI"); off = (e && atoi(e) == 0) ? 1 : 0; }   // =0: generic kernel (A/B)
-  if (off) return false;
-  if (!(A.n_rod > 1 || A.has_head)) return false;
-  if (A.spline_mask || A.muscle_on || A.laplace_order > 0 || A.sucker || A.ext_force || A.ext_couple || A.elem_tab || A.point_force) return false;
-  return A.bc_kind == sr::BC_FREE && A.rot_on == 0;
-}
-
-template <typename T> bool is_lean_config(const sr::RodArgs<T> &A) {
-  return !(A.n_rod > 1 || A.has_head || A.muscle_on || A.spline_mask || A.contact_on || A.rest_kappa ||
-           A.laplace_order > 0 || A.bc_kind == sr::BC_MOVING_BASE || A.sucker || A.ext_force || A.ext_couple || A.elem_tab);
-}
-
-int cluster_setting() {    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster variants too (A/B; same bits)
-  static int v = -1;
-  if (v < 0) { const char *e = getenv("SOFTROD_LEAN_CLUSTER"); v = (e && atoi(e) != 0) ? 1 : 0; }
-  return v;
-}
-
-// CTAs of the cluster that holds one rod of n elements in the cluster variants (9, 10): n + 1 threads of 512 per CTA
-int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
-
-// The cluster variant of rod_kernel_lean.cuh that steps this rod, one rod per thread-block cluster (0: none).  Rods of
-// 1024-4095 elements always take one (sr_create admits variant 0's model and SoftPendulum3D-v0's there: 9 and 10), and
-// so do the filter rods of 768-1023 elements: variant 4 in the 1024-thread CTA they would need takes 243 KB of shared
-// memory, more than a CTA can have.  With SOFTROD_LEAN_CLUSTER=1 so do the other FP64 fast-math rods of 512-1023
-// elements that variant 0 or 4 would step in one CTA.
-int lean_cluster_variant(const sr_handle *h, const sr::RodArgs<double> &A) {
-  if (A.n_elem >= 1024) return A.laplace_order > 0 ? 10 : 9;
-  if (A.n_elem >= 768 && h->cfg.math == SR_MATH_FAST && is_lean_filter_config(A)) return 10;
-  if (!cluster_setting() || A.n_elem < 512 || h->cfg.math != SR_MATH_FAST) return 0;
-  if (is_lean_config(A) && (A.model == sr::MODEL_ROD || A.model == sr::MODEL_SOFT_PENDULUM)) return 9;
-  return is_lean_filter_config(A) ? 10 : 0;
-}
-
-// fast-only kernel + fallback over the envs it flagged, as launch_lean_pair; one cluster per env, no stream-K split
-template <int CVAR> int launch_lean_cluster(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
+// cluster variant CV: one rod per thread-block cluster, no stream-K split
+template <int CV> int launch_cluster(sr_handle *h, sr::RodArgs<double> &A, const StepKernel<double> &k, cudaStream_t s) {
   const int C = lean_cluster_size(A.n_elem);
-  A.sk_rods_per_cta = 1; A.sk_items = A.n_env; A.sk_split = 0; A.sk_rodsync = 0;
+  A.sk_rods_per_cta = 1; A.sk_items = A.n_env; A.sk_split = 0;
   A.sk_scratch = nullptr; A.sk_flag = nullptr;
-  if (use_fast_pair(h, A, s)) {
-    cudaError_t e = sr::launch_lean_cluster_kernel<true, CVAR>(A, C, s);
+  return run_pair(h, A, k.pair, s, [&](auto fast) {
+    cudaError_t e = sr::launch_lean_cluster_kernel<decltype(fast)::value, CV>(A, C, s);
     h->launches++;
     if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
-    A.redo_filter = 1;
-  }
-  cudaError_t e = sr::launch_lean_cluster_kernel<false, CVAR>(A, C, s);
-  h->launches++;
-  if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
-  return SR_OK;
+    return SR_OK;
+  });
+}
+
+// the generic kernel (rod_kernel_packed.cuh) with the features of one group
+enum { G_FILTER, G_CONTACT, G_TORQUE, G_MULTI };   // Laplace filter + moving base / plane contact / + forcing torques / assemblies
+template <typename T, int G> int launch_generic(sr_handle *h, sr::RodArgs<T> &A, const StepKernel<T> &k, cudaStream_t s) {
+  return with_cta(k.nt, [&](auto cta) {
+    using C = decltype(cta);
+    return run_pair(h, A, k.pair, s, [&](auto fast) {
+      constexpr bool FAST = decltype(fast)::value;
+      if constexpr (FAST && !std::is_same<T, double>::value) {
+        return fail(SR_E_INVALID, "rod_packed_kernel: the fast-only kernel is built for FP64 only");
+      } else {
+        return launch_packed_impl<T, C::NT, C::MINB, G == G_FILTER, G == G_FILTER, G != G_FILTER, G == G_MULTI, G == G_TORQUE, FAST>(h, A, s);
+      }
+    });
+  });
 }
 
 // tapered rods: safe kernel with per-element constants in registers (CTA sizes 384 / 1024 only)
-template <int NT> int launch_tapered(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
+template <int NT> int launch_tapered(sr_handle *h, sr::RodArgs<double> &A, const StepKernel<double> &, cudaStream_t s) {
   const bool multi = A.n_rod > 1 || A.has_head;
   const int group = (multi ? A.n_rod : 1) * (A.n_elem + 1) + (multi ? A.has_head : 0);
   const int rods_per_cta = NT / group;
   if (rods_per_cta < 1) return fail(SR_E_INVALID, "environment does not fit one CTA of the packed kernel");
   const int grid = (A.n_env + rods_per_cta - 1) / rods_per_cta;
-  A.sk_rodsync = rodsync_setting();
   if (A.mus_act) {
     if (NT != 384 || !multi) return fail(SR_E_INVALID, "muscle layers: multi-rod assemblies of at most 384 threads only");
     cudaError_t el = sr::launch_packed_lmus_kernel<384>(A, rods_per_cta, grid, s);
@@ -495,193 +497,8 @@ template <int NT> int launch_tapered(sr_handle *h, sr::RodArgs<double> &A, cudaS
   return SR_OK;
 }
 
-template <typename T, int NT, int MINB> int launch_packed(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
-  constexpr bool F64 = std::is_same<T, double>::value;
-  if (A.n_rod > 1 || A.has_head) {
-    if constexpr (F64) {
-      if (use_fast_pair(h, A, s)) {
-        int rc = launch_packed_impl<T, NT, MINB, false, false, true, true, false, true>(h, A, s);
-        if (rc != SR_OK) return rc;
-        A.redo_filter = 1;
-      }
-    }
-    return launch_packed_impl<T, NT, MINB, false, false, true, true>(h, A, s);
-  }
-  if (A.muscle_on || A.spline_mask) {
-    if constexpr (F64) {
-      // (the spline forcing updates its cached control values / magnitudes inside the launch: safe kernel only)
-      if (!A.spline_mask && use_fast_pair(h, A, s)) {
-        int rc = launch_packed_impl<T, NT, MINB, false, false, true, false, true, true>(h, A, s);
-        if (rc != SR_OK) return rc;
-        A.redo_filter = 1;
-      }
-    }
-    return launch_packed_impl<T, NT, MINB, false, false, true, false, true>(h, A, s);
-  }
-  if (A.contact_on || A.rest_kappa || A.sucker || A.ext_force || A.ext_couple) {
-    if constexpr (F64) {
-      if (use_fast_pair(h, A, s)) {
-        int rc = launch_packed_impl<T, NT, MINB, false, false, true, false, false, true>(h, A, s);
-        if (rc != SR_OK) return rc;
-        A.redo_filter = 1;
-      }
-    }
-    return launch_packed_impl<T, NT, MINB, false, false, true, false>(h, A, s);
-  }
-  if (A.laplace_order > 0 || A.bc_kind == sr::BC_MOVING_BASE) {
-    if constexpr (F64) {
-      if (use_fast_pair(h, A, s)) {
-        int rc = launch_packed_impl<T, NT, MINB, true, true, false, false, false, true>(h, A, s);
-        if (rc != SR_OK) return rc;
-        A.redo_filter = 1;
-      }
-    }
-    return launch_packed_impl<T, NT, MINB, true, true, false, false>(h, A, s);
-  }
-  return launch_lean_pair<T, NT, MINB>(h, A, s);   // lean configs (FP64, and FP32 storage = mixed precision): rod_kernel_lean.cuh
-}
-
-// CTA size of the packed kernels.  Registers cap the SM at 512 resident threads (128 regs), so the
-// choice is 2 x 256 or 1 x 512; take whichever wastes fewer lanes for this rod length
-// (n = 50: 5 x 51 = 255/256; n = 100: 2 x 101 = 202/256 but 5 x 101 = 505/512).
-// SOFTROD_PACKED_THREADS={256,384,512} overrides it for experiments.
-int packed_threads_setting(int n_elem, int n_rod = 1, int has_head = 0) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char *e = getenv("SOFTROD_PACKED_THREADS");
-    forced = e ? atoi(e) : 0;
-    if (forced != 256 && forced != 384 && forced != 512 && forced != 544 && forced != 768 && forced != 1024) forced = 0;
-  }
-  const int tpr = (n_rod > 1 ? n_rod : 1) * (n_elem + 1) + has_head;   // threads per env group
-  if (forced && forced >= tpr) return forced;
-  auto util = [&](int nt) { return (double)((nt / tpr) * tpr) / nt; };
-  // 2 x 256 (128 regs) is the default; 1 x 384 (168 regs) / 1 x 512 (128 regs) only when they waste
-  // clearly fewer lanes for this group size
-  int best = 256;
-  if (util(384) > util(best) + 0.02) best = 384;
-  if (util(512) > util(best) + 0.02) best = 512;
-  // long rods: one rod per CTA, as few warps as hold it so that each thread keeps as many registers as
-  // possible (544 threads: 120 registers, 768: 80, 1024: 64)
-  if (tpr > 512) best = tpr <= 544 ? 544 : (tpr <= 768 ? 768 : 1024);
-  return best;
-}
-
-int lean_threads_override() {   // SOFTROD_LEAN_THREADS={160,320}: experimental CTA shapes of the lean FP64 kernel (3 x 160, 2 x 320)
-  static int v = -1;
-  if (v < 0) { const char *e = getenv("SOFTROD_LEAN_THREADS"); v = e ? atoi(e) : 0; }
-  return v;
-}
-
-// CTA size of the lean FP64 kernel.  With per-rod barriers one 512-thread CTA per SM (16 warps, 10 rods of n = 50)
-// beats two of 256 (measured: 1.51 vs 1.64 ms per 4096-env step): take 512 whenever it wastes no more lanes.
-int lean_threads_setting(int n_elem) {
-  const int tpr = n_elem + 1;
-  if (tpr > 512) return packed_threads_setting(n_elem);
-  static int forced = -1;
-  if (forced < 0) { const char *e = getenv("SOFTROD_PACKED_THREADS"); forced = e ? atoi(e) : 0; }
-  if ((forced == 256 || forced == 384 || forced == 512) && forced >= tpr) return forced;
-  auto util = [&](int nt) { return (double)((nt / tpr) * tpr) / nt; };
-  int best = 512;
-  if (util(384) > util(best) + 0.02) best = 384;
-  if (util(256) > util(best) + 0.02) best = 256;
-  return best;
-}
-
-template <typename T> int dispatch_packed(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
-  if constexpr (std::is_same<T, double>::value) {
-    if (A.elem_tab) {
-      const int group = h->n_rod * (h->cfg.n_elem + 1) + (h->cfg.has_head ? 1 : 0);
-      return group <= 384 ? launch_tapered<384>(h, A, s) : launch_tapered<1024>(h, A, s);
-    }
-  }
-  if constexpr (std::is_same<T, double>::value) {
-    // (ahead of the one-CTA variants: the filter variant's CTAs cannot hold a rod of more than 1023 elements)
-    switch (lean_cluster_variant(h, A)) {
-      case 9: return launch_lean_cluster<9>(h, A, s);
-      case 10: return launch_lean_cluster<10>(h, A, s);
-    }
-    if (is_lean_multi_config(A)) {
-      switch (packed_threads_setting(h->cfg.n_elem, h->n_rod, h->cfg.has_head)) {
-        case 1024: return launch_lean_pair<T, 1024, 1, 3>(h, A, s);
-        case 768: return launch_lean_pair<T, 768, 1, 3>(h, A, s);
-        case 544: return launch_lean_pair<T, 544, 1, 3>(h, A, s);
-        case 512: return launch_lean_pair<T, 512, 1, 3>(h, A, s);
-        case 384: return launch_lean_pair<T, 384, 1, 3>(h, A, s);
-        default: return launch_lean_pair<T, 256, 2, 3>(h, A, s);
-      }
-    }
-    if (is_lean_spline_config(A)) {   // (mutates the forcing's cache inside the launch: no fast-only / redo pair)
-      switch (lean_threads_setting(h->cfg.n_elem)) {
-        case 1024: return launch_lean_impl<T, 1024, 1, false, 5>(h, A, s);
-        case 768: return launch_lean_impl<T, 768, 1, false, 5>(h, A, s);
-        case 544: return launch_lean_impl<T, 544, 1, false, 5>(h, A, s);
-        case 512: return launch_lean_impl<T, 512, 1, false, 5>(h, A, s);
-        case 384: return launch_lean_impl<T, 384, 1, false, 5>(h, A, s);
-        default: return launch_lean_impl<T, 256, 2, false, 5>(h, A, s);
-      }
-    }
-    if (is_lean_filter_config(A)) {
-      switch (lean_threads_setting(h->cfg.n_elem)) {
-        case 1024: return launch_lean_pair<T, 1024, 1, 4>(h, A, s);
-        case 768: return launch_lean_pair<T, 768, 1, 4>(h, A, s);
-        case 544: return launch_lean_pair<T, 544, 1, 4>(h, A, s);
-        case 512: return launch_lean_pair<T, 512, 1, 4>(h, A, s);
-        case 384: return launch_lean_pair<T, 384, 1, 4>(h, A, s);
-        default: return launch_lean_pair<T, 256, 2, 4>(h, A, s);
-      }
-    }
-    // a rod of exactly 512 elements: 512 threads with the tip node folded into the last one (128 registers) instead of
-    // 513 threads in a 544-thread CTA (96 registers); SOFTROD_LEAN_FOLD=0 switches back (A/B)
-    static int fold_off = -1;
-    if (fold_off < 0) { const char *e = getenv("SOFTROD_LEAN_FOLD"); fold_off = (e && atoi(e) == 0) ? 1 : 0; }
-    if (!fold_off && A.n_elem == 512 && A.model == sr::MODEL_ROD && !A.muscle_on) {
-      if (is_lean_contact_config(A)) return launch_lean_pair<T, 512, 1, 7>(h, A, s);
-      if (is_lean_config(A)) return launch_lean_pair<T, 512, 1, 6>(h, A, s);
-    }
-    if (is_lean_contact_config(A)) {
-      const int nt = lean_threads_setting(h->cfg.n_elem);
-#define SR_LEANC(NT_, MB_) (A.muscle_on ? launch_lean_pair<T, NT_, MB_, 2>(h, A, s) : launch_lean_pair<T, NT_, MB_, 1>(h, A, s))
-      switch (nt) {
-        case 1024: return SR_LEANC(1024, 1);
-        case 768: return SR_LEANC(768, 1);
-        case 544: return SR_LEANC(544, 1);
-        case 512: return SR_LEANC(512, 1);
-        case 384: return SR_LEANC(384, 1);
-        default: return SR_LEANC(256, 2);
-      }
-#undef SR_LEANC
-    }
-  }
-  if (is_lean_config(A)) {
-    if (A.n_elem + 1 <= 160) {
-      if (lean_threads_override() == 160) return launch_lean_pair<T, 160, 3>(h, A, s);
-      if (lean_threads_override() == 320) return launch_lean_pair<T, 320, 2>(h, A, s);
-    }
-    switch (lean_threads_setting(h->cfg.n_elem)) {
-      case 1024: return launch_lean_pair<T, 1024, 1>(h, A, s);
-      case 768: return launch_lean_pair<T, 768, 1>(h, A, s);
-      case 544: return launch_lean_pair<T, 544, 1>(h, A, s);
-      case 512: return launch_lean_pair<T, 512, 1>(h, A, s);
-      case 384: return launch_lean_pair<T, 384, 1>(h, A, s);
-      default: return launch_lean_pair<T, 256, 2>(h, A, s);
-    }
-  }
-  // single rod on the plane (OctoArmSingle's model): one 512-thread CTA per SM measured 4 % ahead of two of 256
-  // (3.85 vs 4.04 ms per 4096-env step); the filtered / forced / multi-rod models keep the lane-utilisation rule
-  const bool plain_contact = A.contact_on && !A.muscle_on && !A.spline_mask && A.n_rod <= 1 && !A.has_head;
-  switch (plain_contact ? lean_threads_setting(h->cfg.n_elem) : packed_threads_setting(h->cfg.n_elem, h->n_rod, h->cfg.has_head)) {
-    case 1024: return launch_packed<T, 1024, 1>(h, A, s);
-    case 768: return launch_packed<T, 768, 1>(h, A, s);
-    case 544: return launch_packed<T, 544, 1>(h, A, s);
-    case 512: return launch_packed<T, 512, 1>(h, A, s);
-    case 384: return launch_packed<T, 384, 1>(h, A, s);
-    default: return launch_packed<T, 256, 2>(h, A, s);
-  }
-}
-
-int dispatch_substeps(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
-  if (h->cfg.math == SR_MATH_FAST) return dispatch_packed<double>(h, A, s);
-  // faithful math (libm calls in the reference's operation order): warp-per-rod kernel, the parity build
+// faithful math (libm calls in the reference's operation order): warp-per-rod kernel, the parity build
+int launch_faithful(sr_handle *h, sr::RodArgs<double> &A, const StepKernel<double> &, cudaStream_t s) {
   const int grid = (A.n_env + sr::WARPS_PER_CTA - 1) / sr::WARPS_PER_CTA;
   cudaError_t e = h->epl == 1 ? sr::launch_warp_faithful<double, 1>(A, grid, s)
                   : h->epl == 2 ? sr::launch_warp_faithful<double, 2>(A, grid, s)
@@ -689,6 +506,73 @@ int dispatch_substeps(sr_handle *h, sr::RodArgs<double> &A, cudaStream_t s) {
   h->launches++;
   if (e != cudaSuccess) return cuda_fail("rod_substeps_kernel launch", e);
   return SR_OK;
+}
+
+// The one classification: the kernel that steps this handle.  One row per kernel in precedence order; a config takes
+// the first row whose model it is.  The lean variants' models share their exclusions: none of them steps suckers,
+// external loads or per-element constants, and all but the plain one (variant 0) need FP64 and no base point force.
+template <typename T> StepKernel<T> classify(const sr_handle *h, const sr::RodArgs<T> &A) {
+  constexpr bool F64 = std::is_same<T, double>::value;
+  const Switches &sw = switches();
+  const int n = A.n_elem, bc = A.bc_kind;
+  const int lean_nt = lean_threads_setting(n), packed_nt = packed_threads_setting(n, A.n_rod, A.has_head);
+  const bool assembly = A.n_rod > 1 || A.has_head;
+  const bool free_or_clamped = bc == sr::BC_FREE || bc == sr::BC_ONE_END_FIXED;
+  const bool lean_plain = !(A.sucker || A.ext_force || A.ext_couple || A.elem_tab);
+  const bool lean = F64 && lean_plain && !A.point_force;
+  const bool loads = A.contact_on || A.rest_kappa || A.muscle_on;   // the contact variants' plane and actuations
+  // variant 0: one rod under gravity, damping and the base point force, with a free, clamped or slider end
+  const bool plain = lean_plain && !assembly && !loads && !A.spline_mask && A.laplace_order == 0 && bc != sr::BC_MOVING_BASE;
+  // variant 4, SoftPendulum3D-v0's model: the order-7 LaplaceDissipationFilter, or none with the moving base; a moving,
+  // clamped or free base (n >= 8: the filter's ghost records assume one reflection per end)
+  const bool filter = lean && !assembly && !loads && !A.spline_mask && n >= 8 &&
+                      (A.laplace_order == 7 || (A.laplace_order == 0 && bc == sr::BC_MOVING_BASE)) &&
+                      (free_or_clamped || bc == sr::BC_MOVING_BASE);
+  // variants 1 / 2: one rod on the frictional plane / with rest-curvature actuation / with the travelling-wave muscle
+  const bool contact = lean && !assembly && loads && !A.spline_mask && A.laplace_order == 0 && free_or_clamped;
+  if constexpr (F64) {
+    if (h->cfg.math != SR_MATH_FAST) return {launch_faithful};
+    if (A.elem_tab) return {h->n_rod * (n + 1) + (A.has_head ? 1 : 0) <= 384 ? launch_tapered<384> : launch_tapered<1024>};
+    // rods of 1024-4095 elements, and filter rods of 768-1023, whose one-CTA variant would not fit its shared memory
+    if (n >= 1024 || (n >= 768 && filter) || (sw.cluster && n >= 512 && (plain || filter)))
+      return {lean_cluster_variant(A.laplace_order, bc) == 10 ? launch_cluster<10> : launch_cluster<9>, 0, true};
+    // variant 3: assemblies (OctoFlat: arms + rigid head + FixedJoint2Rigid joints on the plane)
+    if (lean && assembly && !A.spline_mask && !A.muscle_on && A.laplace_order == 0 && bc == sr::BC_FREE && A.rot_on == 0)
+      return {launch_lean<T, 3>, packed_nt, true};
+    // variant 5: SoftArmTracking-v0's spline muscle torques; the safe kernel alone, as it updates the forcing's cached
+    // control values and magnitudes inside the launch
+    if (lean && A.spline_mask && !assembly && !loads && A.laplace_order == 0 && free_or_clamped)
+      return {launch_lean<T, 5>, lean_nt, false};
+    if (filter) return {launch_lean<T, 4>, lean_nt, true};
+    // variants 6 / 7: a rod of exactly 512 elements in 512 threads, the tip node folded into the last one (128
+    // registers), instead of 513 threads in a 544-thread CTA (96 registers)
+    if (sw.fold && n == 512 && A.model == sr::MODEL_ROD && !A.muscle_on && (contact || plain))
+      return {contact ? launch_lean<T, 7> : launch_lean<T, 6>, 512, true};
+    if (contact) return {A.muscle_on ? launch_lean<T, 2> : launch_lean<T, 1>, lean_nt, true};
+  }
+  if (plain) {
+    // Its fast-only kernel may be the planar variant 8 when the model keeps the out-of-plane components exact zeros
+    // once the state has them: FP64, gravity in the x-y plane, the base point force along x (the only direction the
+    // kernel applies it in), and a BC that pins in-plane rows (slider, clamp) or none.  The kernel checks the state
+    // itself, per rod, and hands the rods that are not planar over to the safe kernel.
+    const bool planar = F64 && sw.planar && lean_nt <= 512 && (double)A.gdt_cv[2] == 0.0 &&
+                        (free_or_clamped || bc == sr::BC_PENDULUM_SLIDER);
+    return {launch_lean<T, 0>, lean_nt, true, planar};
+  }
+  // The generic kernel: FP32 storage of the other models, suckers, external loads, the base point force with other
+  // forcings, filter orders other than 7.  The single rod on the plane (OctoArmSingle's model) takes the lean CTA-size
+  // rule: one 512-thread CTA per SM measured 4 % ahead of two of 256 (3.85 vs 4.04 ms per 4096-env step).
+  const int nt = A.contact_on && !A.muscle_on && !A.spline_mask && !assembly ? lean_nt : packed_nt;
+  const bool pair = F64 && !A.spline_mask;   // (the spline forcing updates its cache inside the launch: safe kernel only)
+  if (assembly) return {launch_generic<T, G_MULTI>, nt, pair};
+  if (A.muscle_on || A.spline_mask) return {launch_generic<T, G_TORQUE>, nt, pair};
+  if (A.contact_on || A.rest_kappa || A.sucker || A.ext_force || A.ext_couple) return {launch_generic<T, G_CONTACT>, nt, pair};
+  return {launch_generic<T, G_FILTER>, nt, pair};
+}
+
+template <typename T> int launch_step(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
+  const StepKernel<T> k = classify(h, A);
+  return k.launch(h, A, k, s);
 }
 
 }  // namespace
@@ -824,7 +708,8 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   SR_CUDA(cudaSetDevice(cfg->device));
   if (cfg->n_elem > 1023) {
     const int C = lean_cluster_size(cfg->n_elem);
-    const int n_active = cfg->model == SR_MODEL_SOFT_PENDULUM_3D ? sr::lean_cluster_max_active<10>(C) : sr::lean_cluster_max_active<9>(C);
+    const int n_active = lean_cluster_variant(cfg->laplace_filter_order, cfg->bc_kind) == 10 ? sr::lean_cluster_max_active<10>(C)
+                                                                                              : sr::lean_cluster_max_active<9>(C);
     if (n_active < 1)
       return fail(SR_E_CUDA, "sr_create: n_elem = " + std::to_string(cfg->n_elem) + " needs a cluster of " + std::to_string(C) +
                                  " CTAs of 512 threads, and this device cannot launch one");
@@ -1089,12 +974,12 @@ int sr_step(sr_handle *h, const float *action_dev, int n_substeps, float *obs_de
     sr::RodArgs<float> A = h->a32;
     A.action = action_dev; A.obs = obs_dev; A.reward = reward_dev; A.terminated = terminated_dev;
     A.n_substeps = n_substeps;
-    return dispatch_packed<float>(h, A, (cudaStream_t)stream);
+    return launch_step<float>(h, A, (cudaStream_t)stream);
   }
   sr::RodArgs<double> A = h->a64;
   A.action = action_dev; A.obs = obs_dev; A.reward = reward_dev; A.terminated = terminated_dev;
   A.n_substeps = n_substeps;
-  return dispatch_substeps(h, A, (cudaStream_t)stream);
+  return launch_step<double>(h, A, (cudaStream_t)stream);
 }
 
 int sr_observe(sr_handle *h, const float *prev_action_dev, float *obs_dev, void *stream) {

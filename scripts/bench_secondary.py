@@ -1,5 +1,6 @@
 """Device-timed throughput of the non-headline kernel instantiations (contact, SoftPendulum3D, assemblies, long rod):
-one JSON line each.  A/B knobs come from the environment (SOFTROD_RODSYNC, SOFTROD_PACKED_THREADS, SOFTROD_FASTPATH)."""
+one JSON line each.  A/B switches come from the environment (SOFTROD_FASTPATH, SOFTROD_LEAN_FOLD, ...: INTEGRATION.md §6)
+and are recorded in each line."""
 import json, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)

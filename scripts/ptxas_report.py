@@ -1,23 +1,35 @@
-"""Compile libsoftrod.so with -Xptxas -v and print registers / spills per kernel."""
-import re, subprocess, sys, os
+"""Compile every translation unit of libsoftrod.so with -Xptxas -v (into a temporary directory; the library in the
+tree is left alone) and print registers, stack and spills per kernel, one line each, sorted by kernel name."""
+import concurrent.futures, os, re, subprocess, sys, tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from gym_softrobot_b200 import build as b
-cmd = [b._nvcc()] + b.NVCC_FLAGS + ["-Xptxas", "-v", "-o", b.LIB_PATH] + [os.path.join(b.CSRC, s) for s in b.SOURCES]
-out = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True).stdout
-if "error" in out:
-    print(out); sys.exit(1)
-cur = None
+
+
+def ptxas(tu, out_dir):
+    name, src, defs, _ = tu
+    cmd = [b._nvcc()] + b.NVCC_FLAGS + defs + ["-Xptxas", "-v", "-c", os.path.join(b.CSRC, src),
+                                               "-o", os.path.join(out_dir, name + ".o")]
+    res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+    if res.returncode != 0:
+        sys.exit(f"nvcc failed on {name}:\n{res.stdout}")
+    return res.stdout
+
+
+with tempfile.TemporaryDirectory() as tmp, concurrent.futures.ThreadPoolExecutor(os.cpu_count() or 1) as ex:
+    out = "\n".join(ex.map(lambda tu: ptxas(tu, tmp), b.translation_units()))
+rows, cur, spill = {}, None, None
 for line in out.splitlines():
     m = re.search(r"Compiling entry function '(\S+)'", line)
     if m:
-        cur = subprocess.run(["c++filt", m.group(1)], stdout=subprocess.PIPE, text=True).stdout.strip()
-        cur = re.sub(r"\(.*", "", cur).replace("void sr::", "")
-        spill = None
+        cur, spill = m.group(1), None
     m = re.search(r"(\d+) bytes stack frame, (\d+) bytes spill stores, (\d+) bytes spill loads", line)
     if m and cur and spill is None:
         spill = m.groups()
     m = re.search(r"Used (\d+) registers", line)
     if m and cur:
-        print(f"{cur:55s} regs={m.group(1):>3s} stack={spill[0]:>5s} spill_st={spill[1]:>5s} spill_ld={spill[2]:>5s}")
+        rows[cur] = (m.group(1),) + spill
         cur = None
+names = subprocess.run(["c++filt"], input="\n".join(rows), stdout=subprocess.PIPE, text=True).stdout.splitlines()
+for name, (regs, stack, st, ld) in sorted(zip((re.sub(r"\(.*", "", n).replace("void sr::", "") for n in names), rows.values())):
+    print(f"{name:55s} regs={regs:>3s} stack={stack:>5s} spill_st={st:>5s} spill_ld={ld:>5s}")
