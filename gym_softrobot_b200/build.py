@@ -42,7 +42,7 @@ def translation_units():
     for nt, minb in PLANAR_SIZES:     # variant 0 for rods in the x-y plane (fast-only kernel; FP64)
         tus.append((f"leanc8_double_{nt}_{minb}", "inst_lean.cu", ["-DSR_TU_T=double", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", "-DSR_TU_CONTACT=8"],
                     _COMMON + ["rod_kernel_lean.cuh"]))
-    for cv in (9, 10):    # variant 0 / 4 on thread-block clusters: rods of 512-4095 elements
+    for cv in (9, 10, 11, 12):    # variant 0 / 4 / 1 / 2 on thread-block clusters: rods of 512-4095 elements
         tus.append((f"leanc{cv}_double_512", "inst_lean.cu", ["-DSR_TU_T=double", "-DSR_TU_NT=512", "-DSR_TU_MINB=1", f"-DSR_TU_CONTACT={cv}"],
                     _COMMON + ["rod_kernel_lean.cuh"]))
     for cv in (6, 7):     # plain / contact variant with the tip node folded into the last element's thread (n_elem = 512)

@@ -1,5 +1,5 @@
 // inst_lean.cu — the lean kernel (rod_kernel_lean.cuh) for one storage type and CTA size:
-//   -DSR_TU_T=double|float -DSR_TU_NT=<threads> -DSR_TU_MINB=<n> [-DSR_TU_CONTACT=1|2|3|4: contact variant without / with the muscle wave / for assemblies; 4: filter + moving base; 5: spline torques; 6 / 7: variants 0 / 1 with the tip node folded into the last thread; 8: variant 0 in the x-y plane, fast-only kernel only; 9 / 10: variant 0 / 4 on thread-block clusters, 512 threads only; FP64 only]
+//   -DSR_TU_T=double|float -DSR_TU_NT=<threads> -DSR_TU_MINB=<n> [-DSR_TU_CONTACT=1|2|3|4: contact variant without / with the muscle wave / for assemblies; 4: filter + moving base; 5: spline torques; 6 / 7: variants 0 / 1 with the tip node folded into the last thread; 8: variant 0 in the x-y plane, fast-only kernel only; 9 / 10 / 11 / 12: variant 0 / 4 / 1 / 2 on thread-block clusters, 512 threads only; FP64 only]
 #include <atomic>
 #include "launch.cuh"
 #include "rod_kernel_lean.cuh"
@@ -40,7 +40,7 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT> int lean_cta
 #ifndef SR_TU_CONTACT
 #define SR_TU_CONTACT 0
 #endif
-#if SR_TU_CONTACT == 9 || SR_TU_CONTACT == 10
+#if SR_TU_CONTACT >= 9 && SR_TU_CONTACT <= 12
 static_assert(SR_TU_NT == LEAN_CLUSTER_NT, "the cluster variants are built for 512-thread CTAs");
 constexpr int CV = SR_TU_CONTACT;
 

@@ -20,7 +20,7 @@ constexpr int LEAN_SCR_FOLD = 27;      // folded-tip variants: + position and ve
 template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> cudaError_t launch_lean_kernel(const RodArgs<T> &A, int grid, cudaStream_t s);
 // resident CTAs per SM of that instantiation on the current device (sizes the stream-K grid)
 template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int lean_ctas_per_sm();
-// variants 9 / 10 (FP64, 512 threads): one rod per thread-block cluster of `cluster` CTAs, grid = n_env x cluster CTAs
+// cluster variants 9-12 (FP64, 512 threads): one rod per thread-block cluster of `cluster` CTAs, grid = n_env x cluster CTAs
 constexpr int LEAN_CLUSTER_NT = 512;
 template <bool FASTONLY, int CVAR> cudaError_t launch_lean_cluster_kernel(const RodArgs<double> &A, int cluster, cudaStream_t s);
 // clusters of that shape that both kernels of variant CVAR's pair can keep resident at once on the current device (0: none)

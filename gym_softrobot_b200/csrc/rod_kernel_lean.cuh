@@ -3,8 +3,8 @@
 // configs 2 and 3).  Variants 1-7 put the other models on the same skeleton (see the comment at the kernel):
 // 1 plane contact + rest curvature, 2 + travelling-wave muscle, 3 assemblies (arms + rigid head + joints), 4 Laplace
 // filter + moving base, 5 spline muscle torques, 6 / 7 = 0 / 1 with the tip node folded into the last thread, 8 = 0 for
-// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits), 9 / 10 = 0 / 4 for rods of 512-4095
-// elements, one rod per thread-block cluster of 2-8 CTAs (same substep, same bits).
+// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits), 9 / 10 / 11 / 12 = 0 / 4 / 1 / 2 for rods
+// of 512-4095 elements, one rod per thread-block cluster of 2-8 CTAs (same substep, same bits).
 //
 // Same mapping as rod_kernel_packed.cuh (one thread per node/element, rods packed back to back across a
 // 256-thread CTA, state in registers for the whole launch, neighbour data through array-of-structures
@@ -111,9 +111,9 @@ constexpr int LEAN_JREC = 10;      // assemblies: joint record of an arm's first
 // records and taps end within 30 records past NT: sized as rods of >= 9 threads, its ghost array alone would take
 // 73 KB at 544 threads and push the 768- and 1024-thread CTAs past the 227 KB a CTA can have.
 constexpr int lean_ghost_records(int nt) { return nt <= 512 ? nt + 16 * (nt / 9) + 16 : nt + 48; }
-// records of each exchange array beyond the NT threads' own: the cluster variants 9 / 10 have a halo record before
+// records of each exchange array beyond the NT threads' own: the cluster variants 9-12 have a halo record before
 // thread 0, two after thread NT - 1 and a zero record; the others a zero record and a spare one
-__host__ __device__ constexpr int lean_extra_records(int cvar) { return cvar == 9 || cvar == 10 ? 4 : 2; }
+__host__ __device__ constexpr int lean_extra_records(int cvar) { return cvar >= 9 && cvar <= 12 ? 4 : 2; }
 // variant 10: each rank's ghost-padded filter records hold the rod indices [NT c - 8, NT c + NT + 8) (6 of the 8 halo
 // records per side used, as variant 4 pads them)
 constexpr int lean_smem_words(int nt, int cvar = 0) {
@@ -121,7 +121,7 @@ constexpr int lean_smem_words(int nt, int cvar = 0) {
          (cvar == 4 ? 6 * lean_ghost_records(nt) : cvar == 10 ? 6 * (nt + 16) : 0);
 }
 
-// variants 9 / 10: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
+// cluster variants: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
 template <typename T> __device__ __forceinline__ T *cluster_smem(T *p, int rank) {
   return cooperative_groups::this_cluster().map_shared_rank(p, (unsigned)rank);
 }
@@ -166,7 +166,8 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   // threads, not n + 1 — what lets the 512-element rod (BASELINE config 5) run in a 512-thread CTA with 128 registers
   // instead of a 544-thread one capped at 96 (17 warps put five on one scheduler).  One rod per CTA.
   constexpr bool FOLD = CVAR == 6 || CVAR == 7;
-  constexpr bool CONTACT = (CVAR >= 1 && CVAR <= 3) || CVAR == 7, MUS = CVAR == 2, MULTI = CVAR == 3;
+  constexpr bool CONTACT = (CVAR >= 1 && CVAR <= 3) || CVAR == 7 || CVAR == 11 || CVAR == 12;
+  constexpr bool MUS = CVAR == 2 || CVAR == 12, MULTI = CVAR == 3;
   // 8: variant 0 for a rod that stays in the lab x-y plane (SoftPendulum-v0, planar clamped / free rods; the host checks
   // gravity and the base force).  x_z, v_z, d1_z, d3_z, d2_x, d2_y, w_0, w_2, kappa_0, kappa_2 and sigma_1 are exact zeros
   // at every substep, and every product that carries one of them is left out: the same terms in the same order, so the
@@ -190,7 +191,12 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   // halos -1 / NT.  Each rank's ghost-padded array gb holds the rod indices [NT c - 8, NT c + NT + 8), and a g record
   // of index k is stored into every rank whose taps read it (put_g below); the reflected ghosts follow the same rule.
   // The filter's two barriers become cluster barriers as well: four per substep.
-  constexpr bool CLUSTER = CVAR == 9 || CVAR == 10;
+  // 11 / 12: variants 1 / 2 in variant 9's layout (the rod on the frictional plane at 512-4095 elements).  The plane's two
+  // extra exchanges read across the rank boundary too, so the last thread pushes its stage-1 load into the next rank's
+  // rec halo -1 (words 16-17) and its final plane load into the next rank's sn halo -1; thread 0 pushes its stress
+  // record into the previous rank's sn halo NT and its stage-1 load into the previous rank's rec halo NT (words 16-17).
+  // The contact's two barriers become cluster barriers: four per substep.  DESIGN.md §4.1 gives the slot-by-slot order.
+  constexpr bool CLUSTER = CVAR >= 9 && CVAR <= 12;
   static_assert(CVAR == 0 || !MIXED, "the variants are FP64 only");
   static_assert(!FOLD || LEAN_SCR_FOLD >= 27, "hand-over rows of the folded tip");
   constexpr int SCR = FOLD ? LEAN_SCR_FOLD : CONTACT ? LEAN_SCR_CONTACT : LEAN_REC;   // rows of a slot's hand-over scratch
@@ -227,7 +233,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   D *gb = sj;                                       // filter variant: ghost-padded records of the filtered rates
   if (tid < SNR) sn[SNR * ZR + tid] = F(0);
   if (CLUSTER && tid < 256) { sh_dom[tid] = 0; sh_flag[tid] = 0; }   // (rank 0's are the cluster's env-level flags)
-  if (CONTACT && tid < 2) rec[LEAN_REC * NT + 16 + tid] = D(0);   // stage-1 contact load "left of element 0"
+  if (CONTACT && tid < 2) rec[LEAN_REC * ZR + 16 + tid] = D(0);   // stage-1 contact load "left of element 0"
   if (FOLD && tid < LEAN_REC) rec[LEAN_REC * NT + tid] = D(0);     // the folded tip's record: x, v published by the last thread, the rest finite
   __syncthreads();   // (the per-rod barriers below do not order this store against the other rods' reads)
   if constexpr (CLUSTER) cluster_sync();   // every CTA of the cluster runs, with its flags zeroed, before DSMEM is touched
@@ -479,6 +485,8 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         for (int c = 0; c < 3; c++) rk[c] = (D)A.rest_kappa[((size_t)rod * 3 + c) * stride + j];
       }
       if (mus && active) {
+        // (the cluster variant: every rank reads the clock mu[0] here, ahead of its first cluster barrier of the item;
+        // rank 0's lead alone writes it back, after the last one)
         // MuscleTorques (continuum_snake.py:186-198): element k gets Q_k d (m_k [k >= 1] - m_{k+1} [k <= n-2]),
         // m_k = min(1, t/ramp) beta_{n-1-k} sin(w t - kw s_{n-1-k} + phi).  sin(p - s) = sin p cos s - cos p sin s, so
         // m_k - m_{k+1} = ramp (sin p * P - cos p * R) with per-element constants P = b0 cos s0 - b1 cos s1,
@@ -791,7 +799,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       // the first substep of a segment checks the trace once to rule out a state that starts beyond.
       F w2 = dot3(vec, vec);
       if (!vor_ok) w2 = F(0);
-      constexpr bool MIDBEND = CVAR == 1 || CVAR == 2 || CVAR == 7;   // actuated arms on the plane: the 37-degree map
+      constexpr bool MIDBEND = CVAR == 1 || CVAR == 2 || CVAR == 7 || CVAR == 11 || CVAR == 12;   // actuated arms on the plane: the 37-degree map
       bool bend_out = out_of_range(w2, MIDBEND ? A.lim_bendm_hi : A.lim_bend_hi, A.limf_bend);
       F u_ref = F(0);
       if constexpr (MULTI) {
@@ -883,6 +891,10 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         if (CLUSTER && tid == NT - 1 && c_rank + 1 < c_size) {   // element j - 1 of the next rank's thread 0
           double2 *h = cluster_smem(reinterpret_cast<double2 *>(sn - SNR), c_rank + 1);
           h[0] = o[0]; h[1] = o[1]; h[2] = o[2];
+        }
+        if (CLUSTER && CONTACT && tid == 0 && c_rank > 0) {   // element j + 1 of the previous rank's last thread (the plane's stage 1)
+          double2 *h = cluster_smem(reinterpret_cast<double2 *>(sn + SNR * NT), c_rank - 1);
+          h[0] = o[0]; h[1] = o[1];
         }
       }
       // rotational damper c_w^e = c_w exp((e-1) ln c_w) as a quadratic in (e-1) (coefficients made on the host; the
@@ -1054,6 +1066,12 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
           // couple of the rolling friction: Q (arm x F) = Q (rad F_y, -rad F_x, 0); kept in the plane's frame until the end
           D cr0 = rad * fr1, cr1 = -(rad * fr0);
           *reinterpret_cast<double2 *>(rec + LEAN_REC * tid + 16) = make_double2(c1[0], c1[1]);
+          if constexpr (CLUSTER) {   // the stage-1 neighbours across the rank boundary: rec halos NT and -1, words 16-17
+            double2 *h = nullptr;
+            if (tid == 0 && c_rank > 0) h = cluster_smem(reinterpret_cast<double2 *>(rec + LEAN_REC * NT + 16), c_rank - 1);
+            if (tid == NT - 1 && c_rank + 1 < c_size) h = cluster_smem(reinterpret_cast<double2 *>(rec - LEAN_REC + 16), c_rank + 1);
+            if (h) *h = make_double2(c1[0], c1[1]);
+          }
           rod_sync();
           // stage 2: static friction (in-plane components only)
           D e2[2];
@@ -1077,6 +1095,11 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
           const D p0 = c1[0] + fma(sa, ax0, fr0), p1 = c1[1] + fma(sa, ax1, fr1);
           *reinterpret_cast<double2 *>(sn + SNR * tid) = make_double2(p0, p1);
           sn[SNR * tid + 2] = c1[2];
+          if (CLUSTER && tid == NT - 1 && c_rank + 1 < c_size) {   // element j - 1 of the next rank's thread 0: sn halo -1
+            D *h = cluster_smem(reinterpret_cast<D *>(sn - SNR), c_rank + 1);
+            *reinterpret_cast<double2 *>(h) = make_double2(p0, p1);
+            h[2] = c1[2];
+          }
           cr0 = fma(rad, fr1, cr0); cr1 = fma(-rad, fr0, cr1);   // both stages' rolling couples
 #pragma unroll
           for (int i = 0; i < 3; i++) tq[i] = fma(Q[3 * i + 1], cr1, fma(Q[3 * i], cr0, tq[i]));

@@ -358,14 +358,26 @@ int lean_threads_setting(int n_elem) {
   return best;
 }
 
-// CTAs of the cluster that holds one rod of n elements in the cluster variants (9, 10): n + 1 threads of 512 per CTA
+// CTAs of the cluster that holds one rod of n elements in the cluster variants (9-12): n + 1 threads of 512 per CTA
 int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
 
-// The cluster variant that steps a rod of the plain model (9: variant 0's substep) or of SoftPendulum3D-v0's (10:
-// variant 4's, with the Laplace filter and the moving base).  sr_create checks its cluster shape for rods of
-// 1024-4095 elements, the only models it admits there.
-int lean_cluster_variant(int laplace_order, int bc_kind) {
+// The cluster variant that steps a rod of the plain model (9: variant 0's substep), of SoftPendulum3D-v0's (10: variant
+// 4's, with the Laplace filter and the moving base), or the rod on the frictional plane with rest-curvature actuation
+// (`loads`: 11, variant 1's) and the travelling-wave muscle (12, variant 2's).  sr_create checks its cluster shape for
+// rods of 1024-4095 elements, the only models it admits there.
+int lean_cluster_variant(int laplace_order, int bc_kind, bool loads, bool muscle_on) {
+  if (loads) return muscle_on ? 12 : 11;
   return laplace_order > 0 || bc_kind == sr::BC_MOVING_BASE ? 10 : 9;
+}
+
+// clusters of C CTAs that both kernels of cluster variant cv can keep resident at once (0: none)
+int cluster_max_active(int cv, int C) {
+  switch (cv) {
+    case 10: return sr::lean_cluster_max_active<10>(C);
+    case 11: return sr::lean_cluster_max_active<11>(C);
+    case 12: return sr::lean_cluster_max_active<12>(C);
+  }
+  return sr::lean_cluster_max_active<9>(C);
 }
 
 // What steps a handle (classify): the launcher of one kernel, and the launch's shape.
@@ -459,6 +471,15 @@ template <int CV> int launch_cluster(sr_handle *h, sr::RodArgs<double> &A, const
     return SR_OK;
   });
 }
+// the classify row of cluster variant cv
+StepKernel<double> cluster_kernel(int cv) {
+  switch (cv) {
+    case 10: return {launch_cluster<10>, 0, true};
+    case 11: return {launch_cluster<11>, 0, true};
+    case 12: return {launch_cluster<12>, 0, true};
+  }
+  return {launch_cluster<9>, 0, true};
+}
 
 // the generic kernel (rod_kernel_packed.cuh) with the features of one group
 enum { G_FILTER, G_CONTACT, G_TORQUE, G_MULTI };   // Laplace filter + moving base / plane contact / + forcing torques / assemblies
@@ -534,8 +555,8 @@ template <typename T> StepKernel<T> classify(const sr_handle *h, const sr::RodAr
     if (h->cfg.math != SR_MATH_FAST) return {launch_faithful};
     if (A.elem_tab) return {h->n_rod * (n + 1) + (A.has_head ? 1 : 0) <= 384 ? launch_tapered<384> : launch_tapered<1024>};
     // rods of 1024-4095 elements, and filter rods of 768-1023, whose one-CTA variant would not fit its shared memory
-    if (n >= 1024 || (n >= 768 && filter) || (sw.cluster && n >= 512 && (plain || filter)))
-      return {lean_cluster_variant(A.laplace_order, bc) == 10 ? launch_cluster<10> : launch_cluster<9>, 0, true};
+    if (n >= 1024 || (n >= 768 && filter) || (sw.cluster && n >= 512 && (plain || filter || contact)))
+      return cluster_kernel(lean_cluster_variant(A.laplace_order, bc, loads, A.muscle_on));
     // variant 3: assemblies (OctoFlat: arms + rigid head + FixedJoint2Rigid joints on the plane)
     if (lean && assembly && !A.spline_mask && !A.muscle_on && A.laplace_order == 0 && bc == sr::BC_FREE && A.rot_on == 0)
       return {launch_lean<T, 3>, packed_nt, true};
@@ -590,20 +611,27 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   if (cfg->n_env <= 0 || cfg->n_elem < 3) return fail(SR_E_INVALID, "sr_create: n_env > 0 and n_elem >= 3 required");
   if (cfg->n_elem > 4095)
     return fail(SR_E_INVALID, "sr_create: n_elem <= 4095 (rods of 1024-4095 elements span a thread-block cluster of up to 8 CTAs)");
-  // rods of 1024-4095 elements: variant 0's model (cluster variant 9) or SoftPendulum3D-v0's (cluster variant 10)
+  // rods of 1024-4095 elements: variant 0's model (cluster variant 9), SoftPendulum3D-v0's (10), or the rod on the
+  // frictional plane with rest-curvature actuation and / or the travelling-wave muscle (11 / 12)
+  const bool loads = cfg->contact_on || cfg->muscle_on;
   const bool long_rod_model =
       ((cfg->model == SR_MODEL_ROD || cfg->model == SR_MODEL_SOFT_PENDULUM) &&
        (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED || cfg->bc_kind == SR_BC_PENDULUM_SLIDER) &&
-       cfg->laplace_filter_order == 0) ||
+       cfg->laplace_filter_order == 0 && !loads) ||
       (cfg->model == SR_MODEL_SOFT_PENDULUM_3D && cfg->bc_kind == SR_BC_MOVING_BASE && cfg->laplace_filter_order == 7 &&
-       !cfg->point_force_on_base);
+       !cfg->point_force_on_base && !loads) ||
+      (cfg->model == SR_MODEL_ROD && (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED) &&
+       cfg->laplace_filter_order == 0 && !cfg->point_force_on_base && loads);
   if (cfg->n_elem > 1023 &&
-      (cfg->dtype != SR_DTYPE_F64 || cfg->math != SR_MATH_FAST || !long_rod_model || cfg->contact_on || cfg->muscle_on ||
+      (cfg->dtype != SR_DTYPE_F64 || cfg->math != SR_MATH_FAST || !long_rod_model ||
        cfg->spline_dir_mask || cfg->n_rod_per_env > 1 || cfg->has_head || cfg->tip_radius > 0.0 || cfg->sucker_on ||
        cfg->tm_muscle_on || cfg->muscle_layers_on))
     return fail(SR_E_INVALID, "sr_create: n_elem of 1024-4095 is built for SR_DTYPE_F64, SR_MATH_FAST, SR_MODEL_ROD or "
                               "SR_MODEL_SOFT_PENDULUM, one untapered rod per env with a free, clamped or slider end, gravity, "
-                              "damping and the base point force; no contact, muscle or spline torques, suckers or Laplace filter; "
+                              "damping and the base point force; for SR_MODEL_ROD with a free or clamped end on the frictional "
+                              "plane (contact_on) and / or with the travelling-wave muscle (muscle_on), rest curvature, "
+                              "gravity and damping, without the base point force; no spline torques, suckers, transverse "
+                              "muscle, muscle layers or Laplace filter; "
                               "and for SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE and laplace_filter_order = 7, "
                               "without the base point force");
   if (cfg->n_elem > 127 && cfg->math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_create: faithful math supports n_elem <= 127");
@@ -708,8 +736,7 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   SR_CUDA(cudaSetDevice(cfg->device));
   if (cfg->n_elem > 1023) {
     const int C = lean_cluster_size(cfg->n_elem);
-    const int n_active = lean_cluster_variant(cfg->laplace_filter_order, cfg->bc_kind) == 10 ? sr::lean_cluster_max_active<10>(C)
-                                                                                              : sr::lean_cluster_max_active<9>(C);
+    const int n_active = cluster_max_active(lean_cluster_variant(cfg->laplace_filter_order, cfg->bc_kind, loads, cfg->muscle_on), C);
     if (n_active < 1)
       return fail(SR_E_CUDA, "sr_create: n_elem = " + std::to_string(cfg->n_elem) + " needs a cluster of " + std::to_string(C) +
                                  " CTAs of 512 threads, and this device cannot launch one");
@@ -1107,7 +1134,10 @@ int sr_spline_basis(int32_t P, double base_length, double *out) {
 int sr_get_rest_kappa(sr_handle *h, void **rest_kappa_dev) {
   if (!h || !rest_kappa_dev) return fail(SR_E_INVALID, "sr_get_rest_kappa: null argument");
   if (h->cfg.math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for SR_MATH_FAST only");
-  if (h->cfg.n_elem > 1023) return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for n_elem <= 1023");
+  // (above 1023 elements only the rods on the plane / with the muscle wave step on a kernel that reads it: variants 11 / 12)
+  if (h->cfg.n_elem > 1023 && !h->cfg.contact_on && !h->cfg.muscle_on)
+    return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for n_elem <= 1023, and above for rods with "
+                              "contact_on or muscle_on");
   if (!h->rest_kappa) {
     SR_CUDA(cudaSetDevice(h->cfg.device));
     size_t bytes = (size_t)h->cfg.n_env * h->n_rod * 3 * h->stride * h->elem_size;

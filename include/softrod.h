@@ -68,10 +68,13 @@ typedef struct sr_config {
   int32_t math;         /* SR_MATH_* */
   int32_t n_env;        /* independent environments (one rod each) */
   int32_t n_elem;       /* elements per rod: 3-1023; 1024-4095 (one rod per thread-block cluster of up to 8 CTAs) for
-                         * SR_DTYPE_F64, SR_MATH_FAST, one untapered rod per env without contact, muscle / spline
-                         * torques or suckers, and either SR_MODEL_ROD / SR_MODEL_SOFT_PENDULUM with a free, clamped or
-                         * slider end and no filter, or SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE,
-                         * laplace_filter_order = 7 and no base point force */
+                         * SR_DTYPE_F64, SR_MATH_FAST, one untapered rod per env without spline torques, suckers or
+                         * muscle layers, and either SR_MODEL_ROD / SR_MODEL_SOFT_PENDULUM with a free, clamped or
+                         * slider end, no contact, muscle or filter; or SR_MODEL_ROD with a free or clamped end on the
+                         * frictional plane (contact_on) and / or with the travelling-wave muscle (muscle_on), with
+                         * rest curvature (sr_get_rest_kappa) and no base point force or filter; or
+                         * SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE, laplace_filter_order = 7 and no base point
+                         * force */
   int32_t bc_kind;      /* SR_BC_* */
   int32_t point_force_on_base; /* F_ext[0,0] = action[env,0] each substep (build.py:94-105) */
   int32_t damping_before_constraints; /* 1: [dampen_rates, constrain_rates]; 0 (the envs): [constrain_rates, dampers] = build-code call order */
@@ -257,7 +260,7 @@ int sr_get_head(sr_handle *h, void **head_dev, int32_t *dim);
 /* Per-env rest curvature (the actuation of the octopus-arm envs: `rod.rest_kappa[0, :] = ...`,
  * envs/octopus/arm_single_env.py:226-235, flat_env.py:288-311), [n_env][3][stride] of the handle's
  * dtype (n_env * n_rod_per_env rows for assemblies), Voronoi points in slots 0..n_elem-2; allocated on
- * first use, zero-initialised. */
+ * first use, zero-initialised.  Above 1023 elements, for handles with contact_on or muscle_on only. */
 int sr_get_rest_kappa(sr_handle *h, void **rest_kappa_dev);
 
 /* Per-env muscle-torque data (muscle_on handles), [n_env][*dim] float64 whatever the handle's dtype:

@@ -1,8 +1,10 @@
-"""Long rods on thread-block clusters (variants 9 / 10 of rod_kernel_lean.cuh): device time per launch of K = 100 substeps.
+"""Long rods on thread-block clusters (variants 9-12 of rod_kernel_lean.cuh): device time per launch of K = 100 substeps.
 
 Clamped rods (BASELINE config 3's model, variant 9), or with --model pendulum3d SoftPendulum3D-v0's rod (Laplace filter
-and moving base, variant 10; base held still, 608 FLOP per element-substep), with enough envs that the state block
-exceeds the 126 MB L2 (>= 256 MB).
+and moving base, variant 10; base held still, 608 FLOP per element-substep), with --model contact a free rod resting on
+a +z frictional plane with rest curvature, forcing first (OctoArmSingle's plane and friction, variant 11: 720 FLOP per
+element-substep), with --model snake the same on a +y plane with the travelling-wave muscle (variant 12: 840), with
+enough envs that the state block exceeds the 126 MB L2 (>= 256 MB).
 Cases: n = 600 and 1023 (SoftPendulum3D: 600 and 767, whose one-CTA kernel ends at 768 threads; 1023 on the cluster
 kernel alone) on the one-CTA kernel (768 / 1024 threads) and on the forced cluster kernel (C = 2), which
 run as alternating subprocesses (SOFTROD_LEAN_CLUSTER is read once per process), two rounds each; n = 1024, 2047 and
@@ -12,7 +14,7 @@ element-substep (608 for SoftPendulum3D).  A probe compiled into a temporary dir
 (512 threads, > 114 KB of shared memory each) the device keeps resident, and so what fraction of the SMs a full wave
 of C-CTA clusters leaves idle.
 
-    python scripts/bench_long_rods.py [--model rod|pendulum3d] [--out FILE]   (the report goes to stdout, and to FILE if given)
+    python scripts/bench_long_rods.py [--model rod|pendulum3d|contact|snake] [--out FILE]   (the report goes to stdout, and to FILE if given)
 """
 import argparse
 import json
@@ -23,7 +25,7 @@ import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 K, TIMED, WARMUP = 100, 20, 5
-FLOP_PER_ELEMENT_SUBSTEP = {"rod": 440, "pendulum3d": 608}
+FLOP_PER_ELEMENT_SUBSTEP = {"rod": 440, "pendulum3d": 608, "contact": 720, "snake": 840}
 STATE_BYTES = 256 << 20
 
 _PROBE = r"""
@@ -62,6 +64,24 @@ def one(n, cluster, model):
         h = _make_handle(n_env, n, 2e-6 * 1023 / n, K, 0)
         h.reset_host(pendulum3d_init_params(np.random.default_rng(n).uniform(-1, 1, n_env)))
         act = torch.zeros((n_env, 2), dtype=torch.float32, device="cuda")
+    elif model in ("contact", "snake"):
+        from gym_softrobot_b200.envs.arm_single import arm_contact_params
+        r0, normal = 0.004, np.array([0.0, 0.0, 1.0] if model == "contact" else [0.0, 1.0, 0.0])
+        c = arm_contact_params()
+        c["plane_origin"], c["plane_normal"] = list(-r0 * normal), list(normal)
+        mus = dict(period=1.0, ramp_up_time=5e-4, phase_shift=0.7, direction=list(normal)) if model == "snake" else None
+        h = nat.Handle(model=nat.MODEL_ROD, n_env=n_env, n_elem=n, dt=2e-6 * 1023 / n, base_length=1.0, base_radius=r0,
+                       density=1000.0, youngs_modulus=1e6, gravity=tuple(-9.81 * normal), damping_constant=1e-2,
+                       bc_kind=nat.BC_FREE, math=nat.MATH_FAST, contact=c, muscle=mus)
+        axis = np.array([0.0, 1.0, 0.0] if model == "contact" else [0.0, 0.0, -1.0])
+        h.reset_host(np.tile(np.concatenate([np.zeros(3), axis, normal]), (n_env, 1)))
+        rk = np.random.default_rng(n).uniform(-3, 3, (n_env, 1)) * np.sin(3 * np.pi * np.linspace(0.0, 1.0, n - 1))[None, :]
+        h.rest_kappa_tensor()[:, 0, :] = torch.as_tensor(rk, device="cuda")
+        if mus:
+            mu = h.muscle_tensor()
+            mu[:, 1] = 6.0
+            mu[:, 2:] = torch.as_tensor(2e-4 * np.sin(np.pi * np.linspace(0.0, 1.0, n)), device="cuda")
+        torch.cuda.synchronize()
     else:
         h = nat.Handle(model=nat.MODEL_ROD, n_env=n_env, n_elem=n, dt=2e-6 * 1023 / n, base_length=1.0,
                        base_radius=0.004, density=1000.0, youngs_modulus=1e6, gravity=(0.0, -9.80665, 0.0),
@@ -128,7 +148,7 @@ def main():
                 c, nc = map(int, line.split())
                 say(f"clusters of {c} one-CTA-per-SM blocks resident at once: {nc} ({nc * c} of {sm} SMs busy, "
                     f"{100.0 * (sm - nc * c) / sm:.1f} % idle)")
-    if a.model == "rod":
+    if a.model in ("rod", "contact", "snake"):
         cases = [(600, 0), (600, 1), (1023, 0), (1023, 1)] * 2 + [(1024, 1), (2047, 1), (4095, 1)]
     else:    # (variant 4's largest CTA is 768 threads: from 768 elements on the cluster variant is the only one)
         cases = [(600, 0), (600, 1), (767, 0), (767, 1)] * 2 + [(1023, 1), (1024, 1), (2047, 1), (4095, 1)]
