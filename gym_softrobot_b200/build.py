@@ -24,30 +24,40 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
 ]
-PLANAR_SIZES = [(256, 2), (384, 1), (512, 1)]   # the planar variant (CVAR 8) at the lean kernel's CTA sizes for rods of <= 511 elements
 PACKED_SIZES = [(256, 2), (384, 1), (512, 1), (544, 1), (768, 1), (1024, 1)]   # (threads per CTA, CTAs per SM)
+# The lean kernel's translation units: (model, layout, storage types, (threads per CTA, CTAs per SM)), by the
+# enumerator names of LeanModel / LeanLayout in csrc/launch.cuh.  softrod_api.cu's lean_built() names the same sizes.
+LEAN_UNITS = [
+    ("PLAIN", "CTA", ("double", "float"), PACKED_SIZES),
+    ("PLANE", "CTA", ("double",), PACKED_SIZES),
+    ("MUSCLE", "CTA", ("double",), PACKED_SIZES),
+    ("ASSEMBLY", "CTA", ("double",), PACKED_SIZES),
+    # up to 768 threads: filter rods of >= 768 elements take the cluster layout
+    ("FILTER", "CTA", ("double",), [s for s in PACKED_SIZES if s[0] <= 768]),
+    ("SPLINE", "CTA", ("double",), PACKED_SIZES),
+    # the lean kernel's CTA sizes for rods of <= 511 elements (fast-only kernel)
+    ("PLANAR", "CTA", ("double",), [s for s in PACKED_SIZES if s[0] <= 512]),
+    # a rod of exactly 512 elements in 512 threads
+    ("PLAIN", "FOLD", ("double",), [(512, 1)]),
+    ("PLANE", "FOLD", ("double",), [(512, 1)]),
+    # rods of 512-4095 elements, one per thread-block cluster of 512-thread CTAs
+    ("PLAIN", "CLUSTER", ("double",), [(512, 1)]),
+    ("FILTER", "CLUSTER", ("double",), [(512, 1)]),
+    ("PLANE", "CLUSTER", ("double",), [(512, 1)]),
+    ("MUSCLE", "CLUSTER", ("double",), [(512, 1)]),
+]
 
 
 def translation_units():
     """[(object name, source, extra -D flags, header deps)]"""
     tus = [("api", "softrod_api.cu", [], _COMMON), ("warp", "inst_warp.cu", [], _COMMON)]
-    for t in ("double", "float"):
-        for nt, minb in PACKED_SIZES:
-            tus.append((f"lean_{t}_{nt}", "inst_lean.cu", [f"-DSR_TU_T={t}", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}"],
-                        _COMMON + ["rod_kernel_lean.cuh"]))
-    for nt, minb in PACKED_SIZES:      # the lean kernel's contact variant (FP64): plain, with the travelling-wave muscle, for assemblies; 4 = filter + moving base; 5 = spline torques
-        for cv in (1, 2, 3, 4, 5) if nt <= 768 else (1, 2, 3, 5):   # (filter rods of >= 768 elements take variant 10)
-            tus.append((f"leanc{cv}_double_{nt}", "inst_lean.cu", ["-DSR_TU_T=double", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", f"-DSR_TU_CONTACT={cv}"],
-                        _COMMON + ["rod_kernel_lean.cuh"]))
-    for nt, minb in PLANAR_SIZES:     # variant 0 for rods in the x-y plane (fast-only kernel; FP64)
-        tus.append((f"leanc8_double_{nt}_{minb}", "inst_lean.cu", ["-DSR_TU_T=double", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", "-DSR_TU_CONTACT=8"],
-                    _COMMON + ["rod_kernel_lean.cuh"]))
-    for cv in (9, 10, 11, 12):    # variant 0 / 4 / 1 / 2 on thread-block clusters: rods of 512-4095 elements
-        tus.append((f"leanc{cv}_double_512", "inst_lean.cu", ["-DSR_TU_T=double", "-DSR_TU_NT=512", "-DSR_TU_MINB=1", f"-DSR_TU_CONTACT={cv}"],
-                    _COMMON + ["rod_kernel_lean.cuh"]))
-    for cv in (6, 7):     # plain / contact variant with the tip node folded into the last element's thread (n_elem = 512)
-        tus.append((f"leanc{cv}_double_512", "inst_lean.cu", ["-DSR_TU_T=double", "-DSR_TU_NT=512", "-DSR_TU_MINB=1", f"-DSR_TU_CONTACT={cv}"],
-                    _COMMON + ["rod_kernel_lean.cuh"]))
+    for model, layout, types, sizes in LEAN_UNITS:
+        for t in types:
+            for nt, minb in sizes:
+                tus.append((f"lean_{model.lower()}_{layout.lower()}_{t}_{nt}", "inst_lean.cu",
+                            [f"-DSR_TU_T={t}", f"-DSR_TU_NT={nt}", f"-DSR_TU_MINB={minb}", f"-DSR_TU_MODEL={model}",
+                             f"-DSR_TU_LAYOUT={layout}"],
+                            _COMMON + ["rod_kernel_lean.cuh"]))
     for nt, minb in PACKED_SIZES:
         for t in ("double", "float"):
             for grp in (1, 2, 3):    # (the lean configs of both types run rod_kernel_lean.cuh)

@@ -1,12 +1,14 @@
-// inst_lean.cu — the lean kernel (rod_kernel_lean.cuh) for one storage type and CTA size:
-//   -DSR_TU_T=double|float -DSR_TU_NT=<threads> -DSR_TU_MINB=<n> [-DSR_TU_CONTACT=1|2|3|4: contact variant without / with the muscle wave / for assemblies; 4: filter + moving base; 5: spline torques; 6 / 7: variants 0 / 1 with the tip node folded into the last thread; 8: variant 0 in the x-y plane, fast-only kernel only; 9 / 10 / 11 / 12: variant 0 / 4 / 1 / 2 on thread-block clusters, 512 threads only; FP64 only]
+// inst_lean.cu — the lean kernel (rod_kernel_lean.cuh) for one storage type, CTA size, model and layout:
+//   -DSR_TU_T=double|float -DSR_TU_NT=<threads> -DSR_TU_MINB=<n> -DSR_TU_MODEL=<LeanModel> -DSR_TU_LAYOUT=<LeanLayout>
+// (the models and layouts by their enumerator names in launch.cuh; every model but PLAIN in the CTA layout is FP64 only,
+// the cluster layout is built for LEAN_CLUSTER_NT threads only)
 #include <atomic>
 #include "launch.cuh"
 #include "rod_kernel_lean.cuh"
 
 namespace sr {
 
-template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT> static cudaError_t lean_opt_in() {
+template <typename T, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayout LAYOUT> static cudaError_t lean_opt_in() {
   // the opt-in above 48 KB is a per-device attribute of the function: one bit per device ordinal
   static std::atomic<unsigned long long> opted{0};
   int dev = 0;
@@ -14,41 +16,48 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT> static cudaE
   if (e != cudaSuccess) return e;
   const unsigned long long bit = 1ULL << (dev & 63);
   if (!(opted.load(std::memory_order_relaxed) & bit)) {
-    e = cudaFuncSetAttribute(rod_lean_kernel<T, NT, MINB, FASTONLY, CONTACT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             (int)(lean_smem_words(NT, CONTACT) * sizeof(double)));
+    e = cudaFuncSetAttribute(rod_lean_kernel<T, NT, MINB, FASTONLY, MODEL, LAYOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)(lean_smem_words(NT, MODEL, LAYOUT) * sizeof(double)));
     if (e != cudaSuccess) return e;
     opted.fetch_or(bit, std::memory_order_relaxed);
   }
   return cudaSuccess;
 }
 
-template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT> cudaError_t launch_lean_kernel(const RodArgs<T> &A, int grid, cudaStream_t s) {
-  cudaError_t e = lean_opt_in<T, NT, MINB, FASTONLY, CONTACT>();
+template <typename T, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayout LAYOUT>
+cudaError_t launch_lean_kernel(const RodArgs<T> &A, int grid, cudaStream_t s) {
+  cudaError_t e = lean_opt_in<T, NT, MINB, FASTONLY, MODEL, LAYOUT>();
   if (e != cudaSuccess) return e;
-  rod_lean_kernel<T, NT, MINB, FASTONLY, CONTACT><<<grid, NT, lean_smem_words(NT, CONTACT) * sizeof(double), s>>>(A);
+  rod_lean_kernel<T, NT, MINB, FASTONLY, MODEL, LAYOUT><<<grid, NT, lean_smem_words(NT, MODEL, LAYOUT) * sizeof(double), s>>>(A);
   return cudaGetLastError();
 }
 
-template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT> int lean_ctas_per_sm() {
-  if (lean_opt_in<T, NT, MINB, FASTONLY, CONTACT>() != cudaSuccess) return 0;
+template <typename T, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayout LAYOUT> int lean_ctas_per_sm() {
+  if (lean_opt_in<T, NT, MINB, FASTONLY, MODEL, LAYOUT>() != cudaSuccess) return 0;
   int nb = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rod_lean_kernel<T, NT, MINB, FASTONLY, CONTACT>, NT,
-                                                    lean_smem_words(NT, CONTACT) * sizeof(double)) != cudaSuccess) return 0;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, rod_lean_kernel<T, NT, MINB, FASTONLY, MODEL, LAYOUT>, NT,
+                                                    lean_smem_words(NT, MODEL, LAYOUT) * sizeof(double)) != cudaSuccess) return 0;
   return nb;
 }
 
-#ifndef SR_TU_CONTACT
-#define SR_TU_CONTACT 0
-#endif
-#if SR_TU_CONTACT >= 9 && SR_TU_CONTACT <= 12
-static_assert(SR_TU_NT == LEAN_CLUSTER_NT, "the cluster variants are built for 512-thread CTAs");
-constexpr int CV = SR_TU_CONTACT;
+constexpr LeanModel TU_MODEL = LeanModel::SR_TU_MODEL;
+constexpr LeanLayout TU_LAYOUT = LeanLayout::SR_TU_LAYOUT;
+
+// The preprocessor cannot compare the names SR_TU_MODEL and SR_TU_LAYOUT stand for, so its two tests paste a name onto
+// SR_IS_: SR_IS_CLUSTER and SR_IS_PLANAR are 1, and any other SR_IS_<name> is undefined, which #if reads as 0.
+#define SR_IS_PASTE(name) SR_IS_##name
+#define SR_IS(name) SR_IS_PASTE(name)
+#define SR_IS_CLUSTER 1
+#define SR_IS_PLANAR 1
+
+#if SR_IS(SR_TU_LAYOUT)   // the cluster layout
+static_assert(TU_LAYOUT == LeanLayout::CLUSTER && SR_TU_NT == LEAN_CLUSTER_NT, "the cluster layout is built for 512-thread CTAs");
 
 static cudaLaunchConfig_t cluster_config(int grid, int cluster, cudaStream_t s, cudaLaunchAttribute *attr) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3(LEAN_CLUSTER_NT);
-  cfg.dynamicSmemBytes = lean_smem_words(LEAN_CLUSTER_NT, CV) * sizeof(double);
+  cfg.dynamicSmemBytes = lean_smem_words(LEAN_CLUSTER_NT, TU_MODEL, TU_LAYOUT) * sizeof(double);
   cfg.stream = s;
   attr->id = cudaLaunchAttributeClusterDimension;
   attr->val.clusterDim.x = (unsigned)cluster; attr->val.clusterDim.y = 1; attr->val.clusterDim.z = 1;
@@ -56,42 +65,42 @@ static cudaLaunchConfig_t cluster_config(int grid, int cluster, cudaStream_t s, 
   return cfg;
 }
 
-template <bool FASTONLY, int CVAR> cudaError_t launch_lean_cluster_kernel(const RodArgs<double> &A, int cluster, cudaStream_t s) {
-  static_assert(CVAR == CV, "one cluster variant per translation unit");
-  cudaError_t e = lean_opt_in<double, LEAN_CLUSTER_NT, 1, FASTONLY, CV>();
+template <bool FASTONLY, LeanModel MODEL> cudaError_t launch_lean_cluster_kernel(const RodArgs<double> &A, int cluster, cudaStream_t s) {
+  static_assert(MODEL == TU_MODEL, "one cluster model per translation unit");
+  cudaError_t e = lean_opt_in<double, LEAN_CLUSTER_NT, 1, FASTONLY, MODEL, TU_LAYOUT>();
   if (e != cudaSuccess) return e;
   cudaLaunchAttribute attr;
   const cudaLaunchConfig_t cfg = cluster_config(A.n_env * cluster, cluster, s, &attr);
-  return cudaLaunchKernelEx(&cfg, rod_lean_kernel<double, LEAN_CLUSTER_NT, 1, FASTONLY, CV>, A);
+  return cudaLaunchKernelEx(&cfg, rod_lean_kernel<double, LEAN_CLUSTER_NT, 1, FASTONLY, MODEL, TU_LAYOUT>, A);
 }
 
 template <bool FASTONLY> static int cluster_max_active(int cluster) {
-  if (lean_opt_in<double, LEAN_CLUSTER_NT, 1, FASTONLY, CV>() != cudaSuccess) return 0;
+  if (lean_opt_in<double, LEAN_CLUSTER_NT, 1, FASTONLY, TU_MODEL, TU_LAYOUT>() != cudaSuccess) return 0;
   cudaLaunchAttribute attr;
   const cudaLaunchConfig_t cfg = cluster_config(cluster, cluster, nullptr, &attr);
   int nc = 0;
-  if (cudaOccupancyMaxActiveClusters(&nc, rod_lean_kernel<double, LEAN_CLUSTER_NT, 1, FASTONLY, CV>, &cfg) != cudaSuccess) {
+  if (cudaOccupancyMaxActiveClusters(&nc, rod_lean_kernel<double, LEAN_CLUSTER_NT, 1, FASTONLY, TU_MODEL, TU_LAYOUT>, &cfg) != cudaSuccess) {
     (void)cudaGetLastError();
     return 0;
   }
   return nc;
 }
 
-template <int CVAR> int lean_cluster_max_active(int cluster) {
-  static_assert(CVAR == CV, "one cluster variant per translation unit");
+template <LeanModel MODEL> int lean_cluster_max_active(int cluster) {
+  static_assert(MODEL == TU_MODEL, "one cluster model per translation unit");
   const int a = cluster_max_active<true>(cluster), b = cluster_max_active<false>(cluster);
   return a < b ? a : b;
 }
 
-template int lean_cluster_max_active<CV>(int);
-template cudaError_t launch_lean_cluster_kernel<true, CV>(const RodArgs<double> &, int, cudaStream_t);
-template cudaError_t launch_lean_cluster_kernel<false, CV>(const RodArgs<double> &, int, cudaStream_t);
+template int lean_cluster_max_active<TU_MODEL>(int);
+template cudaError_t launch_lean_cluster_kernel<true, TU_MODEL>(const RodArgs<double> &, int, cudaStream_t);
+template cudaError_t launch_lean_cluster_kernel<false, TU_MODEL>(const RodArgs<double> &, int, cudaStream_t);
 #else
-template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, SR_TU_CONTACT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
-template int lean_ctas_per_sm<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, SR_TU_CONTACT>();
-#if SR_TU_CONTACT != 8   // (the planar variant's fallback is variant 0's safe kernel)
-template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, SR_TU_CONTACT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
-template int lean_ctas_per_sm<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, SR_TU_CONTACT>();
+template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, TU_MODEL, TU_LAYOUT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
+template int lean_ctas_per_sm<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, TU_MODEL, TU_LAYOUT>();
+#if !SR_IS(SR_TU_MODEL)   // (the planar model's fallback is the plain model's safe kernel)
+template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, TU_MODEL, TU_LAYOUT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);
+template int lean_ctas_per_sm<SR_TU_T, SR_TU_NT, SR_TU_MINB, false, TU_MODEL, TU_LAYOUT>();
 #endif
 #endif
 

@@ -1,10 +1,11 @@
-// rod_kernel_lean.cuh — the product kernel, sm_100a.  Variant 0 (template parameter CVAR) is the headline: FP64 or
-// FP32 storage, single rod per env, no contact / filter / joints / forcing (SoftPendulum-v0 and plain rods: BASELINE
-// configs 2 and 3).  Variants 1-7 put the other models on the same skeleton (see the comment at the kernel):
-// 1 plane contact + rest curvature, 2 + travelling-wave muscle, 3 assemblies (arms + rigid head + joints), 4 Laplace
-// filter + moving base, 5 spline muscle torques, 6 / 7 = 0 / 1 with the tip node folded into the last thread, 8 = 0 for
-// rods that stay in the lab x-y plane (out-of-plane terms left out, same bits), 9 / 10 / 11 / 12 = 0 / 4 / 1 / 2 for rods
-// of 512-4095 elements, one rod per thread-block cluster of 2-8 CTAs (same substep, same bits).
+// rod_kernel_lean.cuh — the product kernel, sm_100a.  An instantiation is one model (which substep runs) in one layout
+// (where a rod's nodes live), the template parameters MODEL and LAYOUT (LeanModel, LeanLayout in launch.cuh).  The
+// headline is the plain model in the CTA layout: FP64 or FP32 storage, single rod per env, no contact / filter / joints /
+// forcing (SoftPendulum-v0 and plain rods: BASELINE configs 2 and 3).  The other models put the plane contact + rest
+// curvature, + the travelling-wave muscle, assemblies (arms + rigid head + joints), the Laplace filter + moving base,
+// spline muscle torques and rods that stay in the lab x-y plane (out-of-plane terms left out, same bits) on the same
+// skeleton; the fold layout puts the tip node into the last thread, and the cluster layout spreads a rod of 512-4095
+// elements over a thread-block cluster of 2-8 CTAs (same substep, same bits).  See the comment at the kernel.
 //
 // Same mapping as rod_kernel_packed.cuh (one thread per node/element, rods packed back to back across a
 // 256-thread CTA, state in registers for the whole launch, neighbour data through array-of-structures
@@ -27,9 +28,9 @@
 //    log-map factor theta/sin(theta) is a polynomial in |axial(R - R^T)|^2 (no trace needed); the rotational
 //    damper c_w^e is a cubic in (e - 1) with host-made coefficients; range checks run on the integer pipe.
 //
-// Range handling (both variants compute bit-identical results for every thread whose arguments are in range):
+// Range handling (both kernels compute bit-identical results for every thread whose arguments are in range):
 //   FASTONLY = true : no fallback code; a thread that leaves the range flags its env, whose state is then not
-//                     written back and which the safe variant re-runs (redo[]).
+//                     written back and which the safe kernel re-runs (redo[]).
 //   FASTONLY = false: per-thread fallback to the libm-class reference maps (never a warp vote: an env's bits
 //                     must not depend on which other envs share its warps).
 //
@@ -38,6 +39,7 @@
 #pragma once
 #include <cooperative_groups.h>
 #include <type_traits>
+#include "launch.cuh"
 #include "rod_kernels.cuh"
 
 namespace sr {
@@ -86,7 +88,7 @@ __device__ __forceinline__ void rotate_directors_lean(const double (&cg)[3], con
   for (int i = 0; i < 9; i++) Q[i] = nq[i];
 }
 
-// rotate_directors_lean for a rod in the lab x-y plane (variant 8): the rotation vector is (0, a1, 0) about d2 = +-z, and
+// rotate_directors_lean for a rod in the lab x-y plane (planar model): the rotation vector is (0, a1, 0) about d2 = +-z, and
 // only d1 = (Q0, Q1, 0) and d3 = (Q6, Q7, 0) move.  The same terms as above in the same order, with the ones that carry
 // an exact zero factor left out (D = [[-B a1^2, 0, -A a1], [0, 0, 0], [A a1, 0, -B a1^2]]): the same roundings.
 __device__ __forceinline__ void rotate_directors_planar(const double (&cg)[3], const double (&ch)[3], double a1, double q,
@@ -104,24 +106,24 @@ __device__ __forceinline__ void rotate_directors_planar(const double (&cg)[3], c
 
 constexpr int LEAN_REC = 18;        // exchange record per thread (doubles), 144-byte stride: conflict-free LDS.128
 constexpr int LEAN_JREC = 10;      // assemblies: joint record of an arm's first thread {reaction force, couple on the head, couple on element 0, -}
-// filter variant: records of 6 doubles with 6 ghost records on either side of every rod (rods of >= 9 threads)
+// filter model: records of 6 doubles with 6 ghost records on either side of every rod (rods of >= 9 threads)
 // (8 ghost records per side, 6 used: a rod's records then start a multiple of 8 records = 96 words after where the
 // previous rod's would continue, so a quarter-warp that straddles two rods still hits eight distinct 4-bank groups).
 // A CTA of more than 512 threads holds one rod of >= 512 elements and at most the head of an idle second group, whose
 // records and taps end within 30 records past NT: sized as rods of >= 9 threads, its ghost array alone would take
 // 73 KB at 544 threads and push the 768- and 1024-thread CTAs past the 227 KB a CTA can have.
 constexpr int lean_ghost_records(int nt) { return nt <= 512 ? nt + 16 * (nt / 9) + 16 : nt + 48; }
-// records of each exchange array beyond the NT threads' own: the cluster variants 9-12 have a halo record before
-// thread 0, two after thread NT - 1 and a zero record; the others a zero record and a spare one
-__host__ __device__ constexpr int lean_extra_records(int cvar) { return cvar >= 9 && cvar <= 12 ? 4 : 2; }
-// variant 10: each rank's ghost-padded filter records hold the rod indices [NT c - 8, NT c + NT + 8) (6 of the 8 halo
-// records per side used, as variant 4 pads them)
-constexpr int lean_smem_words(int nt, int cvar = 0) {
-  return (LEAN_REC + 6 + (cvar == 3 ? LEAN_JREC : 0)) * (nt + lean_extra_records(cvar)) +
-         (cvar == 4 ? 6 * lean_ghost_records(nt) : cvar == 10 ? 6 * (nt + 16) : 0);
+// records of each exchange array beyond the NT threads' own: the cluster layout has a halo record before thread 0, two
+// after thread NT - 1 and a zero record; the others a zero record and a spare one
+__host__ __device__ constexpr int lean_extra_records(LeanLayout layout) { return layout == LeanLayout::CLUSTER ? 4 : 2; }
+// filter model on clusters: each rank's ghost-padded filter records hold the rod indices [NT c - 8, NT c + NT + 8) (6 of
+// the 8 halo records per side used, as the CTA layout pads them)
+constexpr int lean_smem_words(int nt, LeanModel model, LeanLayout layout) {
+  return (LEAN_REC + 6 + (model == LeanModel::ASSEMBLY ? LEAN_JREC : 0)) * (nt + lean_extra_records(layout)) +
+         (model != LeanModel::FILTER ? 0 : layout == LeanLayout::CLUSTER ? 6 * (nt + 16) : 6 * lean_ghost_records(nt));
 }
 
-// cluster variants: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
+// cluster layout: the address of `p` in the shared memory of CTA `rank` of this cluster (DSMEM)
 template <typename T> __device__ __forceinline__ T *cluster_smem(T *p, int rank) {
   return cooperative_groups::this_cluster().map_shared_rank(p, (unsigned)rank);
 }
@@ -147,70 +149,78 @@ __device__ __forceinline__ bool out_of_range(float x, int, float limf) { return 
 //     into FP64 frames: 56 FP64 instructions + 35 conversions per element-substep) was tried and was slower still,
 //     1.728 ms: F2F conversions issue at the FP64 rate, and velocity error rose to 3.6e-5 (scripts/gpu_r2n.sh).
 //
-// CONTACT = true (FP64 only): the same skeleton for a single rod on the frictional plane — per-env rest curvature
-// (flat_env.py:310-311 style actuation), RodPlaneContactWithAnisotropicFriction (SURVEY A.5; two more exchanges and
-// per-rod barriers per substep), the MuscleTorques travelling wave of ContinuumSnake-v0, and the internal frame whose
-// z axis is the plane normal (see rod_kernel_packed.cuh).  OctoArmSingle-v0, ContinuumSnake-v0 and BASELINE config 5.
-template <typename ST, int NT, int MINB, bool FASTONLY, int CVAR = 0>
+// Models (MODEL: which substep runs; every model but PLAIN is FP64 only):
+//   PLAIN    one rod under gravity, damping and the base point force, with a free, clamped or slider end.
+//   PLANE    (CONTACT, FP64 only) the same skeleton for a single rod on the frictional plane — per-env rest curvature
+//            (flat_env.py:310-311 style actuation), RodPlaneContactWithAnisotropicFriction (SURVEY A.5; two more
+//            exchanges and per-rod barriers per substep), and the internal frame whose z axis is the plane normal (see
+//            rod_kernel_packed.cuh).  OctoArmSingle-v0 and BASELINE config 5.
+//   MUSCLE   PLANE + the MuscleTorques travelling wave of ContinuumSnake-v0.
+//   ASSEMBLY PLANE for assemblies: several rods + one rigid head thread per env, FixedJoint2Rigid joints,
+//            BodyBoundaryCondition on the head (OctoFlat-v0).
+//   FILTER   SoftPendulum3D-v0: LaplaceDissipationFilter + host-commanded moving base (no contact).
+//   SPLINE   clamped / free rod + MuscleTorquesWithVaryingBetaSplines (SoftArmTracking-v0); safe kernel only, see below.
+//   PLANAR   PLAIN for a rod that stays in the lab x-y plane (SoftPendulum-v0, planar clamped / free rods; the host
+//            checks gravity and the base force).  x_z, v_z, d1_z, d3_z, d2_x, d2_y, w_0, w_2, kappa_0, kappa_2 and
+//            sigma_1 are exact zeros at every substep, and every product that carries one of them is left out: the same
+//            terms in the same order, so the same roundings as PLAIN (up to the sign of zeros).  Nine state registers per
+//            thread instead of 18.  Each segment checks those zeros in its input (and the padding of slot n: Q = I,
+//            w = 0, which the stale observables of the last element and the tip assume); a rod that fails is flagged
+//            like a range failure (cause bit 8) and re-run by PLAIN's safe kernel.
+//
+// Layouts (LAYOUT: where a rod's nodes live):
+//   CTA      rods of n elements packed back to back into one CTA, n + 1 threads each (every model).
+//   FOLD     (PLAIN, PLANE) the tip node folded into the last element's thread: a rod of n elements then takes n
+//            threads, not n + 1 — what lets the 512-element rod (BASELINE config 5) run in a 512-thread CTA with 128
+//            registers instead of a 544-thread one capped at 96 (17 warps put five on one scheduler).  One rod per CTA.
+//   CLUSTER  (PLAIN, FILTER, PLANE, MUSCLE) a rod of 512-4095 elements spread over a thread-block cluster of
+//            C = ceil((n + 1) / NT) CTAs (one rod per cluster, launched with the cluster dimension set at run time):
+//            CTA rank c holds nodes / elements j = NT c + tid.  The substep is the model's, instruction for instruction.
+//            Only where the records come from changes: each exchange array has a halo record before thread 0 (the
+//            stress record of element j - 1, stored there by the previous rank's last thread) and two after thread
+//            NT - 1 (the x, v, Q records of nodes j + 1, j + 2, stored there by the next rank's threads 0 and 1), so
+//            every read of the substep stays a local shared-memory load at the same offset.  The substep's two barriers
+//            become cluster barriers; they order the DSMEM halo stores as the CTA barriers order the local ones (a halo
+//            slot is rewritten only after the barrier that follows its last read).  Env-level decisions (range flags,
+//            NaN flag) are reduced into rank 0's shared memory through DSMEM atomics and read back by every CTA.
+//            FILTER: the filter's pass 0 reads the rate records of j - 1 and j + 1: rec gets a halo at -1 too, and the
+//            filter's own record is pushed into the neighbours' halos -1 / NT.  Each rank's ghost-padded array gb holds
+//            the rod indices [NT c - 8, NT c + NT + 8), and a g record of index k is stored into every rank whose taps
+//            read it (put_g below); the reflected ghosts follow the same rule.  The filter's two barriers become
+//            cluster barriers as well: four per substep.
+//            PLANE, MUSCLE: the plane's two extra exchanges read across the rank boundary too, so the last thread
+//            pushes its stage-1 load into the next rank's rec halo -1 (words 16-17) and its final plane load into the
+//            next rank's sn halo -1; thread 0 pushes its stress record into the previous rank's sn halo NT and its
+//            stage-1 load into the previous rank's rec halo NT (words 16-17).  The contact's two barriers become
+//            cluster barriers: four per substep.  DESIGN.md §4.1 gives the slot-by-slot order.
+template <typename ST, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayout LAYOUT>
 __global__ void __launch_bounds__(NT, MINB)
 rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   using D = double;
   constexpr bool MIXED = sizeof(ST) == 4;
-  // CVAR: 0 plain rod, 1 contact variant, 2 contact variant + travelling-wave muscle, 3 contact variant for assemblies
-  // (several rods + one rigid head thread per env, FixedJoint2Rigid joints, BodyBoundaryCondition on the head)
-  // 4: SoftPendulum3D-v0 — LaplaceDissipationFilter + host-commanded moving base (no contact); 10: the same on a cluster
-  constexpr bool LAPL = CVAR == 4 || CVAR == 10;
-  // 5: clamped / free rod + MuscleTorquesWithVaryingBetaSplines (SoftArmTracking-v0); safe variant only, see below
-  constexpr bool SPL = CVAR == 5;
-  // 6 / 7: variants 0 / 1 with the tip node folded into the last element's thread: a rod of n elements then takes n
-  // threads, not n + 1 — what lets the 512-element rod (BASELINE config 5) run in a 512-thread CTA with 128 registers
-  // instead of a 544-thread one capped at 96 (17 warps put five on one scheduler).  One rod per CTA.
-  constexpr bool FOLD = CVAR == 6 || CVAR == 7;
-  constexpr bool CONTACT = (CVAR >= 1 && CVAR <= 3) || CVAR == 7 || CVAR == 11 || CVAR == 12;
-  constexpr bool MUS = CVAR == 2 || CVAR == 12, MULTI = CVAR == 3;
-  // 8: variant 0 for a rod that stays in the lab x-y plane (SoftPendulum-v0, planar clamped / free rods; the host checks
-  // gravity and the base force).  x_z, v_z, d1_z, d3_z, d2_x, d2_y, w_0, w_2, kappa_0, kappa_2 and sigma_1 are exact zeros
-  // at every substep, and every product that carries one of them is left out: the same terms in the same order, so the
-  // same roundings as variant 0 (up to the sign of zeros).  Nine state registers per thread instead of 18.  Each segment
-  // checks those zeros in its input (and the padding of slot n: Q = I, w = 0, which the stale observables of the last
-  // element and the tip assume); a rod that fails is flagged like a range failure (cause bit 8) and re-run by the 3D
-  // safe kernel.
-  constexpr bool PLANAR = CVAR == 8;
-  static_assert(!PLANAR || FASTONLY, "the planar variant is fast-only: its fallback is the 3D safe kernel");
-  // 9: variant 0 for a rod of 512-4095 elements spread over a thread-block cluster of C = ceil((n + 1) / NT) CTAs (one rod
-  // per cluster, launched with the cluster dimension set at run time): CTA rank c holds nodes / elements j = NT c + tid.
-  // The substep is variant 0's, instruction for instruction.  Only where the records come from changes: each exchange
-  // array has a halo record before thread 0 (the stress record of element j - 1, stored there by the previous rank's
-  // last thread) and two after thread NT - 1 (the x, v, Q records of nodes j + 1, j + 2, stored there by the next rank's
-  // threads 0 and 1), so every read of the substep stays a local shared-memory load at the same offset.  The substep's
-  // two barriers become cluster barriers; they order the DSMEM halo stores as the CTA barriers order the local ones (a
-  // halo slot is rewritten only after the barrier that follows its last read).  Env-level decisions (range flags, NaN
-  // flag) are reduced into rank 0's shared memory through DSMEM atomics and read back by every CTA.
-  // 10: variant 4 in variant 9's layout (SoftPendulum3D-v0 at 512-4095 elements).  The filter's pass 0 reads the rate
-  // records of j - 1 and j + 1: rec gets a halo at -1 too, and the filter's own record is pushed into the neighbours'
-  // halos -1 / NT.  Each rank's ghost-padded array gb holds the rod indices [NT c - 8, NT c + NT + 8), and a g record
-  // of index k is stored into every rank whose taps read it (put_g below); the reflected ghosts follow the same rule.
-  // The filter's two barriers become cluster barriers as well: four per substep.
-  // 11 / 12: variants 1 / 2 in variant 9's layout (the rod on the frictional plane at 512-4095 elements).  The plane's two
-  // extra exchanges read across the rank boundary too, so the last thread pushes its stage-1 load into the next rank's
-  // rec halo -1 (words 16-17) and its final plane load into the next rank's sn halo -1; thread 0 pushes its stress
-  // record into the previous rank's sn halo NT and its stage-1 load into the previous rank's rec halo NT (words 16-17).
-  // The contact's two barriers become cluster barriers: four per substep.  DESIGN.md §4.1 gives the slot-by-slot order.
-  constexpr bool CLUSTER = CVAR >= 9 && CVAR <= 12;
-  static_assert(CVAR == 0 || !MIXED, "the variants are FP64 only");
+  constexpr bool CONTACT = MODEL == LeanModel::PLANE || MODEL == LeanModel::MUSCLE || MODEL == LeanModel::ASSEMBLY;
+  constexpr bool MUS = MODEL == LeanModel::MUSCLE, MULTI = MODEL == LeanModel::ASSEMBLY;
+  constexpr bool LAPL = MODEL == LeanModel::FILTER;
+  constexpr bool SPL = MODEL == LeanModel::SPLINE;
+  constexpr bool PLANAR = MODEL == LeanModel::PLANAR;
+  constexpr bool FOLD = LAYOUT == LeanLayout::FOLD;
+  constexpr bool CLUSTER = LAYOUT == LeanLayout::CLUSTER;
+  static_assert(!PLANAR || FASTONLY, "the planar model is fast-only: its fallback is the 3D safe kernel");
+  static_assert((MODEL == LeanModel::PLAIN && LAYOUT == LeanLayout::CTA) || !MIXED, "FP64 only");
   static_assert(!FOLD || LEAN_SCR_FOLD >= 27, "hand-over rows of the folded tip");
   constexpr int SCR = FOLD ? LEAN_SCR_FOLD : CONTACT ? LEAN_SCR_CONTACT : LEAN_REC;   // rows of a slot's hand-over scratch
   using F = typename std::conditional<MIXED, float, double>::type;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int SNR = MIXED ? 8 : 6;
-  constexpr int RX = lean_extra_records(CVAR);
-  constexpr int ZR = CLUSTER ? NT + 2 : NT;   // record ZR = zeros (left of element 0); variant 9: -1, NT, NT + 1 are halos
+  constexpr int RX = lean_extra_records(LAYOUT);
+  constexpr int ZR = CLUSTER ? NT + 2 : NT;   // record ZR = zeros (left of element 0); cluster layout: -1, NT, NT + 1 are halos
   D *rec = reinterpret_cast<D *>(smem_raw) + (CLUSTER ? LEAN_REC : 0);   // {x0 x1 | x2 v0 | v1 v2 | Q0 Q1 | ... | Q6 Q7 | Q8 - | - -}
   // {s0 s1 | s2 N0 | N1 m2} (FP64: 48-byte records; mixed: 8 floats, 32-byte records)
   F *sn = reinterpret_cast<F *>(reinterpret_cast<D *>(smem_raw) + LEAN_REC * (NT + RX)) + (CLUSTER ? SNR : 0);
   __shared__ int sh_flag[256], sh_dom[256];   // one per rod of the CTA (<= NT / 4)
-  __shared__ int sh_need[CVAR == 5 ? 128 : 1];          // spline variant: which directions re-fit their magnitudes this substep, per rod
-  __shared__ double sh_base[CVAR == 4 ? 128 : 1][4];   // filter variant: the moving base's command, per rod (rods of >= 9 threads; variant 10: rank 0's one rod)
+  __shared__ int sh_need[SPL ? 128 : 1];      // spline model: which directions re-fit their magnitudes this substep, per rod
+  // filter model: the moving base's command, per rod (rods of >= 9 threads; cluster layout: rank 0's one rod in row 0)
+  __shared__ double sh_base[LAPL && !CLUSTER ? 128 : 1][4];
 
   const int tid = threadIdx.x;
   const int n = A.n_elem, stride = A.stride, tpr = FOLD ? n : n + 1;
@@ -224,13 +234,13 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   const bool is_head = MULTI && has_head && (u_grp == G - 1);
   const int arm = (MULTI && !is_head) ? u_grp / tpr : 0;
   const int j = is_head ? 0 : u_grp - arm * tpr;
-  const bool in_cta = r < rods_per_cta && (!CLUSTER || j <= n);   // (variant 9: the last rank's threads past the tip idle)
+  const bool in_cta = r < rods_per_cta && (!CLUSTER || j <= n);   // (cluster layout: the last rank's threads past the tip idle)
   const bool first = (j == 0) && !is_head;          // first thread of a rod
   const bool lead = first && arm == 0;              // one thread per env: env-level flags and outputs
   const int t_head = r * G + G - 1;                 // where this env's head publishes its state
   // past the stress records: assemblies: joint records (LEAN_JREC doubles per thread slot)
   D *sj = reinterpret_cast<D *>(sn - (CLUSTER ? SNR : 0) + 6 * (NT + RX));
-  D *gb = sj;                                       // filter variant: ghost-padded records of the filtered rates
+  D *gb = sj;                                       // filter model: ghost-padded records of the filtered rates
   if (tid < SNR) sn[SNR * ZR + tid] = F(0);
   if (CLUSTER && tid < 256) { sh_dom[tid] = 0; sh_flag[tid] = 0; }   // (rank 0's are the cluster's env-level flags)
   if (CONTACT && tid < 2) rec[LEAN_REC * ZR + 16 + tid] = D(0);   // stage-1 contact load "left of element 0"
@@ -261,7 +271,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     if (bar_cnt1) asm volatile("bar.sync %0, %1;" ::"r"(bar_id1), "r"(bar_cnt1) : "memory");
   };
 
-  // contact variant: lab <-> internal frame (z = plane normal), a signed permutation for axis-aligned normals
+  // plane models: lab <-> internal frame (z = plane normal), a signed permutation for axis-aligned normals
   const bool rot_frame = CONTACT && A.rot_on;
   auto to_int = [&](D (&u)[3]) {
     if (!rot_frame) return;
@@ -289,7 +299,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   const D c_cv = MIXED ? A.k_c_v : (D)A.c_v;
 
   // redo_count: [0] env-steps handed over for leaving the fast-math range, [1..3] by cause (an env can count under
-  // several); [4] env-steps the planar variant handed over for not being planar (no range failure)
+  // several); [4] env-steps the planar model handed over for not being planar (no range failure)
   auto count_redo = [&](int dom) {
     if (PLANAR && (dom & 8)) { atomicAdd(A.redo_count + 4, 1ULL); return; }
     atomicAdd(A.redo_count, 1ULL);
@@ -298,7 +308,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
 
   // ---- the segments this CTA runs ------------------------------------------------------------------------------
   const int K = A.n_substeps;
-  const int P = gridDim.x, p = CLUSTER ? blockIdx.x / c_size : blockIdx.x;   // (variant 9: one item per cluster)
+  const int P = gridDim.x, p = CLUSTER ? blockIdx.x / c_size : blockIdx.x;   // (cluster layout: one item per cluster)
   int i0, i1, off0, end1;
   if (A.sk_split) {
     const long long W = (long long)A.sk_items * K, b0 = W * p / P, b1 = W * (p + 1) / P;
@@ -334,19 +344,19 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     const int rod = env * n_rod + arm;                 // global rod slot in the state arrays
     int dom_bad = 0;                                   // which range a fast-only thread left: 1 rotation, 2 bend, 4 stretch (damper map)
     const bool elem_ok = active && j < n, vor_ok = active && j < n - 1;
-    // (folded variants: the tip node's record is record NT, published by the last element's thread)
+    // (fold layout: the tip node's record is record NT, published by the last element's thread)
     const int t_next = elem_ok ? ((FOLD && j == n - 1) ? NT : tid + 1) : tid;
     const int t_next2 = vor_ok ? ((FOLD && j == n - 2) ? NT : tid + 2) : t_next;
     const int t_prev = (active && j > 0) ? tid - 1 : ZR;
 
     D x[3] = {D(0), D(0), D(0)}, v[3] = {D(0), D(0), D(0)}, w[3] = {D(0), D(0), D(0)};
     D Q[9] = {D(1), D(0), D(0), D(0), D(1), D(0), D(0), D(0), D(1)};
-    D xt[3] = {D(0), D(0), D(0)}, vt[3] = {D(0), D(0), D(0)};   // folded variants: the tip node, integrated by the last element's thread
+    D xt[3] = {D(0), D(0), D(0)}, vt[3] = {D(0), D(0), D(0)};   // fold layout: the tip node, integrated by the last element's thread
     const bool is_last = FOLD && active && j == n - 1;
     ST *st = A.state + (size_t)(active ? rod : 0) * N_FIELDS * stride;
     const ST *bc = A.bc + (size_t)(active ? rod : 0) * BC_DIM;
     ST *hd = (MULTI && is_head && live) ? A.head + (size_t)env * HEAD_DIM : nullptr;   // the rigid head's state
-    // travelling-wave muscle torque (contact variant): time, (sin, cos) of the wave's common phase w t + phi, and this
+    // travelling-wave muscle torque (muscle model): time, (sin, cos) of the wave's common phase w t + phi, and this
     // element's two amplitude combinations (below)
     const bool mus = MUS && A.muscle_on;
     D mus_t = D(0), mus_S = D(0), mus_C = D(1);
@@ -438,7 +448,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // never moving the pinned quantities is the same thing (see rod_kernel_packed.cuh): the BC thread integrates its
     // frame with a zero rotation vector
     if constexpr (PLANAR) {
-      // the zeros this variant relies on, in the pre-launch state (the same for every segment of an item)
+      // the zeros this model relies on, in the pre-launch state (the same for every segment of an item)
       if (active) {
         auto f = [&](int field) { return (D)st[field * stride + j]; };
         bool flat = f(F_POS + 2) == D(0) && f(F_VEL + 2) == D(0);
@@ -476,7 +486,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         if (CONTACT) { rows_to_int(Q); to_int(x); }
       }
     }
-    // contact variant: rest curvature at Voronoi point j (actuation), constant during a launch; the muscle wave
+    // plane models: rest curvature at Voronoi point j (actuation), constant during a launch; the muscle wave
     D rk[3] = {D(0), D(0), D(0)};
     D mus_P = D(0), mus_R = D(0);
     if constexpr (CONTACT) {
@@ -485,7 +495,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         for (int c = 0; c < 3; c++) rk[c] = (D)A.rest_kappa[((size_t)rod * 3 + c) * stride + j];
       }
       if (mus && active) {
-        // (the cluster variant: every rank reads the clock mu[0] here, ahead of its first cluster barrier of the item;
+        // (the cluster layout: every rank reads the clock mu[0] here, ahead of its first cluster barrier of the item;
         // rank 0's lead alone writes it back, after the last one)
         // MuscleTorques (continuum_snake.py:186-198): element k gets Q_k d (m_k [k >= 1] - m_{k+1} [k <= n-2]),
         // m_k = min(1, t/ramp) beta_{n-1-k} sin(w t - kw s_{n-1-k} + phi).  sin(p - s) = sin p cos s - cos p sin s, so
@@ -513,7 +523,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // direction d, external_torques[d, k] += mag_d[k]; mag is re-evaluated (not-a-knot cubic through the rate-limited
     // control values, at s = cumsum(current lengths)) in every substep that finds the cached values different from the
     // caller's targets, and kept otherwise — across launches too (the cache lives in HBM, A.spline).  The forcing
-    // mutates that cache inside the launch, so this variant only exists as the safe kernel (a fast-only run that is
+    // mutates that cache inside the launch, so this model only exists as the safe kernel (a fast-only run that is
     // re-done would apply the rate limit twice).
     const bool spl = SPL && A.spline_mask != 0;
     double *sp = (spl && active) ? A.spline + (size_t)env * A.spline_dim : nullptr;
@@ -602,7 +612,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     };
     if (s_begin == 0 && K > 0) { kinematic(c_half_dt, D(1e-14)); head_constrain_values(); }
 
-    bool spl_settled = false;   // spline variant: the cached control values have reached their targets
+    bool spl_settled = false;   // spline model: the cached control values have reached their targets
     bool check_trace = true;   // first substep of the segment: rule out a state that starts beyond 90 degrees of bend
     auto substep = [&](auto last_tag, int s_now) {
       constexpr bool last = decltype(last_tag)::value;
@@ -799,7 +809,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       // the first substep of a segment checks the trace once to rule out a state that starts beyond.
       F w2 = dot3(vec, vec);
       if (!vor_ok) w2 = F(0);
-      constexpr bool MIDBEND = CVAR == 1 || CVAR == 2 || CVAR == 7 || CVAR == 11 || CVAR == 12;   // actuated arms on the plane: the 37-degree map
+      constexpr bool MIDBEND = MODEL == LeanModel::PLANE || MODEL == LeanModel::MUSCLE;   // actuated arms on the plane: the 37-degree map
       bool bend_out = out_of_range(w2, MIDBEND ? A.lim_bendm_hi : A.lim_bend_hi, A.limf_bend);
       F u_ref = F(0);
       if constexpr (MULTI) {
@@ -824,8 +834,8 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         const D cot = fma(D(-2.0), u_ref, D(1.0)) * rsqrt_approx(D(4.0) * u_ref * (D(1.0) - u_ref));   // scales the 1e-14 guard term only
         fs = g * fma(D(0.5e-14), cot, D(-0.5)) * A.inv_rest_vor;
       } else {
-        // ascending powers of w2 (degree 9), pre-multiplied by -1/(2 D); even / odd halves interleaved.  (Contact
-        // variant: indexed through a register the compiler cannot see through, so that the ten coefficients are
+        // ascending powers of w2 (degree 9), pre-multiplied by -1/(2 D); even / odd halves interleaved.  (Plane
+        // models: indexed through a register the compiler cannot see through, so that the ten coefficients are
         // constant-bank loads inside the loop instead of hoisted, spilled and reloaded registers.)
         const F *c = MIDBEND ? Z.bendw_mid : Z.bendw;
         const F z = w2 * w2;
@@ -982,7 +992,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
           for (int i = 0; i < 3; i++) { fint[i] += fj[i]; tq[i] += tj[i]; }
         }
       }
-      D ct[3] = {D(0), D(0), D(0)};      // folded variants: the tip node's half of the plane's load on the last element
+      D ct[3] = {D(0), D(0), D(0)};      // fold layout: the tip node's half of the plane's load on the last element
       if constexpr (CONTACT) {
         // forcing registered before the contact: the static-friction torque balance sees the muscle couple
         if (mus && !A.contact_before_forcing) {
@@ -1181,7 +1191,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
           // its twelve neighbours at fixed offsets.  Nodes reflect about node n, elements about element n-1, so the
           // two halves of a right-hand ghost record come from different threads.
           auto laplace = [&]() {
-            if (A.laplace_order != 7) return;    // (the host only selects this variant for order 7 or none)
+            if (A.laplace_order != 7) return;    // (the host only selects this model for order 7 or none)
             const bool node_in = active && j > 0 && j < n, elem_in = active && j > 0 && j < n - 1;
             double2 *own = reinterpret_cast<double2 *>(rec + LEAN_REC * tid);
             own[0] = make_double2(v[0], v[1]); own[1] = make_double2(v[2], w[0]); own[2] = make_double2(w[1], w[2]);
@@ -1205,7 +1215,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
               for (int c = 0; c < 6; c++) g[c] = ((-rv[c] - lv[c]) + D(2) * mv[c]) * D(0.25);
             }
             D *slot = gb + 6 * (CLUSTER ? 8 + tid : r * (tpr + 16) + 8 + j);
-            // put_g(k, store): `store` writes into the record of rod index k.  Variant 10: into that of every rank whose
+            // put_g(k, store): `store` writes into the record of rod index k.  Cluster layout: into that of every rank whose
             // taps read index k, i.e. whose window [NT c - 6, NT c + NT + 6) holds it — its owner, the previous rank for
             // the first six indices of a rank, the next one for the last six; the ghosts beyond both ends alike.  A
             // thread stores its own index and ghosts at most 13 indices away, so only its own rank and the two next to
@@ -1224,7 +1234,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
                 }
               }
             };
-            if (!CLUSTER || in_cta) {   // (variant 10: the last rank's idle threads hold indices past the ghosts)
+            if (!CLUSTER || in_cta) {   // (cluster layout: the last rank's idle threads hold indices past the ghosts)
               put_g(j, [&](D *p) {
                 double2 *o = reinterpret_cast<double2 *>(p);
                 if (j < n) { o[0] = make_double2(g[0], g[1]); o[1] = make_double2(g[2], g[3]); o[2] = make_double2(g[4], g[5]); }
@@ -1280,7 +1290,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       kinematic(last ? c_half_dt : c_dt, last ? D(1e-14) : D(2e-14));
       head_constrain_values();
     };
-    // variant 8: the substep above with the out-of-plane terms left out (see PLANAR).  Records {x0 x1 | v0 v1 | Q0 Q1 |
+    // planar model: the substep above with the out-of-plane terms left out (see PLANAR).  Records {x0 x1 | v0 v1 | Q0 Q1 |
     // Q6 Q7} and {s0 s1 | N1}.  The pseudo-element of the tip / idle threads lies along x here instead of z (same
     // length; its stress is discarded either way), so the tip's stale observables are rebuilt in the last substep.
     auto substep_planar = [&](auto last_tag) {
@@ -1366,7 +1376,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         cw0 = fma(fma((D)A.cwp[0][2], em1, (D)A.cwp[0][1]), em1, (D)A.cwp[0][0]);
       }
       if (last && active) {
-        // stale observables, as variant 0 computes them.  Its tip thread holds Q = I and the edge (0, 0, l0); its
+        // stale observables, as the plain model computes them.  Its tip thread holds Q = I and the edge (0, 0, l0); its
         // last element forms the curvature against that I: axial(I Q^T - Q) = (d2z - Q7, Q6, Q1).
         D tg[3] = {dx0 * ilg, dx1 * ilg, D(0)}, kp[3] = {D(0), kp1, D(0)};
         D sg0 = Qdx0 * irg, sg2 = s3;

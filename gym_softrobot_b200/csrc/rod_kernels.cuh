@@ -103,9 +103,9 @@ template <typename T> struct RodArgs {
   T half_inv_rest_vor;                // 1 / (2 D)
   T dt_Jinv0;                         // dt / J1
   T bendw[10];                        // -theta'/(2 D sin theta') as a polynomial in |axial(R - R^T)|^2 (SR_COEF_BENDW)
-  T bendw_mid[14]; int lim_bendm_hi;  // the same on the wider range of the contact variants (SR_COEF_BENDW_MID)
+  T bendw_mid[14]; int lim_bendm_hi;  // the same on the wider range of the plane models (SR_COEF_BENDW_MID)
   T cwp[2][3];                        // c_w^e as a quadratic in (e - 1), components 0 (= 1) and 2
-  // contact variant of the lean kernel: c_w^e to degree 6 (|z| <= kLeanExpZc), D / 2, the travelling wave's rotation
+  // the lean kernel's plane models: c_w^e to degree 6 (|z| <= kLeanExpZc), D / 2, the travelling wave's rotation
   // per substep (cos / sin of mus_omega dt) and 1 / ramp-up time
   T cwc[2][7], half_rest_vor; int lim_em1c_hi;
   double mus_cd, mus_sd, mus_inv_ramp;

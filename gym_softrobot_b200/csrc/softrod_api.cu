@@ -56,7 +56,7 @@ struct sr_handle {
   unsigned long long *redo_count = nullptr, *h_redo_count = nullptr, pair_last_count = 0;   // counts: see count_redo (lean kernel)
   cudaEvent_t pair_event = nullptr; bool pair_copy_pending = false;
   long long pair_steps = 0, pair_off_until = 0, pair_steps_at_copy = 0, pair_steps_at_prev_copy = 0;
-  unsigned long long planar_last_count = 0; long long planar_off_until = 0;   // the planar variant's own window
+  unsigned long long planar_last_count = 0; long long planar_off_until = 0;   // the planar model's own window
   int n_rod = 1, init_dim = 9;
   sr::RodArgs<double> a64;
   sr::RodArgs<float> a32;
@@ -247,8 +247,8 @@ int cuda_fail(const char *what, cudaError_t e) {
 struct Switches {
   bool fastpath;   // SOFTROD_FASTPATH=0: the single safe kernel with per-thread fallbacks instead of the pair
   bool planar;     // SOFTROD_LEAN_PLANAR=0: rods in the x-y plane take the 3D kernels too
-  bool cluster;    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster variants too
-  bool fold;       // SOFTROD_LEAN_FOLD=0: a rod of 512 elements takes a 544-thread CTA instead of the folded-tip variant
+  bool cluster;    // SOFTROD_LEAN_CLUSTER=1: rods of 512-1023 elements take the cluster layout too
+  bool fold;       // SOFTROD_LEAN_FOLD=0: a rod of 512 elements takes a 544-thread CTA instead of the fold layout
 };
 const Switches &switches() {
   static const Switches s = [] {
@@ -322,13 +322,20 @@ template <typename F> int with_cta(int nt, F &&launch) {
   return fail(SR_E_INVALID, "no kernel is built for CTAs of " + std::to_string(nt) + " threads");
 }
 
-// Of those sizes, the ones build.py compiles lean variant CV at: the folded-tip variants at 512 threads only, the planar
-// variant up to 512 and the filter variant up to 768 (its 1024-thread CTA would need 243 KB of shared memory).
-constexpr bool lean_built(int cv, int nt) {
-  return (cv == 6 || cv == 7) ? nt == 512 : cv == 8 ? nt <= 512 : cv == 4 ? nt <= 768 : true;
+using sr::LeanLayout;
+using sr::LeanModel;
+
+// Of those sizes, the ones build.py's LEAN_UNITS compile a one-CTA lean model and layout at: the fold layout at 512
+// threads only, the planar model up to 512 and the filter model up to 768 (its 1024-thread CTA would need 243 KB of
+// shared memory).
+constexpr bool lean_built(LeanModel model, LeanLayout layout, int nt) {
+  return layout == LeanLayout::FOLD ? nt == 512
+         : model == LeanModel::PLANAR ? nt <= 512
+         : model == LeanModel::FILTER ? nt <= 768
+                                      : true;
 }
 
-// CTA size of the generic kernel and of the assembly variant.  Registers cap the SM at 512 resident threads (128 regs),
+// CTA size of the generic kernel and of the assembly model.  Registers cap the SM at 512 resident threads (128 regs),
 // so the choice is 2 x 256 or 1 x 512; take whichever wastes fewer lanes for this rod length
 // (n = 50: 5 x 51 = 255/256; n = 100: 2 x 101 = 202/256 but 5 x 101 = 505/512).
 int packed_threads_setting(int n_elem, int n_rod = 1, int has_head = 0) {
@@ -345,7 +352,7 @@ int packed_threads_setting(int n_elem, int n_rod = 1, int has_head = 0) {
   return best;
 }
 
-// CTA size of the one-CTA lean variants of a single rod.  With per-rod barriers one 512-thread CTA per SM (16 warps,
+// CTA size of the one-CTA lean kernels of a single rod.  With per-rod barriers one 512-thread CTA per SM (16 warps,
 // 10 rods of n = 50) beats two of 256 (measured: 1.51 vs 1.64 ms per 4096-env step): take 512 whenever it wastes no
 // more lanes.
 int lean_threads_setting(int n_elem) {
@@ -358,34 +365,35 @@ int lean_threads_setting(int n_elem) {
   return best;
 }
 
-// CTAs of the cluster that holds one rod of n elements in the cluster variants (9-12): n + 1 threads of 512 per CTA
+// CTAs of the cluster that holds one rod of n elements in the cluster layout: n + 1 threads of 512 per CTA
 int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
 
-// The cluster variant that steps a rod of the plain model (9: variant 0's substep), of SoftPendulum3D-v0's (10: variant
-// 4's, with the Laplace filter and the moving base), or the rod on the frictional plane with rest-curvature actuation
-// (`loads`: 11, variant 1's) and the travelling-wave muscle (12, variant 2's).  sr_create checks its cluster shape for
-// rods of 1024-4095 elements, the only models it admits there.
-int lean_cluster_variant(int laplace_order, int bc_kind, bool loads, bool muscle_on) {
-  if (loads) return muscle_on ? 12 : 11;
-  return laplace_order > 0 || bc_kind == sr::BC_MOVING_BASE ? 10 : 9;
+// The model a rod steps with in the cluster layout: the plain model, SoftPendulum3D-v0's (the Laplace filter and the
+// moving base), or the rod on the frictional plane with rest-curvature actuation (`loads`) and the travelling-wave
+// muscle.  sr_create checks its cluster shape for rods of 1024-4095 elements, the only models it admits there.
+LeanModel lean_cluster_model(int laplace_order, int bc_kind, bool loads, bool muscle_on) {
+  if (loads) return muscle_on ? LeanModel::MUSCLE : LeanModel::PLANE;
+  return laplace_order > 0 || bc_kind == sr::BC_MOVING_BASE ? LeanModel::FILTER : LeanModel::PLAIN;
 }
 
-// clusters of C CTAs that both kernels of cluster variant cv can keep resident at once (0: none)
-int cluster_max_active(int cv, int C) {
-  switch (cv) {
-    case 10: return sr::lean_cluster_max_active<10>(C);
-    case 11: return sr::lean_cluster_max_active<11>(C);
-    case 12: return sr::lean_cluster_max_active<12>(C);
+// The one cluster dispatcher: a run-time cluster model to the template argument of the cluster kernels build.py
+// compiles; launch(std::integral_constant<LeanModel, M>()).
+template <typename F> auto with_cluster_model(LeanModel model, F &&launch) {
+  using M = LeanModel;
+  switch (model) {
+    case M::FILTER: return launch(std::integral_constant<M, M::FILTER>());
+    case M::PLANE: return launch(std::integral_constant<M, M::PLANE>());
+    case M::MUSCLE: return launch(std::integral_constant<M, M::MUSCLE>());
+    default: return launch(std::integral_constant<M, M::PLAIN>());   // (lean_cluster_model returns no other model)
   }
-  return sr::lean_cluster_max_active<9>(C);
 }
 
 // What steps a handle (classify): the launcher of one kernel, and the launch's shape.
 template <typename T> struct StepKernel {
   int (*launch)(sr_handle *, sr::RodArgs<T> &, const StepKernel &, cudaStream_t);
-  int nt;        // CTA size of the one-CTA lean variants and the generic kernel
+  int nt;        // CTA size of the one-CTA lean kernels and the generic kernel
   bool pair;     // fast-only kernel + fallback (run_pair)
-  bool planar;   // lean variant 0: the fast-only kernel is the planar variant 8 while the handle's planar window allows
+  bool planar;   // plain model, CTA layout: the fast-only kernel is the planar model's while the handle's planar window allows
 };
 
 template <typename T, int NT, int MINB, bool LAPLACE, bool MOVING, bool CONTACT, bool MULTI, bool TORQUE = false,
@@ -404,8 +412,9 @@ int launch_packed_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
 // Lean FP64 path: grid and stream-K schedule.  With more items than resident CTA slots the grid is the slot
 // count and every slot gets the same number of item-substeps (rod_kernel_lean.cuh); partial items travel through
 // sk_scratch.  The fallback launch (redo_filter) visits flagged envs only and keeps one CTA per item.
-template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int launch_lean_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
-  const bool multi = CONTACT == 3, fold = CONTACT == 6 || CONTACT == 7;   // (fold: the tip node lives in the last element's thread)
+template <typename T, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayout LAYOUT>
+int launch_lean_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
+  const bool multi = MODEL == LeanModel::ASSEMBLY, fold = LAYOUT == LeanLayout::FOLD;   // (fold: the tip node lives in the last element's thread)
   const int group = fold ? A.n_elem : (multi ? A.n_rod : 1) * (A.n_elem + 1) + (multi ? A.has_head : 0);
   const int rods_per_cta = NT / group;   // env groups per CTA
   if (rods_per_cta < 1) return fail(SR_E_INVALID, "environment does not fit one CTA of the lean kernel");
@@ -413,7 +422,7 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int laun
   // resident CTAs per SM of this kernel (a property of the kernel and the device model: asked once); the slot count
   // differs between the kernels of a handle, the scratch is sized for the largest
   static int ctas_per_sm = 0;
-  if (ctas_per_sm == 0) ctas_per_sm = sr::lean_ctas_per_sm<T, NT, MINB, FASTONLY, CONTACT>();
+  if (ctas_per_sm == 0) ctas_per_sm = sr::lean_ctas_per_sm<T, NT, MINB, FASTONLY, MODEL, LAYOUT>();
   if (ctas_per_sm < 1) return fail(SR_E_CUDA, "lean kernel: occupancy query failed");
   if (h->sk_sms == 0) {
     cudaDeviceProp prop;
@@ -433,52 +442,48 @@ template <typename T, int NT, int MINB, bool FASTONLY, int CONTACT = 0> int laun
   A.sk_split = (!A.redo_filter && items > slots && A.n_substeps > 0) ? 1 : 0;
   A.sk_scratch = (double *)h->sk_scratch; A.sk_flag = h->sk_flag;
   const int grid = A.sk_split ? slots : items;
-  cudaError_t e = sr::launch_lean_kernel<T, NT, MINB, FASTONLY, CONTACT>(A, grid, s);
+  cudaError_t e = sr::launch_lean_kernel<T, NT, MINB, FASTONLY, MODEL, LAYOUT>(A, grid, s);
   h->launches++;
   if (e != cudaSuccess) return cuda_fail("rod_lean_kernel launch", e);
   return SR_OK;
 }
 
-// one-CTA lean variant CV of rod_kernel_lean.cuh in CTAs of k.nt threads
-template <typename T, int CV> int launch_lean(sr_handle *h, sr::RodArgs<T> &A, const StepKernel<T> &k, cudaStream_t s) {
+// the lean kernel (rod_kernel_lean.cuh) of one model in the CTA or fold layout, in CTAs of k.nt threads
+template <typename T, LeanModel MODEL, LeanLayout LAYOUT> int launch_lean(sr_handle *h, sr::RodArgs<T> &A, const StepKernel<T> &k, cudaStream_t s) {
   return with_cta(k.nt, [&](auto cta) {
     using C = decltype(cta);
-    if constexpr (!lean_built(CV, C::NT)) {
-      return fail(SR_E_INVALID, "rod_lean_kernel: variant " + std::to_string(CV) + " is not built for " + std::to_string(C::NT) + " threads");
+    if constexpr (!lean_built(MODEL, LAYOUT, C::NT)) {
+      static const char *const model[] = {"plain", "plane", "muscle", "assembly", "filter", "spline", "planar"};   // LeanModel's order
+      static const char *const layout[] = {"CTA", "fold", "cluster"};                                            // LeanLayout's order
+      return fail(SR_E_INVALID, std::string("rod_lean_kernel: the ") + model[(int)MODEL] + " model in the " + layout[(int)LAYOUT] +
+                                    " layout is not built for " + std::to_string(C::NT) + " threads");
     } else {
       return run_pair(h, A, k.pair, s, [&](auto fast) {
         constexpr bool FAST = decltype(fast)::value;
-        if constexpr (FAST && CV == 0 && std::is_same<T, double>::value && lean_built(8, C::NT)) {
+        if constexpr (FAST && MODEL == LeanModel::PLAIN && LAYOUT == LeanLayout::CTA && std::is_same<T, double>::value &&
+                      lean_built(LeanModel::PLANAR, LeanLayout::CTA, C::NT)) {
           // when more than 1 % of a window's env-steps were handed over for not being planar, the handle steps with
           // the 3D pair for the next 512 steps (use_fast_pair)
-          if (k.planar && h->pair_steps >= h->planar_off_until) return launch_lean_impl<T, C::NT, C::MINB, true, 8>(h, A, s);
+          if (k.planar && h->pair_steps >= h->planar_off_until)
+            return launch_lean_impl<T, C::NT, C::MINB, true, LeanModel::PLANAR, LeanLayout::CTA>(h, A, s);
         }
-        return launch_lean_impl<T, C::NT, C::MINB, FAST, CV>(h, A, s);
+        return launch_lean_impl<T, C::NT, C::MINB, FAST, MODEL, LAYOUT>(h, A, s);
       });
     }
   });
 }
 
-// cluster variant CV: one rod per thread-block cluster, no stream-K split
-template <int CV> int launch_cluster(sr_handle *h, sr::RodArgs<double> &A, const StepKernel<double> &k, cudaStream_t s) {
+// the lean kernel of one model in the cluster layout: one rod per thread-block cluster, no stream-K split
+template <LeanModel MODEL> int launch_cluster(sr_handle *h, sr::RodArgs<double> &A, const StepKernel<double> &k, cudaStream_t s) {
   const int C = lean_cluster_size(A.n_elem);
   A.sk_rods_per_cta = 1; A.sk_items = A.n_env; A.sk_split = 0;
   A.sk_scratch = nullptr; A.sk_flag = nullptr;
   return run_pair(h, A, k.pair, s, [&](auto fast) {
-    cudaError_t e = sr::launch_lean_cluster_kernel<decltype(fast)::value, CV>(A, C, s);
+    cudaError_t e = sr::launch_lean_cluster_kernel<decltype(fast)::value, MODEL>(A, C, s);
     h->launches++;
     if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
     return SR_OK;
   });
-}
-// the classify row of cluster variant cv
-StepKernel<double> cluster_kernel(int cv) {
-  switch (cv) {
-    case 10: return {launch_cluster<10>, 0, true};
-    case 11: return {launch_cluster<11>, 0, true};
-    case 12: return {launch_cluster<12>, 0, true};
-  }
-  return {launch_cluster<9>, 0, true};
 }
 
 // the generic kernel (rod_kernel_packed.cuh) with the features of one group
@@ -530,8 +535,8 @@ int launch_faithful(sr_handle *h, sr::RodArgs<double> &A, const StepKernel<doubl
 }
 
 // The one classification: the kernel that steps this handle.  One row per kernel in precedence order; a config takes
-// the first row whose model it is.  The lean variants' models share their exclusions: none of them steps suckers,
-// external loads or per-element constants, and all but the plain one (variant 0) need FP64 and no base point force.
+// the first row whose model it is.  The lean kernel's models share their exclusions: none of them steps suckers,
+// external loads or per-element constants, and all but the plain one need FP64 and no base point force.
 template <typename T> StepKernel<T> classify(const sr_handle *h, const sr::RodArgs<T> &A) {
   constexpr bool F64 = std::is_same<T, double>::value;
   const Switches &sw = switches();
@@ -541,44 +546,49 @@ template <typename T> StepKernel<T> classify(const sr_handle *h, const sr::RodAr
   const bool free_or_clamped = bc == sr::BC_FREE || bc == sr::BC_ONE_END_FIXED;
   const bool lean_plain = !(A.sucker || A.ext_force || A.ext_couple || A.elem_tab);
   const bool lean = F64 && lean_plain && !A.point_force;
-  const bool loads = A.contact_on || A.rest_kappa || A.muscle_on;   // the contact variants' plane and actuations
-  // variant 0: one rod under gravity, damping and the base point force, with a free, clamped or slider end
+  const bool loads = A.contact_on || A.rest_kappa || A.muscle_on;   // the plane models' plane and actuations
+  // the plain model: one rod under gravity, damping and the base point force, with a free, clamped or slider end
   const bool plain = lean_plain && !assembly && !loads && !A.spline_mask && A.laplace_order == 0 && bc != sr::BC_MOVING_BASE;
-  // variant 4, SoftPendulum3D-v0's model: the order-7 LaplaceDissipationFilter, or none with the moving base; a moving,
+  // the filter model, SoftPendulum3D-v0's: the order-7 LaplaceDissipationFilter, or none with the moving base; a moving,
   // clamped or free base (n >= 8: the filter's ghost records assume one reflection per end)
   const bool filter = lean && !assembly && !loads && !A.spline_mask && n >= 8 &&
                       (A.laplace_order == 7 || (A.laplace_order == 0 && bc == sr::BC_MOVING_BASE)) &&
                       (free_or_clamped || bc == sr::BC_MOVING_BASE);
-  // variants 1 / 2: one rod on the frictional plane / with rest-curvature actuation / with the travelling-wave muscle
+  // the plane / muscle models: one rod on the frictional plane / with rest-curvature actuation / with the
+  // travelling-wave muscle
   const bool contact = lean && !assembly && loads && !A.spline_mask && A.laplace_order == 0 && free_or_clamped;
   if constexpr (F64) {
     if (h->cfg.math != SR_MATH_FAST) return {launch_faithful};
     if (A.elem_tab) return {h->n_rod * (n + 1) + (A.has_head ? 1 : 0) <= 384 ? launch_tapered<384> : launch_tapered<1024>};
-    // rods of 1024-4095 elements, and filter rods of 768-1023, whose one-CTA variant would not fit its shared memory
+    // rods of 1024-4095 elements, and filter rods of 768-1023, whose CTA layout would not fit its shared memory
     if (n >= 1024 || (n >= 768 && filter) || (sw.cluster && n >= 512 && (plain || filter || contact)))
-      return cluster_kernel(lean_cluster_variant(A.laplace_order, bc, loads, A.muscle_on));
-    // variant 3: assemblies (OctoFlat: arms + rigid head + FixedJoint2Rigid joints on the plane)
+      return with_cluster_model(lean_cluster_model(A.laplace_order, bc, loads, A.muscle_on),
+                                [](auto m) { return StepKernel<T>{launch_cluster<decltype(m)::value>, 0, true}; });
+    // the assembly model (OctoFlat: arms + rigid head + FixedJoint2Rigid joints on the plane)
     if (lean && assembly && !A.spline_mask && !A.muscle_on && A.laplace_order == 0 && bc == sr::BC_FREE && A.rot_on == 0)
-      return {launch_lean<T, 3>, packed_nt, true};
-    // variant 5: SoftArmTracking-v0's spline muscle torques; the safe kernel alone, as it updates the forcing's cached
-    // control values and magnitudes inside the launch
+      return {launch_lean<T, LeanModel::ASSEMBLY, LeanLayout::CTA>, packed_nt, true};
+    // the spline model, SoftArmTracking-v0's spline muscle torques; the safe kernel alone, as it updates the forcing's
+    // cached control values and magnitudes inside the launch
     if (lean && A.spline_mask && !assembly && !loads && A.laplace_order == 0 && free_or_clamped)
-      return {launch_lean<T, 5>, lean_nt, false};
-    if (filter) return {launch_lean<T, 4>, lean_nt, true};
-    // variants 6 / 7: a rod of exactly 512 elements in 512 threads, the tip node folded into the last one (128
-    // registers), instead of 513 threads in a 544-thread CTA (96 registers)
+      return {launch_lean<T, LeanModel::SPLINE, LeanLayout::CTA>, lean_nt, false};
+    if (filter) return {launch_lean<T, LeanModel::FILTER, LeanLayout::CTA>, lean_nt, true};
+    // the plain / plane model in the fold layout: a rod of exactly 512 elements in 512 threads, the tip node folded
+    // into the last one (128 registers), instead of 513 threads in a 544-thread CTA (96 registers)
     if (sw.fold && n == 512 && A.model == sr::MODEL_ROD && !A.muscle_on && (contact || plain))
-      return {contact ? launch_lean<T, 7> : launch_lean<T, 6>, 512, true};
-    if (contact) return {A.muscle_on ? launch_lean<T, 2> : launch_lean<T, 1>, lean_nt, true};
+      return {contact ? launch_lean<T, LeanModel::PLANE, LeanLayout::FOLD> : launch_lean<T, LeanModel::PLAIN, LeanLayout::FOLD>,
+              512, true};
+    if (contact)
+      return {A.muscle_on ? launch_lean<T, LeanModel::MUSCLE, LeanLayout::CTA> : launch_lean<T, LeanModel::PLANE, LeanLayout::CTA>,
+              lean_nt, true};
   }
   if (plain) {
-    // Its fast-only kernel may be the planar variant 8 when the model keeps the out-of-plane components exact zeros
+    // Its fast-only kernel may be the planar model's when the model keeps the out-of-plane components exact zeros
     // once the state has them: FP64, gravity in the x-y plane, the base point force along x (the only direction the
     // kernel applies it in), and a BC that pins in-plane rows (slider, clamp) or none.  The kernel checks the state
     // itself, per rod, and hands the rods that are not planar over to the safe kernel.
     const bool planar = F64 && sw.planar && lean_nt <= 512 && (double)A.gdt_cv[2] == 0.0 &&
                         (free_or_clamped || bc == sr::BC_PENDULUM_SLIDER);
-    return {launch_lean<T, 0>, lean_nt, true, planar};
+    return {launch_lean<T, LeanModel::PLAIN, LeanLayout::CTA>, lean_nt, true, planar};
   }
   // The generic kernel: FP32 storage of the other models, suckers, external loads, the base point force with other
   // forcings, filter orders other than 7.  The single rod on the plane (OctoArmSingle's model) takes the lean CTA-size
@@ -611,8 +621,8 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   if (cfg->n_env <= 0 || cfg->n_elem < 3) return fail(SR_E_INVALID, "sr_create: n_env > 0 and n_elem >= 3 required");
   if (cfg->n_elem > 4095)
     return fail(SR_E_INVALID, "sr_create: n_elem <= 4095 (rods of 1024-4095 elements span a thread-block cluster of up to 8 CTAs)");
-  // rods of 1024-4095 elements: variant 0's model (cluster variant 9), SoftPendulum3D-v0's (10), or the rod on the
-  // frictional plane with rest-curvature actuation and / or the travelling-wave muscle (11 / 12)
+  // rods of 1024-4095 elements, on clusters: the plain model, SoftPendulum3D-v0's (filter), or the rod on the frictional
+  // plane with rest-curvature actuation and / or the travelling-wave muscle (plane / muscle)
   const bool loads = cfg->contact_on || cfg->muscle_on;
   const bool long_rod_model =
       ((cfg->model == SR_MODEL_ROD || cfg->model == SR_MODEL_SOFT_PENDULUM) &&
@@ -736,7 +746,8 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   SR_CUDA(cudaSetDevice(cfg->device));
   if (cfg->n_elem > 1023) {
     const int C = lean_cluster_size(cfg->n_elem);
-    const int n_active = cluster_max_active(lean_cluster_variant(cfg->laplace_filter_order, cfg->bc_kind, loads, cfg->muscle_on), C);
+    const int n_active = with_cluster_model(lean_cluster_model(cfg->laplace_filter_order, cfg->bc_kind, loads, cfg->muscle_on),
+                                            [&](auto m) { return sr::lean_cluster_max_active<decltype(m)::value>(C); });
     if (n_active < 1)
       return fail(SR_E_CUDA, "sr_create: n_elem = " + std::to_string(cfg->n_elem) + " needs a cluster of " + std::to_string(C) +
                                  " CTAs of 512 threads, and this device cannot launch one");
@@ -1134,7 +1145,8 @@ int sr_spline_basis(int32_t P, double base_length, double *out) {
 int sr_get_rest_kappa(sr_handle *h, void **rest_kappa_dev) {
   if (!h || !rest_kappa_dev) return fail(SR_E_INVALID, "sr_get_rest_kappa: null argument");
   if (h->cfg.math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for SR_MATH_FAST only");
-  // (above 1023 elements only the rods on the plane / with the muscle wave step on a kernel that reads it: variants 11 / 12)
+  // (above 1023 elements only the rods on the plane / with the muscle wave step on a kernel that reads it: the plane
+  // and muscle models on clusters)
   if (h->cfg.n_elem > 1023 && !h->cfg.contact_on && !h->cfg.muscle_on)
     return fail(SR_E_INVALID, "sr_get_rest_kappa: rest curvature is built for n_elem <= 1023, and above for rods with "
                               "contact_on or muscle_on");

@@ -287,7 +287,7 @@ int64_t sr_fallback_count(const sr_handle *h);
  * out[0] rotation per kinematic update > 0.1 rad, out[1] bend between neighbouring elements beyond the log map's
  * polynomial range, out[2] stretch beyond the rotational damper's polynomial range. */
 int sr_fallback_causes(const sr_handle *h, int64_t out[3]);
-/* Env-steps the planar variant of the lean kernel (a rod in the x-y plane, FP64) handed to the 3D safe kernel because
+/* Env-steps the planar model of the lean kernel (a rod in the x-y plane, FP64) handed to the 3D safe kernel because
  * the rod's state was not planar (out-of-plane components not exactly zero).  Not range failures: sr_fallback_count
  * does not include them.  Synchronises the handle's device. */
 int64_t sr_nonplanar_count(const sr_handle *h);

@@ -1,10 +1,11 @@
-"""Long rods on thread-block clusters (variants 9-12 of rod_kernel_lean.cuh): device time per launch of K = 100 substeps.
+"""Long rods on thread-block clusters (the cluster layout of rod_kernel_lean.cuh): device time per launch of K = 100
+substeps.
 
-Clamped rods (BASELINE config 3's model, variant 9), or with --model pendulum3d SoftPendulum3D-v0's rod (Laplace filter
-and moving base, variant 10; base held still, 608 FLOP per element-substep), with --model contact a free rod resting on
-a +z frictional plane with rest curvature, forcing first (OctoArmSingle's plane and friction, variant 11: 720 FLOP per
-element-substep), with --model snake the same on a +y plane with the travelling-wave muscle (variant 12: 840), with
-enough envs that the state block exceeds the 126 MB L2 (>= 256 MB).
+Clamped rods (BASELINE config 3's model, the plain model), or with --model pendulum3d SoftPendulum3D-v0's rod (the
+filter model: Laplace filter and moving base, base held still, 608 FLOP per element-substep), with --model contact a
+free rod resting on a +z frictional plane with rest curvature, forcing first (OctoArmSingle's plane and friction, the
+plane model: 720 FLOP per element-substep), with --model snake the same on a +y plane with the travelling-wave muscle
+(the muscle model: 840), with enough envs that the state block exceeds the 126 MB L2 (>= 256 MB).
 Cases: n = 600 and 1023 (SoftPendulum3D: 600 and 767, whose one-CTA kernel ends at 768 threads; 1023 on the cluster
 kernel alone) on the one-CTA kernel (768 / 1024 threads) and on the forced cluster kernel (C = 2), which
 run as alternating subprocesses (SOFTROD_LEAN_CLUSTER is read once per process), two rounds each; n = 1024, 2047 and
@@ -150,7 +151,7 @@ def main():
                     f"{100.0 * (sm - nc * c) / sm:.1f} % idle)")
     if a.model in ("rod", "contact", "snake"):
         cases = [(600, 0), (600, 1), (1023, 0), (1023, 1)] * 2 + [(1024, 1), (2047, 1), (4095, 1)]
-    else:    # (variant 4's largest CTA is 768 threads: from 768 elements on the cluster variant is the only one)
+    else:    # (the filter model's largest CTA is 768 threads: from 768 elements on the cluster layout is the only one)
         cases = [(600, 0), (600, 1), (767, 0), (767, 1)] * 2 + [(1023, 1), (1024, 1), (2047, 1), (4095, 1)]
     for n, cl in cases:
         env = dict(os.environ)

@@ -31,5 +31,15 @@ for line in out.splitlines():
         rows[cur] = (m.group(1),) + spill
         cur = None
 names = subprocess.run(["c++filt"], input="\n".join(rows), stdout=subprocess.PIPE, text=True).stdout.splitlines()
-for name, (regs, stack, st, ld) in sorted(zip((re.sub(r"\(.*", "", n).replace("void sr::", "") for n in names), rows.values())):
+MODELS = ["PLAIN", "PLANE", "MUSCLE", "ASSEMBLY", "FILTER", "SPLINE", "PLANAR"]   # LeanModel / LeanLayout (csrc/launch.cuh),
+LAYOUTS = ["CTA", "FOLD", "CLUSTER"]                                            # in their order
+
+
+def short(n):   # "void sr::k<..., (sr::LeanModel)2, (sr::LeanLayout)2>(args)" -> "k<..., MUSCLE, CLUSTER>"
+    n = re.sub(r"\(sr::LeanModel\)(\d+)", lambda m: MODELS[int(m.group(1))], n)
+    n = re.sub(r"\(sr::LeanLayout\)(\d+)", lambda m: LAYOUTS[int(m.group(1))], n)
+    return re.sub(r"\(.*", "", n).replace("void sr::", "")
+
+
+for name, (regs, stack, st, ld) in sorted(zip(map(short, names), rows.values())):
     print(f"{name:55s} regs={regs:>3s} stack={stack:>5s} spill_st={st:>5s} spill_ld={ld:>5s}")

@@ -1,10 +1,11 @@
-"""Rods of 512-4095 elements on thread-block clusters (variant 9 of rod_kernel_lean.cuh, DESIGN.md §4.2).
+"""Rods of 512-4095 elements on thread-block clusters (the plain model in the cluster layout of rod_kernel_lean.cuh,
+DESIGN.md §4.2).
 
-One rod spans C = ceil((n + 1) / 512) CTAs of a cluster, and the substep is variant 0's: the cluster kernel must give the
-bits of the one-CTA kernels where both exist (SOFTROD_LEAN_CLUSTER=1 forces it for 512-1023 elements), and match the C
-oracle above 1023 elements, where it is the only kernel.
+One rod spans C = ceil((n + 1) / 512) CTAs of a cluster, and the substep is the plain model's: the cluster kernel must
+give the bits of the one-CTA kernels where both exist (SOFTROD_LEAN_CLUSTER=1 forces it for 512-1023 elements), and
+match the C oracle above 1023 elements, where it is the only kernel.
 
-CPU: sr_create admits 1024-4095 elements for variant 0's model only, with a message naming what is built; the C oracle
+CPU: sr_create admits 1024-4095 elements for the plain model only, with a message naming what is built; the C oracle
 steps such rods.
 GPU: each kernel setting runs in a subprocess of its own (the settings are read once per process), and the saved
 outputs are compared: the forced cluster kernel against the default kernels, the default (cluster) pair against the
@@ -320,10 +321,10 @@ def test_cluster_kernel_gives_the_bits_of_the_one_cta_kernels(worker, n):
     orientations under gravity with three non-zero components, the damper on or off, and SoftPendulum-v0's model with
     random +-22 actions; 7 envs and 300 envs.  After each of two launches (400 and 600 substeps) the whole state
     block (all 32 fields; a digest per env for the 300-env batches), the observations, rewards and terminated flags
-    are equal bit for bit, with no range fallback.  At n = 512 the reference is variant 0's 544-thread kernel
-    (SOFTROD_LEAN_FOLD=0); the folded-tip kernel must give the same bits outside the padding slots into which variant 0
-    writes the tip thread's pseudo-element observables (tangent, sigma and dilatation slot n, kappa slot n - 1), and
-    which the folded kernel leaves alone."""
+    are equal bit for bit, with no range fallback.  At n = 512 the reference is the plain model's 544-thread
+    kernel (SOFTROD_LEAN_FOLD=0); the fold layout's kernel must give the same bits outside the padding slots into which
+    the CTA layout writes the tip thread's pseudo-element observables (tangent, sigma and dilatation slot n, kappa
+    slot n - 1), and which the folded kernel leaves alone."""
     ref, cl = worker("nofold" if n == 512 else "default"), worker("cluster")
     for model in [f"bc{bc}" for bc in LONG_BCS] + ["pendulum"]:
         for size, _ in EQ_BATCHES:

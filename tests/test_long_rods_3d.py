@@ -1,14 +1,14 @@
-"""SoftPendulum3D-v0 rods of 512-4095 elements on thread-block clusters (variant 10 of rod_kernel_lean.cuh, DESIGN.md
-§4.1): the order-7 Laplace filter and the moving base across CTAs.
+"""SoftPendulum3D-v0 rods of 512-4095 elements on thread-block clusters (the filter model in the cluster layout of
+rod_kernel_lean.cuh, DESIGN.md §4.1): the order-7 Laplace filter and the moving base across CTAs.
 
-Variant 10 is variant 4 (the one-CTA filter kernel) in variant 9's cluster layout: it must give variant 4's bits where
+The filter model's substep in the cluster layout must give the bits of its CTA layout (the one-CTA filter kernel) where
 both exist (512-767 elements, where SOFTROD_LEAN_CLUSTER=1 forces it), and match the C oracle from 768 elements on,
-where it is the only lean filter kernel (variant 4 would need a 1024-thread CTA, whose shared memory it overflows).
+where it is the only lean filter kernel (the CTA layout would need a 1024-thread CTA, whose shared memory it overflows).
 
 CPU: sr_create admits SoftPendulum3D-v0's model at 1024-4095 elements, and nothing else of that model; the C oracle
 steps such a rod.
 GPU: each kernel setting runs in a subprocess of its own (the settings are read once per process), and the saved
-outputs are compared: the forced cluster kernel against variant 4, the default (cluster) pair against the safe kernel
+outputs are compared: the forced cluster kernel against the CTA layout, the default (cluster) pair against the safe kernel
 alone (SOFTROD_FASTPATH=0) and the C oracle."""
 import ctypes as C
 import functools
@@ -25,7 +25,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 EQ_SIZES = (512, 513, 517, 600, 700, 767)   # 512: the tip alone in rank 1; 517: right ghosts across the boundary
 EQ_BATCHES = (("small", 7), ("big", 300))
-# C = 2 ... 8; 768-1023: the cluster variant is the default; 1024: the last rank holds only the tip node
+# C = 2 ... 8; 768-1023: the cluster layout is the default; 1024: the last rank holds only the tip node
 LONG_SIZES = (768, 1000, 1023, 1024, 1026, 1535, 2047, 2048, 4095)
 STEP_FPS = 2500                     # step_skip = int(1 / (2500 * time_step)) substeps per env-step (400 at n = 2048)
 STEPS = 2                           # env-steps (launches) per case
@@ -244,9 +244,9 @@ def worker(tmp_path_factory):
 @pytest.mark.gpu
 @pytest.mark.parametrize("n", EQ_SIZES)
 def test_cluster_filter_kernel_gives_the_bits_of_variant_4(worker, n):
-    """SOFTROD_LEAN_CLUSTER=1 (variant 10, two CTAs per rod) against the default one-CTA filter kernel (variant 4 in
-    544 / 768-thread CTAs), 7 and 300 envs, random +-1 actions with every third env's base starting next to the
-    (0.5, -0.5) corner and driven into the clip: after each of two env-steps the whole state block (all 32 fields), aux
+    """SOFTROD_LEAN_CLUSTER=1 (the filter model on clusters, two CTAs per rod) against the default one-CTA filter kernel
+    (the CTA layout, 544 / 768-thread CTAs), 7 and 300 envs, random +-1 actions with every third env's base starting next
+    to the (0.5, -0.5) corner and driven into the clip: after each of two env-steps the whole state block (all 32 fields), aux
     (base controller and tilt), the observations, rewards and terminated flags are equal bit for bit, with no range
     fallback in either."""
     ref, cl = worker("default"), worker("cluster")

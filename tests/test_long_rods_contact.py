@@ -1,12 +1,13 @@
-"""Rods on the frictional plane of 512-4095 elements on thread-block clusters (variants 11 / 12 of rod_kernel_lean.cuh,
-DESIGN.md §4.2): plane contact with anisotropic friction, per-env rest curvature and the travelling-wave muscle.
+"""Rods on the frictional plane of 512-4095 elements on thread-block clusters (the plane and muscle models in the
+cluster layout of rod_kernel_lean.cuh, DESIGN.md §4.2): plane contact with anisotropic friction, per-env rest curvature
+and the travelling-wave muscle.
 
-One rod spans C = ceil((n + 1) / 512) CTAs of a cluster, and the substep is variant 1's / 2's: the cluster kernel must
-give the bits of the one-CTA kernels where both exist (SOFTROD_LEAN_CLUSTER=1 forces it for 512-1023 elements), and
-match the C oracle above 1023 elements, where it is the only kernel.
+One rod spans C = ceil((n + 1) / 512) CTAs of a cluster, and the substep is the plane / muscle model's: the cluster
+kernel must give the bits of the one-CTA kernels where both exist (SOFTROD_LEAN_CLUSTER=1 forces it for 512-1023
+elements), and match the C oracle above 1023 elements, where it is the only kernel.
 
 CPU: sr_create admits 1024-4095 elements for the rod on the plane and / or with the muscle wave, and rejects that model
-combined with anything the cluster variants do not build; the C oracle steps such rods.
+combined with anything the cluster layout does not build; the C oracle steps such rods.
 GPU: each kernel setting runs in a subprocess of its own (the settings are read once per process), and the saved
 outputs are compared, as in test_long_rods.py."""
 import ctypes as C
@@ -35,7 +36,7 @@ LONG_ENVS = 2
 REACH_N, REACH_FROM = 2047, 1024               # rest curvature only on the Voronoi points of ranks 2 and 3
 KINK_N, KINK_ENVS, KINK_DEEP, KINK_EDGE = 2047, 5, 1, 3
 KINK_AT = {KINK_DEEP: 1200, KINK_EDGE: 512}    # first element turned: inside rank 2 / rank 1's first (Voronoi 511)
-KINK_DEG = 60.0     # past the contact variants' 37-degree bend map for all 12 substeps
+KINK_DEG = 60.0     # past the plane models' 37-degree bend map for all 12 substeps
 KINK_LAUNCHES = (3, 3, 3, 3)                   # (the pair stays on: the fallback counters are first polled at step 8)
 R0 = 0.004
 TILTED = (0.3, -0.2, 1.0)
@@ -422,10 +423,10 @@ def _vs_oracle(res, key, name, n, envs, launches, rng_seed, lo=0, kinked=False):
 @pytest.mark.gpu
 @pytest.mark.parametrize("n", EQ_SIZES)
 def test_cluster_contact_kernel_gives_the_bits_of_the_one_cta_kernels(worker, n):
-    """SOFTROD_LEAN_CLUSTER=1 (two CTAs per rod, variants 11 / 12) against the default kernels (variants 1 / 2 in 544 /
-    768 / 1024-thread CTAs; at n = 512 the reference is variant 1's 544-thread kernel, SOFTROD_LEAN_FOLD=0, since the
-    folded-tip variant 7 differs in the padding slots; variant 2 has no folded form): a free rod on a +z plane,
-    contact first; a clamped rod on a tilted plane under a gravity that drags it sideways, forcing first; a free rod on
+    """SOFTROD_LEAN_CLUSTER=1 (two CTAs per rod, the plane / muscle model on clusters) against the default kernels (the
+    CTA layout in 544 / 768 / 1024-thread CTAs; at n = 512 the reference is the plane model's 544-thread kernel,
+    SOFTROD_LEAN_FOLD=0, since its fold layout differs in the padding slots; the muscle model has no fold layout): a free rod on a +z
+    plane, contact first; a clamped rod on a tilted plane under a gravity that drags it sideways, forcing first; a free rod on
     a +y plane with the travelling-wave muscle (random beta(s) and wave number), forcing first; a fresh random rest
     curvature before every launch; 7 envs and 300 envs.  After each of two launches (400 and 600 substeps) the whole
     state block (a digest per env for the 300-env batches), the observations, rewards and terminated flags are equal

@@ -299,7 +299,7 @@ def _tilted_init(n_env, seed=42, max_deg=5.0):
 
 @pytest.mark.parametrize("n_elem,dt,radius", [(100, 5e-5, 0.025), (20, 1e-4, 0.05), (63, 5e-5, 0.03), (200, 2e-5, 0.025),
                                               (3, 1e-4, 0.05), (4, 1e-4, 0.05), (255, 1e-5, 0.01), (1023, 2e-6, 0.004),
-                                              (512, 5e-6, 0.008)])     # 512: the folded-tip variant of the lean kernel
+                                              (512, 5e-6, 0.008)])     # 512: the lean kernel's fold layout
 def test_generic_rod_vs_oracle(n_elem, dt, radius):
     """BASELINE config 3 family: clamped rod (OneEndFixedBC) + gravity + analytical damping, no action."""
     import rod_oracle as ro
@@ -1443,7 +1443,7 @@ def test_tapered_muscle_octopus_topology_vs_c_oracle():
 def test_two_handles_on_two_devices_agree():
     """The opt-in above 48 KB of dynamic shared memory is a per-device attribute of a kernel (cudaFuncSetAttribute):
     a second handle on another device of the same process has to set it again (round-1 advisory).  Two SoftPendulum
-    handles (lean kernel, split schedule: 600 envs > resident slots) and two contact handles (lean contact variant) on
+    handles (lean kernel, split schedule: 600 envs > resident slots) and two contact handles (lean plane model) on
     cuda:0 and cuda:1 are stepped through host buffers, interleaved, and must agree bit for bit."""
     import torch
     if torch.cuda.device_count() < 2:
@@ -1649,7 +1649,7 @@ def test_rod_on_a_tilted_frictional_plane_vs_c_oracle(normal):
 
 @pytest.mark.parametrize("seed", range(6))
 def test_randomized_contact_rods_vs_c_oracle(seed):
-    """The lean kernel's contact variant over its whole configuration space, drawn per seed: rod size (12..160 elements:
+    """The lean kernel's plane model over its whole configuration space, drawn per seed: rod size (12..160 elements:
     different CTA shapes and rods per CTA), material, plane orientation (arbitrary normal), free or clamped base, rest
     curvature about both bending axes and twist, friction coefficients, slip tolerance, contact spring and damping, the
     order of contact vs forcing, gravity pressing the rod onto the plane at an angle, and an initial slide.  CUDA vs the C
@@ -1705,7 +1705,7 @@ def test_randomized_contact_rods_vs_c_oracle(seed):
 
 @pytest.mark.parametrize("n_elem,bc,damp_first", [(8, 1, False), (9, 0, True), (13, 1, True), (20, 0, False), (63, 1, False), (100, 1, True), (160, 0, False)])
 def test_filtered_rods_vs_c_oracle(n_elem, bc, damp_first):
-    """The LaplaceDissipationFilter (order 7) outside SoftPendulum3D-v0's one shape: rods of 8 (the variant's minimum: one
+    """The LaplaceDissipationFilter (order 7) outside SoftPendulum3D-v0's one shape: rods of 8 (the filter model's minimum: one
     reflection per end) to 160 elements, free or clamped, both dampen / constrain orders, swinging under gravity from a
     tilted start.  The lean kernel evaluates passes 1..6 as one 13-tap stencil on ghost-padded records; the C oracle
     runs the reference's seven passes.  Every field, after 500 and 800 substeps, 1e-9 — or 20 x the oracle's own divergence, measured

@@ -1,8 +1,8 @@
-"""The planar variant of the lean kernel (CVAR 8, rod_kernel_lean.cuh): rods that stay in the lab x-y plane are stepped
+"""The planar model of the lean kernel (rod_kernel_lean.cuh): rods that stay in the lab x-y plane are stepped
 with the out-of-plane terms left out, and must give the bits of the 3D kernels (DESIGN.md §5).
 
 CPU: the C oracle keeps every out-of-plane component exactly zero, for SoftPendulum-v0 and for every clamped, free and
-slider rod the host hands to the planar kernel (the premise of the variant); the shape table below follows the host's
+slider rod the host hands to the planar kernel (the premise of the model); the shape table below follows the host's
 CTA rule.
 GPU: each case runs in a subprocess per kernel setting — SOFTROD_LEAN_PLANAR=0 (3D kernels), the default (planar) and,
 for the range fallbacks, SOFTROD_FASTPATH=0 (safe kernel only) — and the whole state block, observations, rewards and

@@ -88,7 +88,7 @@ def test_lean_kernel_maps():
         return float(th / mp.sin(th))
     want = np.array([ref(w) for w in w2])
     assert np.abs(horner(c, w2) / want - 1.0).max() < 8e-16
-    cm, him = table("SR_COEF_BENDW_MID"), const("kMidBendW2")        # contact variants: 37 degrees, degree 13
+    cm, him = table("SR_COEF_BENDW_MID"), const("kMidBendW2")        # plane models: 37 degrees, degree 13
     assert len(cm) == 14 and abs(him - 4 * np.sin(np.deg2rad(37.0)) ** 2) < 1e-3
     w2m = np.concatenate([rng.uniform(0, him, 1500), [0.0, him, 1e-12, 1e-6]])
     assert np.abs(horner(cm, w2m) / np.array([ref(w) for w in w2m]) - 1.0).max() < 1.5e-15
