@@ -35,8 +35,8 @@ LEAN_UNITS = [
     # up to 768 threads: filter rods of >= 768 elements take the cluster layout
     ("FILTER", "CTA", ("double",), [s for s in PACKED_SIZES if s[0] <= 768]),
     ("SPLINE", "CTA", ("double",), PACKED_SIZES),
-    # the lean kernel's CTA sizes for rods of <= 511 elements (fast-only kernel)
-    ("PLANAR", "CTA", ("double",), [s for s in PACKED_SIZES if s[0] <= 512]),
+    # the lean kernel's CTA sizes for rods of <= 511 elements (fast-only kernel), and 768 threads: 15 rods of n = 50
+    ("PLANAR", "CTA", ("double",), [s for s in PACKED_SIZES if s[0] <= 512 or s[0] == 768]),
     # a rod of exactly 512 elements in 512 threads
     ("PLAIN", "FOLD", ("double",), [(512, 1)]),
     ("PLANE", "FOLD", ("double",), [(512, 1)]),

@@ -252,18 +252,22 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
   // (named barriers over the warps that hold the rod's threads; a warp holding the end of one rod and the start of
   // the next takes part in both, in rod order) instead of CTA-wide: rods then drift apart and fill each other's
   // pipeline bubbles.  Needs tpr >= 32 (a warp touches at most two rods) and <= 15 rods per CTA (barrier ids 1..15).
+  // Planar model: warps past the last rod join the last rod's barrier, so that every warp has a first barrier.
   int bar_id0 = 0, bar_cnt0 = 0, bar_id1 = 0, bar_cnt1 = 0;
   const bool rod_barriers = A.sk_rodsync && G >= 32 && rods_per_cta >= 2 && rods_per_cta <= 15;
   if (rod_barriers) {
     const int wp = tid >> 5;
     for (int rr = 0; rr < rods_per_cta; rr++) {
-      const int wa = (rr * G) >> 5, wb = (rr * G + G - 1) >> 5;
+      const int wa = (rr * G) >> 5, wb = (PLANAR && rr == rods_per_cta - 1) ? NT / 32 - 1 : (rr * G + G - 1) >> 5;
       if (wp >= wa && wp <= wb) {
         if (bar_cnt0 == 0) { bar_id0 = rr + 1; bar_cnt0 = 32 * (wb - wa + 1); }
         else { bar_id1 = rr + 1; bar_cnt1 = 32 * (wb - wa + 1); }
       }
     }
   }
+  // planar model: whether this warp holds the start of a second rod, voted once so that the compiler knows it is the same
+  // for the whole warp: the predicated second barrier then needs no WARPSYNC, and the substep loop branches uniformly
+  const bool bar_two = PLANAR && __any_sync(0xffffffffu, bar_cnt1 != 0);
   auto rod_sync = [&]() {
     if (CLUSTER) { cluster_sync(); return; }
     if (!rod_barriers) { __syncthreads(); return; }
@@ -1293,14 +1297,25 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // planar model: the substep above with the out-of-plane terms left out (see PLANAR).  Records {x0 x1 | v0 v1 | Q0 Q1 |
     // Q6 Q7} and {s0 s1 | N1}.  The pseudo-element of the tip / idle threads lies along x here instead of z (same
     // length; its stress is discarded either way), so the tip's stale observables are rebuilt in the last substep.
-    auto substep_planar = [&](auto last_tag) {
-      constexpr bool last = decltype(last_tag)::value;
+    // NAMED: the per-rod barriers (rod_barriers), chosen once outside the loop; every warp takes part in its first
+    // rod's barrier, and a warp that holds the end of one rod and the start of the next in the next rod's as well
+    auto substep_planar = [&](auto last_tag, auto named_tag) {
+      constexpr bool last = decltype(last_tag)::value, NAMED = decltype(named_tag)::value;
+      auto sync = [&]() {
+        if constexpr (NAMED) {
+          asm volatile("bar.sync %0, %1;" ::"r"(bar_id0), "r"(bar_cnt0) : "memory");
+          asm volatile("{ .reg .pred p; setp.ne.s32 p, %2, 0; @p bar.sync %0, %1; }" ::"r"(bar_id1), "r"(bar_cnt1),
+                       "r"((int)bar_two) : "memory");
+        } else {
+          __syncthreads();
+        }
+      };
       {
         double2 *o = reinterpret_cast<double2 *>(rec + LEAN_REC * tid);
         o[0] = make_double2(x[0], x[1]); o[1] = make_double2(v[0], v[1]);
         o[2] = make_double2(Q[0], Q[1]); o[3] = make_double2(Q[6], Q[7]);
       }
-      rod_sync();
+      sync();
       D dx0, dx1, dv0, dv1, dn0, dn1, Qn0, Qn1, Qn6, Qn7;
       {
         const double2 *qq = reinterpret_cast<const double2 *>(rec + LEAN_REC * t_next);
@@ -1396,7 +1411,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
         st[(F_SIGMA + 2) * stride + j] = (ST)sg2;
         st[F_DIL * stride + j] = (ST)e;
       }
-      rod_sync();
+      sync();
       D f0, f1, tq1;
       {
         const double2 l = *reinterpret_cast<const double2 *>(sn + SNR * t_prev);
@@ -1415,9 +1430,13 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // body, so that the loop carries neither the selects nor the branch
     const int s_loop_end = (s_end == K) ? K - 1 : s_end;
     if constexpr (PLANAR) {
+      auto run = [&](auto named_tag) {
 #pragma unroll 1
-      for (int s = s_begin; s < s_loop_end; s++) substep_planar(std::false_type{});
-      if (s_end == K && s_begin < K) substep_planar(std::true_type{});
+        for (int s = s_begin; s < s_loop_end; s++) substep_planar(std::false_type{}, named_tag);
+        if (s_end == K && s_begin < K) substep_planar(std::true_type{}, named_tag);
+      };
+      if (rod_barriers) run(std::true_type{});
+      else run(std::false_type{});
     } else {
 #pragma unroll 1
       for (int s = s_begin; s < s_loop_end; s++) substep(std::false_type{}, s);

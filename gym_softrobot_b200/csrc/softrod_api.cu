@@ -12,6 +12,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <new>
 #include <string>
 #include <type_traits>
@@ -69,6 +70,7 @@ struct sr_handle {
   int64_t launches = 0;
   // stream-K schedule of the lean kernel: SM count, slots the hand-over scratch and flags are allocated for
   int sk_sms = 0, sk_slots = 0; void *sk_scratch = nullptr; int *sk_flag = nullptr;
+  long long sk_slot_threads = 0;   // slots x CTA threads sk_scratch holds (LEAN_SCR_FOLD rows each)
 };
 
 namespace {
@@ -326,11 +328,11 @@ using sr::LeanLayout;
 using sr::LeanModel;
 
 // Of those sizes, the ones build.py's LEAN_UNITS compile a one-CTA lean model and layout at: the fold layout at 512
-// threads only, the planar model up to 512 and the filter model up to 768 (its 1024-thread CTA would need 243 KB of
-// shared memory).
+// threads only, the planar model up to 512 and at 768 (planar_threads_setting) and the filter model up to 768 (its
+// 1024-thread CTA would need 243 KB of shared memory).
 constexpr bool lean_built(LeanModel model, LeanLayout layout, int nt) {
   return layout == LeanLayout::FOLD ? nt == 512
-         : model == LeanModel::PLANAR ? nt <= 512
+         : model == LeanModel::PLANAR ? nt <= 512 || nt == 768
          : model == LeanModel::FILTER ? nt <= 768
                                       : true;
 }
@@ -365,6 +367,19 @@ int lean_threads_setting(int n_elem) {
   return best;
 }
 
+// CTA size of the planar model's fast-only kernel.  Its nine state doubles per thread fit the 80 registers of one
+// 768-thread CTA per SM: 24 warps, six per scheduler instead of four, to hide the substep's dependent chains.  Taken
+// wherever those 768 threads hold 2-15 rods of >= 32 threads (the per-rod barriers), even where they leave more lanes
+// idle than lean_threads_setting's CTA: measured (B200, 1000 W, 1965 MHz), n = 50 (15 x 51 = 765 / 768 lanes against
+// 10 x 51 = 510 / 512) steps 7 % faster than in 512 threads, n = 100 (7 x 101 = 707 / 768 against 505 / 512) 9 %.
+// Also measured faster at n = 95, 160 (the most idle lanes relative to 512), 255 and 256; the other lengths of 48-383
+// elements are not measured and follow these six (DESIGN.md §4.1).
+// Otherwise that CTA, which the 3D pair and the safe fallback use in any case.
+int planar_threads_setting(int n_elem) {
+  const int tpr = n_elem + 1, rods = 768 / tpr;
+  return tpr >= 32 && rods >= 2 && rods <= 15 ? 768 : lean_threads_setting(n_elem);
+}
+
 // CTAs of the cluster that holds one rod of n elements in the cluster layout: n + 1 threads of 512 per CTA
 int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
 
@@ -394,6 +409,7 @@ template <typename T> struct StepKernel {
   int nt;        // CTA size of the one-CTA lean kernels and the generic kernel
   bool pair;     // fast-only kernel + fallback (run_pair)
   bool planar;   // plain model, CTA layout: the fast-only kernel is the planar model's while the handle's planar window allows
+  int planar_nt;  // CTA size of that planar kernel (planar_threads_setting)
 };
 
 template <typename T, int NT, int MINB, bool LAPLACE, bool MOVING, bool CONTACT, bool MULTI, bool TORQUE = false,
@@ -430,13 +446,16 @@ int launch_lean_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
     h->sk_sms = prop.multiProcessorCount;
   }
   const int slots = h->sk_sms * ctas_per_sm;
-  if (slots > h->sk_slots) {
+  // (the kernels of a handle may differ in CTA size too: the planar one's 768 threads against the 3D pair's 512)
+  if (slots > h->sk_slots || (long long)slots * NT > h->sk_slot_threads) {
+    const int n_slots = std::max(slots, h->sk_slots);
+    const long long n_threads = std::max((long long)slots * NT, h->sk_slot_threads);
     cudaFree(h->sk_scratch); cudaFree(h->sk_flag);
-    h->sk_scratch = nullptr; h->sk_flag = nullptr; h->sk_slots = 0;
-    SR_CUDA(cudaMalloc(&h->sk_scratch, (size_t)slots * sr::LEAN_SCR_FOLD * NT * sizeof(double)));
-    SR_CUDA(cudaMalloc(&h->sk_flag, (size_t)slots * sizeof(int)));
-    SR_CUDA(cudaMemset(h->sk_flag, 0, (size_t)slots * sizeof(int)));
-    h->sk_slots = slots;
+    h->sk_scratch = nullptr; h->sk_flag = nullptr; h->sk_slots = 0; h->sk_slot_threads = 0;
+    SR_CUDA(cudaMalloc(&h->sk_scratch, (size_t)n_threads * sr::LEAN_SCR_FOLD * sizeof(double)));
+    SR_CUDA(cudaMalloc(&h->sk_flag, (size_t)n_slots * sizeof(int)));
+    SR_CUDA(cudaMemset(h->sk_flag, 0, (size_t)n_slots * sizeof(int)));
+    h->sk_slots = n_slots; h->sk_slot_threads = n_threads;
   }
   A.sk_rods_per_cta = rods_per_cta; A.sk_items = items;
   A.sk_split = (!A.redo_filter && items > slots && A.n_substeps > 0) ? 1 : 0;
@@ -448,7 +467,18 @@ int launch_lean_impl(sr_handle *h, sr::RodArgs<T> &A, cudaStream_t s) {
   return SR_OK;
 }
 
-// the lean kernel (rod_kernel_lean.cuh) of one model in the CTA or fold layout, in CTAs of k.nt threads
+// the planar model's fast-only kernel (FP64) in CTAs of nt threads
+template <typename T> int launch_planar(sr_handle *h, sr::RodArgs<T> &A, int nt, cudaStream_t s) {
+  return with_cta(nt, [&](auto cta) {
+    using C = decltype(cta);
+    if constexpr (!std::is_same<T, double>::value || !lean_built(LeanModel::PLANAR, LeanLayout::CTA, C::NT))
+      return fail(SR_E_INVALID, "rod_lean_kernel: the planar model is not built for this type or " + std::to_string(C::NT) + " threads");
+    else return launch_lean_impl<T, C::NT, C::MINB, true, LeanModel::PLANAR, LeanLayout::CTA>(h, A, s);
+  });
+}
+
+// the lean kernel (rod_kernel_lean.cuh) of one model in the CTA or fold layout, in CTAs of k.nt threads (the planar
+// fast-only kernel in CTAs of k.planar_nt)
 template <typename T, LeanModel MODEL, LeanLayout LAYOUT> int launch_lean(sr_handle *h, sr::RodArgs<T> &A, const StepKernel<T> &k, cudaStream_t s) {
   return with_cta(k.nt, [&](auto cta) {
     using C = decltype(cta);
@@ -460,12 +490,10 @@ template <typename T, LeanModel MODEL, LeanLayout LAYOUT> int launch_lean(sr_han
     } else {
       return run_pair(h, A, k.pair, s, [&](auto fast) {
         constexpr bool FAST = decltype(fast)::value;
-        if constexpr (FAST && MODEL == LeanModel::PLAIN && LAYOUT == LeanLayout::CTA && std::is_same<T, double>::value &&
-                      lean_built(LeanModel::PLANAR, LeanLayout::CTA, C::NT)) {
+        if constexpr (FAST && MODEL == LeanModel::PLAIN && LAYOUT == LeanLayout::CTA && std::is_same<T, double>::value) {
           // when more than 1 % of a window's env-steps were handed over for not being planar, the handle steps with
           // the 3D pair for the next 512 steps (use_fast_pair)
-          if (k.planar && h->pair_steps >= h->planar_off_until)
-            return launch_lean_impl<T, C::NT, C::MINB, true, LeanModel::PLANAR, LeanLayout::CTA>(h, A, s);
+          if (k.planar && h->pair_steps >= h->planar_off_until) return launch_planar(h, A, k.planar_nt, s);
         }
         return launch_lean_impl<T, C::NT, C::MINB, FAST, MODEL, LAYOUT>(h, A, s);
       });
@@ -588,7 +616,7 @@ template <typename T> StepKernel<T> classify(const sr_handle *h, const sr::RodAr
     // itself, per rod, and hands the rods that are not planar over to the safe kernel.
     const bool planar = F64 && sw.planar && lean_nt <= 512 && (double)A.gdt_cv[2] == 0.0 &&
                         (free_or_clamped || bc == sr::BC_PENDULUM_SLIDER);
-    return {launch_lean<T, LeanModel::PLAIN, LeanLayout::CTA>, lean_nt, true, planar};
+    return {launch_lean<T, LeanModel::PLAIN, LeanLayout::CTA>, lean_nt, true, planar, planar_threads_setting(n)};
   }
   // The generic kernel: FP32 storage of the other models, suckers, external loads, the base point force with other
   // forcings, filter orders other than 7.  The single rod on the plane (OctoArmSingle's model) takes the lean CTA-size
