@@ -45,6 +45,7 @@ LEAN_UNITS = [
     ("FILTER", "CLUSTER", ("double",), [(512, 1)]),
     ("PLANE", "CLUSTER", ("double",), [(512, 1)]),
     ("MUSCLE", "CLUSTER", ("double",), [(512, 1)]),
+    ("SPLINE", "CLUSTER", ("double",), [(512, 1)]),
 ]
 
 

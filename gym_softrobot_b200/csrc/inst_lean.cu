@@ -43,12 +43,16 @@ template <typename T, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayo
 constexpr LeanModel TU_MODEL = LeanModel::SR_TU_MODEL;
 constexpr LeanLayout TU_LAYOUT = LeanLayout::SR_TU_LAYOUT;
 
-// The preprocessor cannot compare the names SR_TU_MODEL and SR_TU_LAYOUT stand for, so its two tests paste a name onto
+// The preprocessor cannot compare the names SR_TU_MODEL and SR_TU_LAYOUT stand for, so its tests paste a name onto
 // SR_IS_: SR_IS_CLUSTER and SR_IS_PLANAR are 1, and any other SR_IS_<name> is undefined, which #if reads as 0.
+// SR_SAFE_ONLY(<model>) is 1 for the models whose cluster layout is built as the safe kernel alone (SPLINE).
 #define SR_IS_PASTE(name) SR_IS_##name
 #define SR_IS(name) SR_IS_PASTE(name)
 #define SR_IS_CLUSTER 1
 #define SR_IS_PLANAR 1
+#define SR_SAFE_ONLY_PASTE(name) SR_SAFE_ONLY_##name
+#define SR_SAFE_ONLY(name) SR_SAFE_ONLY_PASTE(name)
+#define SR_SAFE_ONLY_SPLINE 1
 
 #if SR_IS(SR_TU_LAYOUT)   // the cluster layout
 static_assert(TU_LAYOUT == LeanLayout::CLUSTER && SR_TU_NT == LEAN_CLUSTER_NT, "the cluster layout is built for 512-thread CTAs");
@@ -88,12 +92,18 @@ template <bool FASTONLY> static int cluster_max_active(int cluster) {
 
 template <LeanModel MODEL> int lean_cluster_max_active(int cluster) {
   static_assert(MODEL == TU_MODEL, "one cluster model per translation unit");
+#if SR_SAFE_ONLY(SR_TU_MODEL)
+  return cluster_max_active<false>(cluster);
+#else
   const int a = cluster_max_active<true>(cluster), b = cluster_max_active<false>(cluster);
   return a < b ? a : b;
+#endif
 }
 
 template int lean_cluster_max_active<TU_MODEL>(int);
+#if !SR_SAFE_ONLY(SR_TU_MODEL)   // (the spline model updates its forcing's cache inside the launch: no fast-only kernel)
 template cudaError_t launch_lean_cluster_kernel<true, TU_MODEL>(const RodArgs<double> &, int, cudaStream_t);
+#endif
 template cudaError_t launch_lean_cluster_kernel<false, TU_MODEL>(const RodArgs<double> &, int, cudaStream_t);
 #else
 template cudaError_t launch_lean_kernel<SR_TU_T, SR_TU_NT, SR_TU_MINB, true, TU_MODEL, TU_LAYOUT>(const RodArgs<SR_TU_T> &, int, cudaStream_t);

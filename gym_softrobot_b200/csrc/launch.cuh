@@ -21,7 +21,7 @@ enum class LeanModel {
   MUSCLE,     // PLANE + the travelling-wave muscle torque (ContinuumSnake-v0)
   ASSEMBLY,   // arms + rigid head + joints on the plane (OctoFlat-v0)
   FILTER,     // the Laplace dissipation filter + moving base (SoftPendulum3D-v0)
-  SPLINE,     // spline muscle torques (SoftArmTracking-v0); safe kernel only
+  SPLINE,     // spline muscle torques (SoftArmTracking-v0); safe kernel only, in the CTA and cluster layouts
   PLANAR,     // PLAIN for a rod that stays in the lab x-y plane; fast-only kernel only
 };
 // The layout is where a rod's nodes live:
@@ -42,7 +42,8 @@ template <typename T, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayo
 // cluster layout (FP64, 512 threads): one rod per thread-block cluster of `cluster` CTAs, grid = n_env x cluster CTAs
 constexpr int LEAN_CLUSTER_NT = 512;
 template <bool FASTONLY, LeanModel MODEL> cudaError_t launch_lean_cluster_kernel(const RodArgs<double> &A, int cluster, cudaStream_t s);
-// clusters of that shape that both kernels of MODEL's pair can keep resident at once on the current device (0: none)
+// clusters of that shape that both kernels of MODEL's pair (the spline model: its safe kernel) can keep resident at once
+// on the current device (0: none)
 template <LeanModel MODEL> int lean_cluster_max_active(int cluster);
 
 // warp-per-rod kernel, faithful (libm, reference operation order) math: the parity build

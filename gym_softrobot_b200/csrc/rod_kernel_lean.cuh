@@ -173,7 +173,7 @@ __device__ __forceinline__ bool out_of_range(float x, int, float limf) { return 
 //   FOLD     (PLAIN, PLANE) the tip node folded into the last element's thread: a rod of n elements then takes n
 //            threads, not n + 1 — what lets the 512-element rod (BASELINE config 5) run in a 512-thread CTA with 128
 //            registers instead of a 544-thread one capped at 96 (17 warps put five on one scheduler).  One rod per CTA.
-//   CLUSTER  (PLAIN, FILTER, PLANE, MUSCLE) a rod of 512-4095 elements spread over a thread-block cluster of
+//   CLUSTER  (PLAIN, FILTER, PLANE, MUSCLE, SPLINE) a rod of 512-4095 elements spread over a thread-block cluster of
 //            C = ceil((n + 1) / NT) CTAs (one rod per cluster, launched with the cluster dimension set at run time):
 //            CTA rank c holds nodes / elements j = NT c + tid.  The substep is the model's, instruction for instruction.
 //            Only where the records come from changes: each exchange array has a halo record before thread 0 (the
@@ -193,6 +193,9 @@ __device__ __forceinline__ bool out_of_range(float x, int, float limf) { return 
 //            next rank's sn halo -1; thread 0 pushes its stress record into the previous rank's sn halo NT and its
 //            stage-1 load into the previous rank's rec halo NT (words 16-17).  The contact's two barriers become
 //            cluster barriers: four per substep.  DESIGN.md §4.1 gives the slot-by-slot order.
+//            SPLINE (safe kernel only): rank 0's lead keeps the forcing's bookkeeping and stores `need` into every rank's
+//            sh_need[0] before the second barrier; the arc-length prefix sum continues a per-rank carry, the earlier
+//            ranks' length words summed in order through DSMEM by warp 0, behind one CTA barrier in substeps that re-fit.
 template <typename ST, int NT, int MINB, bool FASTONLY, LeanModel MODEL, LeanLayout LAYOUT>
 __global__ void __launch_bounds__(NT, MINB)
 rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
@@ -701,7 +704,11 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
                 need |= 1 << d;
               }
             }
-            sh_need[r] = need;
+            if constexpr (CLUSTER) {   // every rank reads it, also when 0: rank 0's lead stores it into each rank's sh_need[0]
+              for (int c = 0; c < c_size; c++) *cluster_smem(&sh_need[0], c) = need;
+            } else {
+              sh_need[r] = need;
+            }
             spl_settled = (need == 0);
           }
         }
@@ -963,10 +970,35 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       }
       if constexpr (SPL) {
         if (spl) {
-          const int need = active ? sh_need[r] : 0;
+          // (cluster layout: every thread reads it, the last rank's idle ones too, as all of them join the carry's barrier)
+          const int need = (CLUSTER || active) ? sh_need[r] : 0;
+          double s_k = 0.0;                                          // np.cumsum(system.lengths)[j]
+          if constexpr (CLUSTER) {
+            // l_0 + ... + l_{NT c - 1}, added left to right, is an exact intermediate of the sequential sum: warp 0 adds
+            // the earlier ranks' length words (DSMEM, written before the last barrier and rewritten only after the next
+            // substep's first) into that carry, and every thread of the rank continues it over its own rank's words.
+            // Each lane loads one word of 32 and every lane adds the 32 in order, so the chain is the reference's.
+            __shared__ double sh_carry;
+            if (need && c_rank > 0) {
+              if (tid < 32) {
+                double cs = 0.0;
+                for (int c = 0; c < c_rank; c++) {
+                  const D *w = cluster_smem(rec, c) + 15;
+                  for (int b = 0; b < NT; b += 32) {
+                    const double l = w[LEAN_REC * (b + tid)];
+#pragma unroll
+                    for (int k = 0; k < 32; k++) cs += __shfl_sync(0xffffffffu, l, k);
+                  }
+                }
+                if (tid == 0) sh_carry = cs;
+              }
+              __syncthreads();
+              s_k = sh_carry;
+            }
+          }
+          const int jl = CLUSTER ? tid : j;   // this element's index among the words this CTA holds
           if (need && elem_ok) {
-            double s_k = 0.0;                                        // np.cumsum(system.lengths)[j]
-            for (int i = 0; i <= j; i++) s_k += rec[LEAN_REC * (tid - j + i) + 15];
+            for (int i = 0; i <= jl; i++) s_k += rec[LEAN_REC * (tid - jl + i) + 15];
             const int m = min(max((int)floor(s_k * A.spline_inv_dx), 0), sP);
             const double t = s_k - (double)m / A.spline_inv_dx;
             for (int d = 0; d < 3; d++) {

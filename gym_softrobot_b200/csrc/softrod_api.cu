@@ -384,9 +384,11 @@ int planar_threads_setting(int n_elem) {
 int lean_cluster_size(int n_elem) { return (n_elem + sr::LEAN_CLUSTER_NT) / sr::LEAN_CLUSTER_NT; }
 
 // The model a rod steps with in the cluster layout: the plain model, SoftPendulum3D-v0's (the Laplace filter and the
-// moving base), or the rod on the frictional plane with rest-curvature actuation (`loads`) and the travelling-wave
-// muscle.  sr_create checks its cluster shape for rods of 1024-4095 elements, the only models it admits there.
-LeanModel lean_cluster_model(int laplace_order, int bc_kind, bool loads, bool muscle_on) {
+// moving base), the rod on the frictional plane with rest-curvature actuation (`loads`) and the travelling-wave
+// muscle, or SoftArmTracking-v0's spline torques.  sr_create checks its cluster shape for rods of 1024-4095 elements,
+// the only models it admits there.
+LeanModel lean_cluster_model(int laplace_order, int bc_kind, bool loads, bool muscle_on, bool spline) {
+  if (spline) return LeanModel::SPLINE;
   if (loads) return muscle_on ? LeanModel::MUSCLE : LeanModel::PLANE;
   return laplace_order > 0 || bc_kind == sr::BC_MOVING_BASE ? LeanModel::FILTER : LeanModel::PLAIN;
 }
@@ -399,6 +401,7 @@ template <typename F> auto with_cluster_model(LeanModel model, F &&launch) {
     case M::FILTER: return launch(std::integral_constant<M, M::FILTER>());
     case M::PLANE: return launch(std::integral_constant<M, M::PLANE>());
     case M::MUSCLE: return launch(std::integral_constant<M, M::MUSCLE>());
+    case M::SPLINE: return launch(std::integral_constant<M, M::SPLINE>());
     default: return launch(std::integral_constant<M, M::PLAIN>());   // (lean_cluster_model returns no other model)
   }
 }
@@ -507,10 +510,15 @@ template <LeanModel MODEL> int launch_cluster(sr_handle *h, sr::RodArgs<double> 
   A.sk_rods_per_cta = 1; A.sk_items = A.n_env; A.sk_split = 0;
   A.sk_scratch = nullptr; A.sk_flag = nullptr;
   return run_pair(h, A, k.pair, s, [&](auto fast) {
-    cudaError_t e = sr::launch_lean_cluster_kernel<decltype(fast)::value, MODEL>(A, C, s);
-    h->launches++;
-    if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
-    return SR_OK;
+    constexpr bool FAST = decltype(fast)::value;
+    if constexpr (FAST && MODEL == LeanModel::SPLINE) {
+      return fail(SR_E_INVALID, "rod_lean_kernel: the spline model on clusters is built as the safe kernel only");
+    } else {
+      cudaError_t e = sr::launch_lean_cluster_kernel<FAST, MODEL>(A, C, s);
+      h->launches++;
+      if (e != cudaSuccess) return cuda_fail("rod_lean_kernel (cluster) launch", e);
+      return SR_OK;
+    }
   });
 }
 
@@ -585,20 +593,21 @@ template <typename T> StepKernel<T> classify(const sr_handle *h, const sr::RodAr
   // the plane / muscle models: one rod on the frictional plane / with rest-curvature actuation / with the
   // travelling-wave muscle
   const bool contact = lean && !assembly && loads && !A.spline_mask && A.laplace_order == 0 && free_or_clamped;
+  // the spline model, SoftArmTracking-v0's spline muscle torques; the safe kernel alone, as it updates the forcing's
+  // cached control values and magnitudes inside the launch
+  const bool spline = lean && A.spline_mask && !assembly && !loads && A.laplace_order == 0 && free_or_clamped;
   if constexpr (F64) {
     if (h->cfg.math != SR_MATH_FAST) return {launch_faithful};
     if (A.elem_tab) return {h->n_rod * (n + 1) + (A.has_head ? 1 : 0) <= 384 ? launch_tapered<384> : launch_tapered<1024>};
     // rods of 1024-4095 elements, and filter rods of 768-1023, whose CTA layout would not fit its shared memory
-    if (n >= 1024 || (n >= 768 && filter) || (sw.cluster && n >= 512 && (plain || filter || contact)))
-      return with_cluster_model(lean_cluster_model(A.laplace_order, bc, loads, A.muscle_on),
-                                [](auto m) { return StepKernel<T>{launch_cluster<decltype(m)::value>, 0, true}; });
+    if (n >= 1024 || (n >= 768 && filter) || (sw.cluster && n >= 512 && (plain || filter || contact || spline)))
+      return with_cluster_model(lean_cluster_model(A.laplace_order, bc, loads, A.muscle_on, A.spline_mask != 0), [](auto m) {
+        return StepKernel<T>{launch_cluster<decltype(m)::value>, 0, decltype(m)::value != LeanModel::SPLINE};
+      });
     // the assembly model (OctoFlat: arms + rigid head + FixedJoint2Rigid joints on the plane)
     if (lean && assembly && !A.spline_mask && !A.muscle_on && A.laplace_order == 0 && bc == sr::BC_FREE && A.rot_on == 0)
       return {launch_lean<T, LeanModel::ASSEMBLY, LeanLayout::CTA>, packed_nt, true};
-    // the spline model, SoftArmTracking-v0's spline muscle torques; the safe kernel alone, as it updates the forcing's
-    // cached control values and magnitudes inside the launch
-    if (lean && A.spline_mask && !assembly && !loads && A.laplace_order == 0 && free_or_clamped)
-      return {launch_lean<T, LeanModel::SPLINE, LeanLayout::CTA>, lean_nt, false};
+    if (spline) return {launch_lean<T, LeanModel::SPLINE, LeanLayout::CTA>, lean_nt, false};
     if (filter) return {launch_lean<T, LeanModel::FILTER, LeanLayout::CTA>, lean_nt, true};
     // the plain / plane model in the fold layout: a rod of exactly 512 elements in 512 threads, the tip node folded
     // into the last one (128 registers), instead of 513 threads in a 544-thread CTA (96 registers)
@@ -649,27 +658,32 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   if (cfg->n_env <= 0 || cfg->n_elem < 3) return fail(SR_E_INVALID, "sr_create: n_env > 0 and n_elem >= 3 required");
   if (cfg->n_elem > 4095)
     return fail(SR_E_INVALID, "sr_create: n_elem <= 4095 (rods of 1024-4095 elements span a thread-block cluster of up to 8 CTAs)");
-  // rods of 1024-4095 elements, on clusters: the plain model, SoftPendulum3D-v0's (filter), or the rod on the frictional
-  // plane with rest-curvature actuation and / or the travelling-wave muscle (plane / muscle)
+  // rods of 1024-4095 elements, on clusters: the plain model, SoftPendulum3D-v0's (filter), the rod on the frictional
+  // plane with rest-curvature actuation and / or the travelling-wave muscle (plane / muscle), or SoftArmTracking-v0's
+  // spline torques (spline)
   const bool loads = cfg->contact_on || cfg->muscle_on;
+  const bool rod_free_or_clamped = cfg->model == SR_MODEL_ROD && (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED) &&
+                                   cfg->laplace_filter_order == 0 && !cfg->point_force_on_base;
   const bool long_rod_model =
-      ((cfg->model == SR_MODEL_ROD || cfg->model == SR_MODEL_SOFT_PENDULUM) &&
-       (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED || cfg->bc_kind == SR_BC_PENDULUM_SLIDER) &&
-       cfg->laplace_filter_order == 0 && !loads) ||
-      (cfg->model == SR_MODEL_SOFT_PENDULUM_3D && cfg->bc_kind == SR_BC_MOVING_BASE && cfg->laplace_filter_order == 7 &&
-       !cfg->point_force_on_base && !loads) ||
-      (cfg->model == SR_MODEL_ROD && (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED) &&
-       cfg->laplace_filter_order == 0 && !cfg->point_force_on_base && loads);
+      cfg->spline_dir_mask ? rod_free_or_clamped && !loads
+                           : ((cfg->model == SR_MODEL_ROD || cfg->model == SR_MODEL_SOFT_PENDULUM) &&
+                              (cfg->bc_kind == SR_BC_FREE || cfg->bc_kind == SR_BC_ONE_END_FIXED || cfg->bc_kind == SR_BC_PENDULUM_SLIDER) &&
+                              cfg->laplace_filter_order == 0 && !loads) ||
+                                 (cfg->model == SR_MODEL_SOFT_PENDULUM_3D && cfg->bc_kind == SR_BC_MOVING_BASE &&
+                                  cfg->laplace_filter_order == 7 && !cfg->point_force_on_base && !loads) ||
+                                 (rod_free_or_clamped && loads);
   if (cfg->n_elem > 1023 &&
       (cfg->dtype != SR_DTYPE_F64 || cfg->math != SR_MATH_FAST || !long_rod_model ||
-       cfg->spline_dir_mask || cfg->n_rod_per_env > 1 || cfg->has_head || cfg->tip_radius > 0.0 || cfg->sucker_on ||
+       cfg->n_rod_per_env > 1 || cfg->has_head || cfg->tip_radius > 0.0 || cfg->sucker_on ||
        cfg->tm_muscle_on || cfg->muscle_layers_on))
     return fail(SR_E_INVALID, "sr_create: n_elem of 1024-4095 is built for SR_DTYPE_F64, SR_MATH_FAST, SR_MODEL_ROD or "
                               "SR_MODEL_SOFT_PENDULUM, one untapered rod per env with a free, clamped or slider end, gravity, "
                               "damping and the base point force; for SR_MODEL_ROD with a free or clamped end on the frictional "
                               "plane (contact_on) and / or with the travelling-wave muscle (muscle_on), rest curvature, "
-                              "gravity and damping, without the base point force; no spline torques, suckers, transverse "
-                              "muscle, muscle layers or Laplace filter; "
+                              "gravity and damping, without the base point force; for SR_MODEL_ROD with a free or clamped end "
+                              "and spline torques (spline_dir_mask), gravity and damping, without the base point force, "
+                              "contact, the muscle wave or rest curvature; no suckers, transverse muscle, muscle layers or "
+                              "Laplace filter, and spline torques with no other model; "
                               "and for SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE and laplace_filter_order = 7, "
                               "without the base point force");
   if (cfg->n_elem > 127 && cfg->math != SR_MATH_FAST) return fail(SR_E_INVALID, "sr_create: faithful math supports n_elem <= 127");
@@ -774,7 +788,8 @@ int sr_create(const sr_config *cfg, sr_handle **out) {
   SR_CUDA(cudaSetDevice(cfg->device));
   if (cfg->n_elem > 1023) {
     const int C = lean_cluster_size(cfg->n_elem);
-    const int n_active = with_cluster_model(lean_cluster_model(cfg->laplace_filter_order, cfg->bc_kind, loads, cfg->muscle_on),
+    const int n_active = with_cluster_model(lean_cluster_model(cfg->laplace_filter_order, cfg->bc_kind, loads, cfg->muscle_on,
+                                                               cfg->spline_dir_mask != 0),
                                             [&](auto m) { return sr::lean_cluster_max_active<decltype(m)::value>(C); });
     if (n_active < 1)
       return fail(SR_E_CUDA, "sr_create: n_elem = " + std::to_string(cfg->n_elem) + " needs a cluster of " + std::to_string(C) +

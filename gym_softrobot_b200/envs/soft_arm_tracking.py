@@ -42,33 +42,66 @@ def target_trajectory(final_time, sim_dt, v_scale, rng):
     return out
 
 
-def _make_handle(n_env, device, dtype=nat.DTYPE_F64):
+def substeps_per_step(time_step):
+    """Substeps per env-step: the reference's 0.01 s of simulated time per env-step (50 at its 2e-4 s step)."""
+    return int(np.rint(0.01 / time_step))
+
+
+def truncation_steps(update, time_step, final_time=_FINAL_TIME):
+    """Env-steps after which an episode is truncated: the first k with `tick * sim_dt >= final_time`, tick = k * update
+    substeps as an integer and the product in float64, as the reference evaluates it (soft_arm_tracking.py:254)."""
+    k = max(1, int(final_time / (update * time_step)) - 1)
+    while k > 1 and (k - 1) * update * time_step >= final_time:
+        k -= 1
+    while not (k * update * time_step >= final_time):
+        k += 1
+    return k
+
+
+def spline_scale(n_elems):
+    """Spline torque magnitude per element: the reference's 10 R E at its 40 elements, times 40 / n_elems, so that the
+    torque summed over the arm does not grow with refinement (exactly the reference's value at n_elems = 40)."""
+    return 10 * _R * _E * (_N_ELEM / n_elems)
+
+
+def _make_handle(n_env, device, dtype=nat.DTYPE_F64, n_elems=_N_ELEM, time_step=_DT):
     return nat.Handle(
-        model=nat.MODEL_ROD, n_env=n_env, n_elem=_N_ELEM, dt=_DT, base_length=_L, base_radius=_R,
+        model=nat.MODEL_ROD, n_env=n_env, n_elem=n_elems, dt=time_step, base_length=_L, base_radius=_R,
         density=1000 * 1e-6, youngs_modulus=_E, damping_constant=_E * 1e-7 * 1, bc_kind=nat.BC_ONE_END_FIXED,
         damping_before_constraints=True,          # dampen() is called before constrain() (lines 300-309)
         device=device, dtype=dtype,
-        spline=dict(directions=(0, 1), n_ctrl=_N_CTRL, scale=10 * _R * _E, max_rate=float("inf")))
+        spline=dict(directions=(0, 1), n_ctrl=_N_CTRL, scale=spline_scale(n_elems), max_rate=float("inf")))
 
 
 class SoftArmTrackingVectorEnv:
-    """N independent SoftArmTracking-v0 envs (torch CUDA I/O, float64), one physics launch per env-step."""
+    """N independent SoftArmTracking-v0 envs (torch CUDA I/O, float64), one physics launch per env-step.
 
-    def __init__(self, n_env, game_mode: int = 1, device: int = 0, autoreset: bool = True):
+    `n_elems` (3-4095; 1024 and more step on thread-block clusters) and `time_step` refine the arm.  An env-step stays
+    0.01 s of simulated time, rint(0.01 / time_step) substeps, and truncation follows `tick * sim_dt >= 5`.  The spline
+    torque is applied per element, so a finer arm would feel a larger total torque: the magnitude is scaled by
+    40 / n_elems (spline_scale), 1.0 at the reference's 40 elements.  With the reference's unscaled magnitude a
+    2048-element arm diverges within its first env-step at 5e-6 s and at 2.5e-6 s; scaled, it tracks a 1024-element arm
+    at 1e-5 s to 0.02 mm at the tip after three env-steps of random targets (longer horizons not checked).  A finer arm
+    needs a smaller step: 5e-6 s at 2048 elements."""
+
+    def __init__(self, n_env, game_mode: int = 1, device: int = 0, autoreset: bool = True, n_elems: int = _N_ELEM,
+                 time_step: float = _DT):
         import torch
         self.torch = torch
         self.n_env, self.mode = n_env, game_mode
+        self.n_elems, self.time_step = n_elems, time_step
+        self.update = substeps_per_step(time_step)
         self.device = torch.device(f"cuda:{device}")
         self.autoreset = autoreset
         self.single_action_space = Box(-1.0, 1.0, shape=(2 * _N_CTRL,), dtype=np.float64)
         self.single_observation_space = Box(-np.inf, np.inf, shape=(_N_CTRL * 2 + 6,), dtype=np.float64)
-        self.handle = _make_handle(n_env, device)
+        self.handle = _make_handle(n_env, device, n_elems=n_elems, time_step=time_step)
         self._scratch = (torch.empty((n_env, 6), dtype=torch.float32, device=self.device),
                          torch.empty(n_env, dtype=torch.float64, device=self.device),
                          torch.empty(n_env, dtype=torch.uint8, device=self.device))
         self._init = np.zeros((1, 9)); self._init[0, 4] = 1.0; self._init[0, 8] = 1.0   # direction +y, normal +z
         # tick -> truncated: `self.tick * self.sim_dt >= 5` evaluated in float64 as the reference does
-        self.n_updates = int(np.argmax(np.arange(0, 40000, _UPDATE) * _DT >= _FINAL_TIME))
+        self.n_updates = truncation_steps(self.update, time_step)
         self._targets = torch.zeros((n_env, self.n_updates + 1, 3), dtype=torch.float64, device=self.device)
         self.tick = torch.zeros(n_env, dtype=torch.int64, device=self.device)      # in env-steps
         self._seq = None
@@ -83,7 +116,7 @@ class SoftArmTrackingVectorEnv:
         torch = self.torch
         f = self.handle.fields()
         kap = f["kappa"]                                     # stale, as in the reference (SURVEY A.6)
-        seg = int((_N_ELEM - 1) / _N_CTRL)
+        seg = int((self.n_elems - 1) / _N_CTRL)
         parts = []
         for c in (0, 1):
             m = [kap[:, c, seg * i:seg * (i + 1)].mean(dim=1) for i in range(_N_CTRL - 1)]
@@ -102,8 +135,8 @@ class SoftArmTrackingVectorEnv:
         rows = []
         for _ in range(len(idx)):                            # one independent stream per episode
             rng = np.random.Generator(np.random.PCG64(self._seq.spawn(1)[0]))
-            w = target_trajectory(_FINAL_TIME, _DT, 0.1, rng)
-            rows.append(w[::_UPDATE][:self.n_updates + 1])
+            w = target_trajectory(_FINAL_TIME, self.time_step, 0.1, rng)
+            rows.append(w[::self.update][:self.n_updates + 1])
         self._targets[idx] = torch.as_tensor(np.stack(rows), device=self.device)
 
     def _reset_envs(self, idx=None, seed=None, new_targets=True):
@@ -128,7 +161,7 @@ class SoftArmTrackingVectorEnv:
         pts[:, 0, :_N_CTRL] = action[:, :_N_CTRL]           # spline_points_func_array_normal_dir[:] = ...
         pts[:, 1, :_N_CTRL] = action[:, _N_CTRL:]
         obs6, rew, term = self._scratch
-        self.handle.step(None, _UPDATE, obs6, rew, term)
+        self.handle.step(None, self.update, obs6, rew, term)
         self.tick += 1
         tip = self.handle.fields()["position_collection"][:, :, -1]
         tip_to_target = (self._target_now() - tip) / 1000

@@ -68,11 +68,13 @@ typedef struct sr_config {
   int32_t math;         /* SR_MATH_* */
   int32_t n_env;        /* independent environments (one rod each) */
   int32_t n_elem;       /* elements per rod: 3-1023; 1024-4095 (one rod per thread-block cluster of up to 8 CTAs) for
-                         * SR_DTYPE_F64, SR_MATH_FAST, one untapered rod per env without spline torques, suckers or
-                         * muscle layers, and either SR_MODEL_ROD / SR_MODEL_SOFT_PENDULUM with a free, clamped or
-                         * slider end, no contact, muscle or filter; or SR_MODEL_ROD with a free or clamped end on the
+                         * SR_DTYPE_F64, SR_MATH_FAST, one untapered rod per env without suckers or muscle layers, and
+                         * either SR_MODEL_ROD / SR_MODEL_SOFT_PENDULUM with a free, clamped or slider end, no contact,
+                         * muscle, spline torques or filter; or SR_MODEL_ROD with a free or clamped end on the
                          * frictional plane (contact_on) and / or with the travelling-wave muscle (muscle_on), with
-                         * rest curvature (sr_get_rest_kappa) and no base point force or filter; or
+                         * rest curvature (sr_get_rest_kappa) and no base point force, spline torques or filter; or
+                         * SR_MODEL_ROD with a free or clamped end and spline torques (spline_dir_mask), without
+                         * contact, muscle, rest curvature, base point force or filter; or
                          * SR_MODEL_SOFT_PENDULUM_3D with SR_BC_MOVING_BASE, laplace_filter_order = 7 and no base point
                          * force */
   int32_t bc_kind;      /* SR_BC_* */
