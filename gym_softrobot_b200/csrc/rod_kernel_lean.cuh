@@ -620,7 +620,9 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     if (s_begin == 0 && K > 0) { kinematic(c_half_dt, D(1e-14)); head_constrain_values(); }
 
     bool spl_settled = false;   // spline model: the cached control values have reached their targets
-    bool check_trace = true;   // first substep of the segment: rule out a state that starts beyond 90 degrees of bend
+    // first substep of the segment: rule out a state that starts beyond 90 degrees of bend (the planar model runs that
+    // substep as a copy of its own instead)
+    bool check_trace = true;
     auto substep = [&](auto last_tag, int s_now) {
       constexpr bool last = decltype(last_tag)::value;
       D mtq[3] = {D(0), D(0), D(0)};
@@ -1330,9 +1332,13 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // Q6 Q7} and {s0 s1 | N1}.  The pseudo-element of the tip / idle threads lies along x here instead of z (same
     // length; its stress is discarded either way), so the tip's stale observables are rebuilt in the last substep.
     // NAMED: the per-rod barriers (rod_barriers), chosen once outside the loop; every warp takes part in its first
-    // rod's barrier, and a warp that holds the end of one rod and the start of the next in the next rod's as well
-    auto substep_planar = [&](auto last_tag, auto named_tag) {
+    // rod's barrier, and a warp that holds the end of one rod and the start of the next in the next rod's as well.
+    // FIRST: the segment's first substep, the only one that runs the trace check.  It is a copy of its own so that the
+    // check's reads of the pre-launch state (st, bc, stride, j) are not live across the loop: at the 80-register cap
+    // they made ptxas re-derive the thread's indices and addresses in every substep.
+    auto substep_planar = [&](auto last_tag, auto named_tag, auto first_tag) {
       constexpr bool last = decltype(last_tag)::value, NAMED = decltype(named_tag)::value;
+      constexpr bool FIRST = decltype(first_tag)::value;
       auto sync = [&]() {
         if constexpr (NAMED) {
           asm volatile("bar.sync %0, %1;" ::"r"(bar_id0), "r"(bar_cnt0) : "memory");
@@ -1379,8 +1385,7 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
       D w2 = vec1 * vec1;
       if (!vor_ok) w2 = D(0);
       bool bend_out = out_of_range(w2, A.lim_bend_hi, A.limf_bend);
-      if (check_trace) {
-        check_trace = false;
+      if constexpr (FIRST) {
         if (vor_ok) {
           // d2 = (0, 0, d2z) of this element and the next: invariant under in-plane rotations, read from the
           // pre-launch state (the clamp's from its anchor)
@@ -1462,10 +1467,17 @@ rod_lean_kernel(const __grid_constant__ RodArgs<ST> A) {
     // body, so that the loop carries neither the selects nor the branch
     const int s_loop_end = (s_end == K) ? K - 1 : s_end;
     if constexpr (PLANAR) {
+      using yes = std::true_type;
+      using no = std::false_type;
       auto run = [&](auto named_tag) {
+        if (s_begin < s_loop_end) {
+          substep_planar(no{}, named_tag, yes{});
 #pragma unroll 1
-        for (int s = s_begin; s < s_loop_end; s++) substep_planar(std::false_type{}, named_tag);
-        if (s_end == K && s_begin < K) substep_planar(std::true_type{}, named_tag);
+          for (int s = s_begin + 1; s < s_loop_end; s++) substep_planar(no{}, named_tag, no{});
+          if (s_end == K) substep_planar(yes{}, named_tag, no{});
+        } else if (s_end == K && s_begin < K) {   // a segment of the item's last substep alone
+          substep_planar(yes{}, named_tag, yes{});
+        }
       };
       if (rod_barriers) run(std::true_type{});
       else run(std::false_type{});
