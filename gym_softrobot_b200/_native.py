@@ -21,7 +21,7 @@ MATH_FAST, MATH_FAITHFUL = 0, 1
 EXPORTED_SYMBOLS = [
     "sr_abi_version", "sr_last_error", "sr_create", "sr_destroy", "sr_obs_dim", "sr_action_dim",
     "sr_init_dim", "sr_reset", "sr_step", "sr_reset_host", "sr_step_host", "sr_observe",
-    "sr_get_state", "sr_set_state", "sr_copy_from", "sr_get_aux", "sr_get_head", "sr_get_rest_kappa", "sr_get_sucker", "sr_get_sucker_index", "sr_get_tm_activation", "sr_get_muscle_activation", "sr_get_fixed_suckers", "sr_get_ext_loads", "sr_get_muscle", "sr_get_spline", "sr_spline_basis", "sr_launch_count", "sr_fallback_count", "sr_fallback_causes", "sr_nonplanar_count", "sr_measure_fp64_peak", "sr_measure_fp64_peak_regs", "sr_selftest_reciprocals", "sr_probe_latency",
+    "sr_get_state", "sr_set_state", "sr_copy_from", "sr_copy_envs", "sr_get_aux", "sr_get_head", "sr_get_rest_kappa", "sr_get_sucker", "sr_get_sucker_index", "sr_get_tm_activation", "sr_get_muscle_activation", "sr_get_fixed_suckers", "sr_get_ext_loads", "sr_get_muscle", "sr_get_spline", "sr_spline_basis", "sr_launch_count", "sr_fallback_count", "sr_fallback_causes", "sr_nonplanar_count", "sr_measure_fp64_peak", "sr_measure_fp64_peak_regs", "sr_selftest_reciprocals", "sr_probe_latency",
 ]
 
 
@@ -100,6 +100,7 @@ def load_library():
     L.sr_get_state.argtypes = [C.c_void_p, C.POINTER(SrStateView)]
     L.sr_set_state.argtypes = [C.c_void_p, C.POINTER(SrStateView), C.c_void_p]
     L.sr_copy_from.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.sr_copy_envs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
     L.sr_get_aux.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int32)]
     L.sr_get_head.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int32)]
     L.sr_get_rest_kappa.argtypes = [C.c_void_p, C.POINTER(C.c_void_p)]
@@ -141,6 +142,35 @@ class _DevMem:
             "shape": tuple(shape), "typestr": typestr, "data": (int(ptr), False), "version": 2,
             "strides": None,
         }
+
+
+def copy_env_indices(dst_idx, src_idx, n_dst, n_src):
+    """The index pairs of a copy_envs call as two int64 NumPy arrays, checked: ints, sequences, NumPy arrays or torch
+    tensors (a CUDA tensor costs one device sync) of integers, equal lengths, every destination in [0, n_dst) and
+    every source in [0, n_src), no destination twice.  Raises ValueError otherwise."""
+    def as_index(x, what):
+        if hasattr(x, "detach"):
+            x = x.detach().cpu().numpy()
+        a = np.asarray(x)
+        if a.ndim == 0:
+            a = a.reshape(1)
+        if a.ndim != 1:
+            raise ValueError(f"{what} must be one-dimensional, got shape {a.shape}")
+        if a.size == 0:
+            return a.astype(np.int64)
+        if a.dtype == np.bool_ or not np.issubdtype(a.dtype, np.integer):
+            raise ValueError(f"{what} must hold integers, got {a.dtype}")
+        return a.astype(np.int64)
+    d, s = as_index(dst_idx, "dst_idx"), as_index(src_idx, "src_idx")
+    if d.size != s.size:
+        raise ValueError(f"dst_idx and src_idx differ in length ({d.size} and {s.size})")
+    if d.size and (d.min() < 0 or d.max() >= n_dst):
+        raise ValueError(f"dst_idx out of range [0, {n_dst})")
+    if s.size and (s.min() < 0 or s.max() >= n_src):
+        raise ValueError(f"src_idx out of range [0, {n_src})")
+    if np.unique(d).size != d.size:
+        raise ValueError("dst_idx names an env twice")
+    return d, s
 
 
 def spline_basis(n_ctrl: int, base_length: float):
@@ -476,6 +506,20 @@ class Handle:
         """Rod arrays only (sr_set_state): see clone_from for a whole-handle copy."""
         v = other.state_view()
         _check(self._lib.sr_set_state(self._h, C.byref(v), self._stream_ptr()))
+
+    def copy_envs(self, dst_idx, src_idx, src: "Handle" = None):
+        """Fork envs (sr_copy_envs): env dst_idx[i] of this handle takes everything that evolves or parametrises env
+        src_idx[i] of `src` (default: this handle), the per-env rows of what clone_from copies.  Indices: ints,
+        sequences, NumPy arrays or torch tensors, checked by copy_env_indices (ValueError).  Stream-ordered on the
+        current stream."""
+        import torch
+        src = self if src is None else src
+        d, s = copy_env_indices(dst_idx, src_idx, self.n_env, src.n_env)
+        dev = f"cuda:{self.device}"
+        dt = torch.as_tensor(d.astype(np.int32), device=dev).contiguous()
+        st = torch.as_tensor(s.astype(np.int32), device=dev).contiguous()
+        _check(self._lib.sr_copy_envs(self._h, C.c_void_p(dt.data_ptr()), src._h, C.c_void_p(st.data_ptr()),
+                                      int(d.size), self._stream_ptr()))
 
     def clone_from(self, other: "Handle"):
         """Everything that evolves or parametrises the envs (sr_copy_from): rod arrays, BC anchors, base controller,

@@ -51,7 +51,7 @@ LEAN_UNITS = [
 
 def translation_units():
     """[(object name, source, extra -D flags, header deps)]"""
-    tus = [("api", "softrod_api.cu", [], _COMMON), ("warp", "inst_warp.cu", [], _COMMON)]
+    tus = [("api", "softrod_api.cu", [], _COMMON + ["copy_kernels.cuh"]), ("warp", "inst_warp.cu", [], _COMMON)]
     for model, layout, types, sizes in LEAN_UNITS:
         for t in types:
             for nt, minb in sizes:

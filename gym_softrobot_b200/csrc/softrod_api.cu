@@ -20,6 +20,7 @@
 #include <vector>
 
 #include "../../include/softrod.h"
+#include "copy_kernels.cuh"
 #include "launch.cuh"
 #include "util_kernels.cuh"
 
@@ -71,6 +72,7 @@ struct sr_handle {
   // stream-K schedule of the lean kernel: SM count, slots the hand-over scratch and flags are allocated for
   int sk_sms = 0, sk_slots = 0; void *sk_scratch = nullptr; int *sk_flag = nullptr;
   long long sk_slot_threads = 0;   // slots x CTA threads sk_scratch holds (LEAN_SCR_FOLD rows each)
+  void *copy_stage = nullptr; size_t copy_stage_bytes = 0;   // sr_copy_envs within one handle: the source rows, gathered
 };
 
 namespace {
@@ -643,6 +645,72 @@ template <typename T> int launch_step(sr_handle *h, sr::RodArgs<T> &A, cudaStrea
   return k.launch(h, A, k, s);
 }
 
+// The per-env buffers of a handle: everything that evolves or parametrises an env, which sr_copy_from clones and
+// sr_copy_envs copies row by row.  Env e's row of a buffer is the `bytes` bytes at base + e * bytes (rod-level buffers
+// hold an env's n_rod rows back to back); base is null for a buffer the handle has not allocated.  `lazy`: allocated
+// on first use by its getter, zero until then (alloc_lazy_like).
+struct EnvBuf { void *base; size_t bytes; bool lazy; };
+enum { EB_STATE, EB_BC, EB_AUX, EB_HEAD, EB_REST_KAPPA, EB_EXT_FORCE, EB_EXT_COUPLE, EB_SUCKER, EB_SUCKER_IDX, EB_TM_ACT,
+       EB_MUS_ACT, EB_MSUCKER, EB_MUSCLE, EB_SPLINE, EB_COUNT };
+static_assert(EB_COUNT <= sr::COPY_MAX_BUFS, "sr::CopyTable holds every per-env buffer");
+void env_buffers(const sr_handle *h, EnvBuf (&b)[EB_COUNT]) {
+  const size_t nr = (size_t)h->n_rod, es = h->elem_size, rows3 = nr * 3 * h->stride * es;
+  b[EB_STATE] = {h->state, nr * sr::N_FIELDS * h->stride * es, false};
+  b[EB_BC] = {h->bc, nr * sr::BC_DIM * es, false};
+  b[EB_AUX] = {h->aux, sr::AUX_DIM * es, false};
+  b[EB_HEAD] = {h->head, sr::HEAD_DIM * es, false};
+  b[EB_REST_KAPPA] = {h->rest_kappa, rows3, true};
+  b[EB_EXT_FORCE] = {h->ext_force, rows3, true};
+  b[EB_EXT_COUPLE] = {h->ext_couple, rows3, true};
+  b[EB_SUCKER] = {h->sucker, nr * es, false};
+  b[EB_SUCKER_IDX] = {h->sucker_idx, nr * sizeof(int32_t), false};
+  b[EB_TM_ACT] = {h->tm_act, nr * es, false};
+  b[EB_MUS_ACT] = {h->mus_act, nr * 3 * (size_t)h->cfg.n_elem * sizeof(double), false};
+  b[EB_MSUCKER] = {h->msucker, nr * 3 * sizeof(double), false};
+  b[EB_MUSCLE] = {h->muscle, (size_t)h->muscle_dim * sizeof(double), false};
+  b[EB_SPLINE] = {h->spline, (size_t)h->spline_dim * sizeof(double), false};
+}
+
+// The lazily allocated buffers `src` has and `dst` has not, allocated in dst through their getters.
+int alloc_lazy_like(sr_handle *dst, const sr_handle *src) {
+  void *p = nullptr, *q = nullptr;
+  if (src->rest_kappa) {
+    const int rc = sr_get_rest_kappa(dst, &p);
+    if (rc != SR_OK) return rc;
+  }
+  if (src->ext_force) {
+    const int rc = sr_get_ext_loads(dst, &p, &q);
+    if (rc != SR_OK) return rc;
+  }
+  return SR_OK;
+}
+
+// The shapes sr_copy_from and sr_copy_envs need to agree, apart from the env count.
+bool same_env_shape(const sr_handle *a, const sr_handle *b) {
+  return a->cfg.n_elem == b->cfg.n_elem && a->n_rod == b->n_rod && a->cfg.dtype == b->cfg.dtype && a->cfg.model == b->cfg.model &&
+         a->cfg.has_head == b->cfg.has_head && a->stride == b->stride && a->muscle_dim == b->muscle_dim &&
+         a->spline_dim == b->spline_dim;
+}
+
+// The widest unit (16, 8 or 4 bytes) that divides the row size and both bases.
+int copy_vec(const void *src, const void *dst, size_t bytes) {
+  const uintptr_t m = (uintptr_t)src | (uintptr_t)dst | (uintptr_t)bytes;
+  return m % 16 == 0 ? 16 : m % 8 == 0 ? 8 : 4;
+}
+
+// One launch of copy_envs_kernel over the n pairs of the index arrays (h: the handle whose launches it counts).
+int launch_copy(sr_handle *h, sr::CopyTable &t, const int32_t *dst_idx, const int32_t *src_idx, int n, cudaStream_t s) {
+  unsigned long long units = 0;   // the largest row in units of its vector width
+  for (int k = 0; k < t.n_buf; k++) units = std::max(units, t.buf[k].bytes / t.buf[k].vec);
+  // about four units per thread of a row; pairs on grid.y (at most 65535, the kernel strides over the rest)
+  const unsigned gx = (unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>((units + 4 * sr::COPY_NT - 1) / (4 * sr::COPY_NT), 1024));
+  const dim3 grid(gx, (unsigned)std::min(n, 65535));
+  sr::copy_envs_kernel<<<grid, sr::COPY_NT, 0, s>>>(t, dst_idx, src_idx, n);
+  h->launches++;
+  const cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? SR_OK : cuda_fail("copy_envs_kernel launch", e);
+}
+
 }  // namespace
 
 extern "C" {
@@ -980,7 +1048,7 @@ void sr_destroy(sr_handle *h) {
   if (!h) return;
   cudaSetDevice(h->cfg.device);
   cudaFree(h->mus_act); cudaFree(h->msucker);
-  cudaFree(h->state); cudaFree(h->bc); cudaFree(h->aux); cudaFree(h->rest_kappa); cudaFree(h->head); cudaFree(h->muscle); cudaFree(h->spline); cudaFree(h->spline_tab); cudaFree(h->redo); cudaFree(h->redo_count); cudaFree(h->sucker); cudaFree(h->sucker_idx); cudaFree(h->tm_act); cudaFree(h->ext_force); cudaFree(h->ext_couple); cudaFree(h->elem_tab); cudaFree(h->sk_scratch); cudaFree(h->sk_flag); cudaFreeHost(h->h_redo_count); if (h->pair_event) cudaEventDestroy(h->pair_event); cudaFree(h->d_action); cudaFree(h->d_obs);
+  cudaFree(h->state); cudaFree(h->bc); cudaFree(h->aux); cudaFree(h->rest_kappa); cudaFree(h->head); cudaFree(h->muscle); cudaFree(h->spline); cudaFree(h->spline_tab); cudaFree(h->redo); cudaFree(h->redo_count); cudaFree(h->sucker); cudaFree(h->sucker_idx); cudaFree(h->tm_act); cudaFree(h->ext_force); cudaFree(h->ext_couple); cudaFree(h->elem_tab); cudaFree(h->sk_scratch); cudaFree(h->sk_flag); cudaFree(h->copy_stage); cudaFreeHost(h->h_redo_count); if (h->pair_event) cudaEventDestroy(h->pair_event); cudaFree(h->d_action); cudaFree(h->d_obs);
   cudaFree(h->d_reward); cudaFree(h->d_term); cudaFree(h->d_init); cudaFree(h->d_idx);
   cudaFreeHost(h->h_action); cudaFreeHost(h->h_obs); cudaFreeHost(h->h_reward); cudaFreeHost(h->h_term);
   cudaFreeHost(h->h_init);
@@ -1289,42 +1357,74 @@ int sr_set_state(sr_handle *h, const sr_state_view *src, void *stream) {
 int sr_copy_from(sr_handle *dst, sr_handle *src, void *stream) {
   if (!dst || !src) return fail(SR_E_INVALID, "sr_copy_from: null argument");
   const sr_config &a = dst->cfg, &b = src->cfg;
-  if (a.n_env != b.n_env || a.n_elem != b.n_elem || dst->n_rod != src->n_rod || a.dtype != b.dtype || a.model != b.model ||
-      a.has_head != b.has_head || dst->stride != src->stride || dst->muscle_dim != src->muscle_dim ||
-      dst->spline_dim != src->spline_dim)
+  if (a.n_env != b.n_env || !same_env_shape(dst, src))
     return fail(SR_E_INVALID, "sr_copy_from: the two handles were created with different shapes");
   SR_CUDA(cudaSetDevice(a.device));
   cudaStream_t s = (cudaStream_t)stream;
-  const size_t n_env = (size_t)a.n_env, n_rods = n_env * dst->n_rod, es = dst->elem_size;
-  auto cp = [&](void *d, const void *sp, size_t bytes) {
-    return (a.device == b.device) ? cudaMemcpyAsync(d, sp, bytes, cudaMemcpyDeviceToDevice, s)
-                                  : cudaMemcpyPeerAsync(d, a.device, sp, b.device, bytes, s);
-  };
-  SR_CUDA(cp(dst->state, src->state, n_rods * sr::N_FIELDS * dst->stride * es));
-  SR_CUDA(cp(dst->bc, src->bc, n_rods * sr::BC_DIM * es));
-  SR_CUDA(cp(dst->aux, src->aux, n_env * sr::AUX_DIM * es));
-  SR_CUDA(cp(dst->head, src->head, n_env * sr::HEAD_DIM * es));
-  if (src->rest_kappa) {
-    void *rk = nullptr;
-    int rc = sr_get_rest_kappa(dst, &rk);     // allocates on first use
-    if (rc != SR_OK) return rc;
-    SR_CUDA(cp(rk, src->rest_kappa, n_rods * 3 * dst->stride * es));
+  const int rc = alloc_lazy_like(dst, src);
+  if (rc != SR_OK) return rc;
+  EnvBuf d[EB_COUNT], sb[EB_COUNT];
+  env_buffers(dst, d);
+  env_buffers(src, sb);
+  for (int k = 0; k < EB_COUNT; k++) {
+    if (!d[k].base || !sb[k].base) continue;
+    const size_t bytes = (size_t)a.n_env * d[k].bytes;
+    SR_CUDA(a.device == b.device ? cudaMemcpyAsync(d[k].base, sb[k].base, bytes, cudaMemcpyDeviceToDevice, s)
+                                 : cudaMemcpyPeerAsync(d[k].base, a.device, sb[k].base, b.device, bytes, s));
   }
-  if (src->sucker && dst->sucker) SR_CUDA(cp(dst->sucker, src->sucker, n_rods * es));
-  if (src->sucker_idx && dst->sucker_idx) SR_CUDA(cp(dst->sucker_idx, src->sucker_idx, n_rods * sizeof(int32_t)));
-  if (src->tm_act && dst->tm_act) SR_CUDA(cp(dst->tm_act, src->tm_act, n_rods * es));
-  if (src->msucker && dst->msucker) SR_CUDA(cp(dst->msucker, src->msucker, n_rods * 3 * sizeof(double)));
-  if (src->mus_act && dst->mus_act) SR_CUDA(cp(dst->mus_act, src->mus_act, n_rods * 3 * (size_t)src->cfg.n_elem * sizeof(double)));
-  if (src->ext_force) {
-    void *f = nullptr, *c = nullptr;
-    int rc = sr_get_ext_loads(dst, &f, &c);
-    if (rc != SR_OK) return rc;
-    SR_CUDA(cp(f, src->ext_force, n_rods * 3 * dst->stride * es));
-    SR_CUDA(cp(c, src->ext_couple, n_rods * 3 * dst->stride * es));
-  }
-  if (src->muscle) SR_CUDA(cp(dst->muscle, src->muscle, n_env * dst->muscle_dim * sizeof(double)));
-  if (src->spline) SR_CUDA(cp(dst->spline, src->spline, n_env * dst->spline_dim * sizeof(double)));
   return SR_OK;
+}
+
+int sr_copy_envs(sr_handle *dst, const int32_t *dst_idx_dev, const sr_handle *src, const int32_t *src_idx_dev, int n,
+                 void *stream) {
+  if (!dst || !src) return fail(SR_E_INVALID, "sr_copy_envs: null handle");
+  if (n < 0 || n > dst->cfg.n_env) return fail(SR_E_INVALID, "sr_copy_envs: n out of range (0 <= n <= n_env of dst)");
+  if (n == 0) return SR_OK;
+  if (!dst_idx_dev || !src_idx_dev) return fail(SR_E_INVALID, "sr_copy_envs: null index array");
+  if (dst->cfg.device != src->cfg.device)
+    return fail(SR_E_INVALID, "sr_copy_envs: the two handles are on different devices (sr_copy_from copies across devices)");
+  if (!same_env_shape(dst, src))
+    return fail(SR_E_INVALID, "sr_copy_envs: the two handles were created with different shapes (n_elem, n_rod, dtype, model, "
+                              "head, muscle or spline forcing)");
+  SR_CUDA(cudaSetDevice(dst->cfg.device));
+  cudaStream_t s = (cudaStream_t)stream;
+  const int rc = alloc_lazy_like(dst, src);
+  if (rc != SR_OK) return rc;
+  EnvBuf d[EB_COUNT], sb[EB_COUNT];
+  env_buffers(dst, d);
+  env_buffers(src, sb);
+  // a buffer dst has and src has not: zeros for the lazy ones (their value before first use), untouched otherwise
+  // (as sr_copy_from leaves it)
+  sr::CopyTable t{};
+  for (int k = 0; k < EB_COUNT; k++) {
+    if (!d[k].base || (!sb[k].base && !d[k].lazy)) continue;
+    t.buf[t.n_buf++] = {(const char *)sb[k].base, (char *)d[k].base, d[k].bytes, copy_vec(sb[k].base, d[k].base, d[k].bytes)};
+  }
+  t.n_src = src->cfg.n_env;
+  t.n_dst = dst->cfg.n_env;
+  if (src != dst) return launch_copy(dst, t, dst_idx_dev, src_idx_dev, n, s);
+  // within one handle every source row is read before any destination row is written: gather the n source rows into
+  // the staging buffer (one region of n rows per buffer), then scatter them
+  size_t stage = 0;
+  for (int k = 0; k < t.n_buf; k++) stage += ((size_t)n * t.buf[k].bytes + 15) / 16 * 16;
+  if (stage > dst->copy_stage_bytes) {
+    cudaFree(dst->copy_stage);
+    dst->copy_stage = nullptr; dst->copy_stage_bytes = 0;
+    SR_CUDA(cudaMalloc(&dst->copy_stage, stage));
+    dst->copy_stage_bytes = stage;
+  }
+  sr::CopyTable gather = t, scatter = t;
+  gather.mode = sr::COPY_GATHER;
+  scatter.mode = sr::COPY_SCATTER;
+  char *region = (char *)dst->copy_stage;
+  for (int k = 0; k < t.n_buf; k++) {
+    gather.buf[k].dst = region;
+    scatter.buf[k].src = region;
+    // (the region's base is 16-byte aligned, so the vector width of the row size holds on both sides)
+    region += ((size_t)n * t.buf[k].bytes + 15) / 16 * 16;
+  }
+  const int rg = launch_copy(dst, gather, dst_idx_dev, src_idx_dev, n, s);
+  return rg != SR_OK ? rg : launch_copy(dst, scatter, dst_idx_dev, src_idx_dev, n, s);
 }
 
 static int measure_fp64_peak_impl(int device, double *tflops_out, bool three_regs) {

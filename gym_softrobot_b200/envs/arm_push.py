@@ -17,6 +17,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Discrete, Env
 from .soft_pendulum import _advance_time
 
@@ -67,9 +68,11 @@ def _make_handle(n_env, time_step, device, pull_weight):
                       tm_muscle=dict(max_stress=1.0, radius_ref=_ARM["base_radius"]), **_ARM, **kw)
 
 
-class ArmPushVectorEnv:
+class ArmPushVectorEnv(ForkableVectorEnv):
     """N independent OctoArmPush / OctoArmPullWeight envs (torch CUDA I/O), one physics launch per env-step.
     `mode` "discrete": actions are an integer tensor [n_env] in {0, 1}; "continuous": float [n_env, 2] in [0, 1]."""
+
+    PER_ENV = ("step_count", "prev_action")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=2.5, time_step=5.0e-5, recording_fps=40, mode="discrete",
                  pull_weight=False, device: int = 0, autoreset: bool = True, config_early_termination: bool = False):

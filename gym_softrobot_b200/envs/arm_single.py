@@ -12,6 +12,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 from .soft_pendulum import _advance_time
 
@@ -44,8 +45,10 @@ def _make_handle(n_env, n_elems, time_step, device, dtype=nat.DTYPE_F64):
                       device=device, dtype=dtype, contact=arm_contact_params(), **_ROD)
 
 
-class ArmSingleVectorEnv:
+class ArmSingleVectorEnv(ForkableVectorEnv):
     """N independent OctoArmSingle-v0 envs (torch CUDA I/O), one physics launch per env-step."""
+
+    PER_ENV = ("step_count", "prev_action", "prev_kappa", "prev_com", "prev_dist")   # per-env host state (copy_envs)
 
     kappa_range = [-49.33508476187419, 49.33545827754751]
     kappa_rate_range = [-21.063520620377012, 24.664591289161944]

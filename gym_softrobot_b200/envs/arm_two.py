@@ -15,6 +15,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 from .octo_crawl import _ARM, _DAMPER_TIME_STEP, _HEAD_DENSITY, _HEAD_RADIUS, _JOINT
 from .octo_reach import _LM_MAX_STRESS, _TM_MAX_STRESS, es_longitudinal_positions
@@ -46,8 +47,10 @@ def activation_interp_matrix(control_location, n_elems):
     return np.stack(cols, axis=1)
 
 
-class ArmTwoVectorEnv:
+class ArmTwoVectorEnv(ForkableVectorEnv):
     """N independent OctoArmTwo-v0 envs (torch CUDA I/O), one physics launch per env-step; actions float [n_env, 18]."""
+
+    PER_ENV = ("step_count", "prev_action", "prev_kappa")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=5.0, time_step=5.0e-5, recording_fps=25, n_elems=20, device: int = 0,
                  autoreset: bool = True):

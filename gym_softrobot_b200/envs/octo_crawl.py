@@ -14,6 +14,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 from .soft_pendulum import _advance_time
 
@@ -37,8 +38,10 @@ def crawl_init_params(n_arm=_N_ARM):
     return np.array([row]), angles
 
 
-class OctoCrawlVectorEnv:
+class OctoCrawlVectorEnv(ForkableVectorEnv):
     """N independent OctoCrawl-v0 envs (torch CUDA I/O), one physics launch per env-step; actions float [n_env, 24]."""
+
+    PER_ENV = ("step_count", "prev_action", "_final")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=10.0, time_step=5.0e-5, recording_fps=25, n_elems=20,
                  config_random_final_time=False, device: int = 0, autoreset: bool = True):

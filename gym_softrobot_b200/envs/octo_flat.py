@@ -12,6 +12,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Dict, Env
 from .arm_single import arm_contact_params, _ROD, _G
 from .soft_pendulum import _advance_time
@@ -60,10 +61,12 @@ def count_crossings(p1, p2):
     return hit.sum(dim=(1, 2))
 
 
-class OctoFlatVectorEnv:
+class OctoFlatVectorEnv(ForkableVectorEnv):
     """N independent OctoFlat-v0 envs, torch CUDA I/O.  `policy_mode` as in the reference (flat_env.py:84-145,
     248-271): "decentralized" declares a per-arm action space and appends the arm's one-hot id to each
     row of the individual observation; the physics and the batched action layout are the same."""
+
+    PER_ENV = ("step_count", "prev_action", "target")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=5.0, time_step=7.0e-5, recording_fps=5, n_elems=10, n_arm=8,
                  n_action=3, device: int = 0, autoreset: bool = True, env_offset: int = 0,

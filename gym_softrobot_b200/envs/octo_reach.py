@@ -14,6 +14,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 from .octo_crawl import _ARM, _DAMPER_TIME_STEP, _HEAD_DENSITY, _HEAD_RADIUS, _JOINT, _N_ARM, crawl_init_params
 from .soft_pendulum import _advance_time
@@ -31,9 +32,11 @@ def es_longitudinal_positions():
     return out
 
 
-class OctoReachVectorEnv:
+class OctoReachVectorEnv(ForkableVectorEnv):
     """N independent OctoReach-v0 envs (torch CUDA I/O), one physics launch per env-step; actions float
     [n_env, 8 * 3 * n_elems]."""
+
+    PER_ENV = ("step_count", "prev_action", "target")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=5.0, time_step=5.0e-5, recording_fps=25, n_elems=20, device: int = 0,
                  autoreset: bool = True):

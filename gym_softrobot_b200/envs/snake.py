@@ -15,6 +15,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 
 _L0 = 0.35
@@ -67,9 +68,11 @@ def projected_forward_velocity(times, com, vel, period):
     return along[:, 2 * P:].mean(dim=1)[:, 2]
 
 
-class ContinuumSnakeVectorEnv:
+class ContinuumSnakeVectorEnv(ForkableVectorEnv):
     """N independent ContinuumSnake-v0 envs (torch CUDA I/O); they advance in lockstep (the reference
     env never terminates early, so every env truncates at the same step)."""
+
+    PER_ENV = ("_com", "_vel")   # per-env host state (copy_envs)
 
     period = 2.0
     time_step = 8e-6
@@ -132,6 +135,14 @@ class ContinuumSnakeVectorEnv:
         n = self.n_env
         return self.torch.cat([f["position_collection"].reshape(n, -1), f["velocity_collection"].reshape(n, -1),
                                f["director_collection"].reshape(n, -1)], dim=1).float()
+
+    def _check_copy_source(self, src):
+        # the envs of a batch share one host clock and sample history: envs of another batch continue here only
+        # from the same instant
+        if src is not self and (src._clock != self._clock or src._substeps != self._substeps or src._times != self._times):
+            raise ValueError("copy_envs: a ContinuumSnake env continues only in a vector env at the same clock "
+                             f"(src at t = {float(src._clock)}, {src._substeps} substeps; here t = {float(self._clock)}, "
+                             f"{self._substeps} substeps)")
 
     def _projected_velocity(self):
         S = len(self._times)

@@ -15,6 +15,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 from .soft_pendulum import _advance_time
 
@@ -73,7 +74,7 @@ def _make_handle(n_env, device, dtype=nat.DTYPE_F64, n_elems=_N_ELEM, time_step=
         spline=dict(directions=(0, 1), n_ctrl=_N_CTRL, scale=spline_scale(n_elems), max_rate=float("inf")))
 
 
-class SoftArmTrackingVectorEnv:
+class SoftArmTrackingVectorEnv(ForkableVectorEnv):
     """N independent SoftArmTracking-v0 envs (torch CUDA I/O, float64), one physics launch per env-step.
 
     `n_elems` (3-4095; 1024 and more step on thread-block clusters) and `time_step` refine the arm.  An env-step stays
@@ -83,6 +84,8 @@ class SoftArmTrackingVectorEnv:
     2048-element arm diverges within its first env-step at 5e-6 s and at 2.5e-6 s; scaled, it tracks a 1024-element arm
     at 1e-5 s to 0.02 mm at the tip after three env-steps of random targets (longer horizons not checked).  A finer arm
     needs a smaller step: 5e-6 s at 2048 elements."""
+
+    PER_ENV = ("tick", "_targets")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, game_mode: int = 1, device: int = 0, autoreset: bool = True, n_elems: int = _N_ELEM,
                  time_step: float = _DT):

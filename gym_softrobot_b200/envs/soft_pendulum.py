@@ -15,6 +15,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 
 # defaults of the reference build function (soft_pendulum/build.py:19-26)
@@ -135,7 +136,7 @@ class SoftPendulumEnv(Env):
             self._handle = None
 
 
-class SoftPendulumVectorEnv:
+class SoftPendulumVectorEnv(ForkableVectorEnv):
     """N independent SoftPendulum-v0 envs stepped by one kernel launch per env-step.
 
     Observations / rewards / flags are torch tensors on the GPU; actions are a
@@ -144,6 +145,8 @@ class SoftPendulumVectorEnv:
     are reset inside the same `step` call (final observation returned in
     `info["final_obs"]`).
     """
+
+    PER_ENV = ("step_count", "prev_action")   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=5.0, time_step=1.0e-4, recording_fps=25, n_elems=50,
                  device: int = 0, math: int = nat.MATH_FAST, autoreset: bool = True,

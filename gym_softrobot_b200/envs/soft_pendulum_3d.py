@@ -15,6 +15,7 @@ from typing import Optional
 import numpy as np
 
 from .. import _native as nat
+from .fork import ForkableVectorEnv
 from ..compat import Box, Env
 from .soft_pendulum import _advance_time
 
@@ -110,8 +111,10 @@ class SoftPendulum3DEnv(Env):
             self._handle = None
 
 
-class SoftPendulum3DVectorEnv:
+class SoftPendulum3DVectorEnv(ForkableVectorEnv):
     """N independent SoftPendulum3D-v0 envs, one kernel launch per env-step (torch CUDA I/O)."""
+
+    PER_ENV = ("step_count",)   # per-env host state (copy_envs)
 
     def __init__(self, n_env, final_time=5.0, time_step=1.0e-4, recording_fps=25, n_elems=50,
                  device: int = 0, autoreset: bool = True, env_offset: int = 0):

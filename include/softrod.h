@@ -250,6 +250,21 @@ int sr_get_ext_loads(sr_handle *h, void **force_dev, void **couple_dev);
  * arrays, BC anchors, model scratch, rigid heads, rest curvatures, muscle / spline forcing state.  Checkpoint /
  * restore; works across devices (peer copy).  Stream-ordered on `stream` of dst's device. */
 int sr_copy_from(sr_handle *dst, sr_handle *src, void *stream);
+/* Fork envs: for i < n, env dst_idx[i] of `dst` takes everything that evolves or parametrises env src_idx[i] of `src`
+ * (the per-env rows of what sr_copy_from clones: rod arrays, BC anchors, model scratch, rigid head, rest curvatures,
+ * external loads, sucker ratios and indices, muscle activations, muscle / spline forcing state).  `src` may be `dst`.
+ * Index arrays are int32 device arrays.  Stream-ordered on `stream` (dst's device).  A copy within one handle goes
+ * through a staging buffer the handle owns: issue the copies of one handle on one stream (or order their streams), as
+ * for the handle's other calls.
+ *   - Every source row is read before any destination row is written, so permutations and swaps within one handle
+ *     work; destinations must be distinct; a pair with src_idx[i] == dst_idx[i] within one handle leaves the env as is.
+ *   - 0 <= n <= dst's n_env (n = 0: nothing to do).  Both handles on the same device, created with the same shapes
+ *     apart from n_env (as for sr_copy_from).  A pair with an index outside [0, n_env) of its handle is skipped.
+ *   - A rest-curvature or external-load buffer the source never allocated zeroes the destination rows (its initial
+ *     value); one the destination lacks is allocated first.
+ *   - Handle-level state is not copied (fallback counters and windows, launch count): it does not change an env's bits. */
+int sr_copy_envs(sr_handle *dst, const int32_t *dst_idx_dev, const sr_handle *src, const int32_t *src_idx_dev,
+                 int n, void *stream);
 
 /* Per-env model scratch, [n_env][*dim] of the handle's dtype: SoftPendulum3D keeps the base controller there
  * (0-2 position, 3-5 velocity, 6 last tilt angle, `info["tilt"]` of soft_pendulum_3d.py:157). */
